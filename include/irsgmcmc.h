@@ -162,8 +162,8 @@ int irs_vd_factor_residual(const float* r, const unsigned char* mask, double* al
                            unsigned int* counter, int D, int H, int W, void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------------ *
- * Per-sample evaluation -- replaces calc_no_non_diffeomorphic_voxels + calc_det_J (utils/util.py:72-91,209-212) and
- * calc_DSC_GPU (utils/util.py:123-148).
+ * Per-sample evaluation -- replaces calc_no_non_diffeomorphic_voxels + calc_det_J (utils/util.py:72-91,209-212),
+ * calc_DSC_GPU (utils/util.py:123-148) and the average surface distance of calc_metrics (utils/util.py:171-176).
  *   log_det (C,D,H,W) optional: log det J of the transformation T (normalised units, spacing 2/(n-1));
  *   n_folded: C ints = number of voxels whose log det J is NaN (negative determinant)
  *   counts (C, n_labels, 3) unsigned: |A = l|, |B = l|, |A = l and B = l| for int16 label volumes; labels != 0
@@ -171,6 +171,26 @@ int irs_vd_factor_residual(const float* r, const unsigned char* mask, double* al
 int irs_log_det_jacobian(const float* T, float* log_det, int* n_folded, int C, int D, int H, int W, void* stream);
 int irs_dice_counts(const short* seg_a, long long a_chain_stride, const short* seg_b, const int* labels_host,
                     int n_labels, unsigned int* counts, int C, long long V, void* stream);
+
+/* Average surface distance -- replaces the LabelContour + HausdorffDistanceImageFilter.GetAverageHausdorffDistance() part of
+ * calc_metrics (utils/util.py:171-176).  For sample c and label l, A = (seg_a[c] == l), B = (seg_b[c] == l); the contour of a
+ * set is its voxels with a face neighbour outside it (outside the volume = outside); ASD = (mean over the contour of A of the
+ * Euclidean distance to the contour of B + the same from B to A) / 2, inf when A or B is empty, spacing applied.
+ *   irs_surface_boxes: boxes (C, n_labels, 8) ints = bounding box of A u B (z0, y0, x0, z1, y1, x1 inclusive), |A|, |B|.
+ *   irs_average_surface_distance: for the pairs p = c * n_labels + l in [pair_begin, pair_end), asd[p] (asd is the whole
+ *     (C, n_labels) double array).  boxes_host = the table above copied to the host; spacing_host = 3 floats (x, y, z), the W
+ *     axis uses x; workspace >= 2 * (box voxels) floats summed over the non-empty pairs of the range, else IRS_ERR_WORKSPACE;
+ *     partials IRS_ASD_PARTIALS_DOUBLES doubles; counters IRS_ASD_MAX_BOXES unsigned.  Deterministic (no float atomics).
+ * seg_a / seg_b int16 as for irs_dice_counts; labels != 0 (IRS_ERR_UNSUPPORTED); spacing finite and > 0 (IRS_ERR_BAD_ARG). */
+#define IRS_ASD_MAX_BOXES 48          /* (sample, label) boxes per launch group */
+#define IRS_ASD_REDUCE_BLOCKS 64      /* blocks of the reduction per box, at most */
+#define IRS_ASD_PARTIALS_DOUBLES (IRS_ASD_MAX_BOXES * 4 * IRS_ASD_REDUCE_BLOCKS)
+int irs_surface_boxes(const short* seg_a, long long a_chain_stride, const short* seg_b, const int* labels_host,
+                      int n_labels, int* boxes, int C, int D, int H, int W, void* stream);
+int irs_average_surface_distance(const short* seg_a, long long a_chain_stride, const short* seg_b, const int* labels_host,
+                                 int n_labels, const int* boxes_host, const float* spacing_host, int pair_begin,
+                                 int pair_end, float* workspace, long long workspace_floats, double* partials,
+                                 unsigned int* counters, double* asd, int C, int D, int H, int W, void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------------ *
  * Posterior moments -- replaces calc_posterior_statistics (utils/util.py:114-120) without the host-side sample buffer:

@@ -74,6 +74,9 @@ class ViBuffers(ctypes.Structure):
                 ('adam_eps', ctypes.c_double)]
 
 
+# average surface distance scratch (include/irsgmcmc.h): IRS_ASD_MAX_BOXES counters, IRS_ASD_PARTIALS_DOUBLES partials
+ASD_MAX_BOXES, ASD_PARTIALS_DOUBLES = 48, 48 * 4 * 64
+
 VI_STATE_SIZE, VI_STEP, VI_BETA_POW, VI_X, VI_SUMS, VI_ENTROPY = 16, 0, 1, 3, 4, 8
 
 # name -> (restype, argtypes); every symbol include/irsgmcmc.h declares
@@ -108,6 +111,9 @@ SYMBOLS = {
     'irs_vd_factor_residual': (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _vp]),
     'irs_log_det_jacobian': (_i, [_vp, _vp, _vp, _i, _i, _i, _i, _vp]),
     'irs_dice_counts': (_i, [_vp, _ll, _vp, _vp, _i, _vp, _i, _ll, _vp]),
+    'irs_surface_boxes': (_i, [_vp, _ll, _vp, _vp, _i, _vp, _i, _i, _i, _i, _vp]),
+    'irs_average_surface_distance': (_i, [_vp, _ll, _vp, _vp, _i, _vp, _vp, _i, _i, _vp, _ll, _vp, _vp, _vp, _i, _i, _i, _i,
+                                          _vp]),
     'irs_welford_update': (_i, [_vp, _i, _ll, _d, _vp, _vp, _vp]),
     'irs_welford_std': (_i, [_vp, _d, _vp, _ll, _vp]),
     'irs_sgld_partials_doubles': (_sz, [ctypes.POINTER(SgldConfig)]),

@@ -55,6 +55,12 @@ __device__ __forceinline__ float irs_jitter_normalised(float u01, float alpha, i
     return __fdiv_rn(__fmul_rn(noise, 2.0f), (float)(n - 1));
 }
 
+// up to 32 segmentation labels of one per-sample evaluation launch (Dice counts, surface distance)
+struct LabelList {
+    int n;
+    int v[32];
+};
+
 struct IrsTaps {
     int n;
     float w[IRS_MAX_TAPS + 1];

@@ -38,11 +38,6 @@ log_det_j_kernel(const float* __restrict__ T_all, float* __restrict__ log_det, i
     if ((threadIdx.x & 31) == 0 && folded) atomicAdd(n_folded + c, folded);   // integer: order independent
 }
 
-struct LabelList {
-    int n;
-    int v[32];
-};
-
 // counts[c][l] = (|A == l|, |B == l|, |A == l and B == l|)
 __global__ void __launch_bounds__(256)
 dice_counts_kernel(const short* __restrict__ seg_a, long long a_cs, const short* __restrict__ seg_b, LabelList labels,

@@ -340,3 +340,57 @@ def dice_counts(seg_a, seg_b, labels):
     _lib.check(lib.irs_dice_counts(_lib.ptr(seg_a), stride, _lib.ptr(seg_b), lab, len(labels), _lib.ptr(counts), C, V,
                                    _lib.stream()))
     return counts
+
+
+def average_surface_distance(seg_a, seg_b, labels, spacing, workspace_bytes=512 << 20):
+    """float64 (C, n_labels) average surface distance of the structures seg_a == l and seg_b[c] == l (the reference's
+    LabelContour + average Hausdorff distance, utils/util.py:171-176): inf when either is empty.  int16 label volumes (C or
+    1, 1, D, H, W); seg_a may be one volume shared by all samples; spacing (x, y, z).  The distance transforms run over the
+    bounding box of each (sample, structure), 8 bytes per box voxel, in batches of pairs whose workspace fits
+    `workspace_bytes` (a pair larger than that runs alone).  One host synchronisation per 32 labels (the box table)."""
+    import ctypes
+    lib = _lib.load()
+    _lib.require_cuda(seg_a, seg_b)
+    if seg_a.dtype != torch.int16 or seg_b.dtype != torch.int16:
+        raise NotImplementedError('int16 segmentations only')
+    if seg_b.dim() < 4 or seg_b[0].numel() != seg_b.shape[-3] * seg_b.shape[-2] * seg_b.shape[-1]:
+        raise ValueError('expected (C, [1,] D, H, W) label volumes')
+    C, (D, H, W) = seg_b.shape[0], seg_b.shape[-3:]
+    if seg_a.shape[0] not in (1, C) or seg_a.shape[1:] != seg_b.shape[1:]:
+        raise ValueError(f'seg_a {tuple(seg_a.shape)} does not match seg_b {tuple(seg_b.shape)}')
+    stride = 0 if seg_a.shape[0] == 1 else D * H * W
+    sp = _lib.host_floats([float(x) for x in spacing])
+    if len(sp) != 3:
+        raise ValueError('spacing: three values (x, y, z)')
+    labels = [int(x) for x in labels]
+    dev = seg_b.device
+    out = torch.empty(C, len(labels), device=dev, dtype=torch.float64)
+    partials = torch.empty(_lib.ASD_PARTIALS_DOUBLES, device=dev, dtype=torch.float64)
+    counters = torch.empty(_lib.ASD_MAX_BOXES, device=dev, dtype=torch.int32)
+    budget = max(1, int(workspace_bytes) // 4)
+    for l0 in range(0, len(labels), 32):
+        chunk = labels[l0:l0 + 32]
+        n = len(chunk)
+        lab = (ctypes.c_int * n)(*chunk)
+        boxes = torch.empty(C, n, 8, device=dev, dtype=torch.int32)
+        _lib.check(lib.irs_surface_boxes(_lib.ptr(seg_a), stride, _lib.ptr(seg_b), lab, n, _lib.ptr(boxes), C, D, H, W,
+                                         _lib.stream()))
+        bh = boxes.cpu().view(-1, 8)
+        ext = (bh[:, 3:6] - bh[:, 0:3] + 1).long()
+        need = torch.where((bh[:, 6] > 0) & (bh[:, 7] > 0), 2 * ext.prod(1), torch.zeros_like(ext[:, 0])).tolist()
+        batches, begin, acc = [], 0, 0   # consecutive pairs whose workspace fits the budget
+        for p, f in enumerate(need):
+            if acc + f > budget and p > begin:
+                batches.append((begin, p, acc))
+                begin, acc = p, 0
+            acc += f
+        batches.append((begin, len(need), acc))
+        ws = torch.empty(max(1, max(b[2] for b in batches)), device=dev, dtype=torch.float32)
+        asd = torch.empty(C, n, device=dev, dtype=torch.float64)
+        host_boxes = bh.contiguous().numpy()
+        for b, e, f in batches:
+            _lib.check(lib.irs_average_surface_distance(
+                _lib.ptr(seg_a), stride, _lib.ptr(seg_b), lab, n, host_boxes.ctypes.data_as(ctypes.c_void_p), sp, b, e,
+                _lib.ptr(ws), ws.numel(), _lib.ptr(partials), _lib.ptr(counters), _lib.ptr(asd), C, D, H, W, _lib.stream()))
+        out[:, l0:l0 + n] = asd
+    return out

@@ -20,6 +20,7 @@ which calls the adjoint op (the closed forms of SURVEY Appendix A, no scatter at
     calc_posterior_statistics (utils/util.py:114-120)                     irsgmcmc::welford_update (in place), ::welford_std
     calc_no_non_diffeomorphic_voxels (utils/util.py:209-212)              irsgmcmc::log_det_jacobian
     calc_DSC_GPU (utils/util.py:123-148)                                  irsgmcmc::dice_counts
+    calc_metrics, ASD part (utils/util.py:171-176)                        irsgmcmc::average_surface_distance
     Trainer._SGLD_transition (trainer/trainer.py:291-356)                 irsgmcmc::sgld_step (the fused transition, in place)
 
 The drop-in modules (utils/, model/) and the fused sampler use the same launchers; this module adds the dispatcher-visible
@@ -390,6 +391,18 @@ def _(seg_a, seg_b, labels):
     return seg_b.new_empty(seg_b.shape[0], len(labels), 3, dtype=torch.int32)
 
 
+@_op('average_surface_distance')
+def average_surface_distance(seg_a: Tensor, seg_b: Tensor, labels: Sequence[int], spacing: Sequence[float]) -> Tensor:
+    """float64 (C, n_labels): average surface distance of seg_a == l and seg_b[c] == l, spacing (x, y, z); inf when either is
+    empty (seg_a may be one volume shared by all samples)"""
+    return ops.average_surface_distance(seg_a.contiguous(), seg_b.contiguous(), list(labels), list(spacing))
+
+
+@average_surface_distance.register_fake
+def _(seg_a, seg_b, labels, spacing):
+    return seg_b.new_empty(seg_b.shape[0], len(labels), dtype=torch.float64)
+
+
 # ---- the fused transition -------------------------------------------------------------------------------------------------------------
 _SAMPLERS = {}
 
@@ -420,4 +433,5 @@ def _(v, hyper, stats, handle, n):
 
 OPS = ('warp3d', 'warp3d_bwd_grid', 'warp3d_nearest', 'svf_exp', 'svf_exp_bwd', 'sobolev_smooth', 'lcc_normalise',
        'lcc_normalise_bwd', 'reg_energy', 'reg_energy_grad', 'ffd', 'ffd_adjoint', 'langevin_proposal', 'gmm_log_pdf',
-       'gmm_log_pdf_param_grads', 'vd_factor', 'welford_update', 'welford_std', 'log_det_jacobian', 'dice_counts', 'sgld_step')
+       'gmm_log_pdf_param_grads', 'vd_factor', 'welford_update', 'welford_std', 'log_det_jacobian', 'dice_counts', 'average_surface_distance',
+       'sgld_step')

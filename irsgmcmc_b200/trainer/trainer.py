@@ -525,8 +525,9 @@ class Trainer:
     def _run_MCMC(self, data_loss=None, reg_loss=None, speed_test_iters=100, with_ASD=False):
         """burn-in + sampling; returns {'mean','std_dev', 'im_mean','im_std', 'n', 'DSC', 'ASD', 'no_non_diffeomorphic_voxels',
         'samples_per_sec'}; posterior statistics are over the kept samples of ALL ranks.  'ASD' (average surface distance,
-        reference utils/util.py:171-176 through SimpleITK on the host): with_ASD=True computes it per kept sample on the host with
-        scipy (utils.util.calc_ASD_host, parity unpinned); otherwise the entry is a string saying that it was not computed."""
+        reference utils/util.py:171-176 through SimpleITK on the host): with_ASD=True computes it per kept sample on the device
+        (utils.util.calc_metrics -> calc_ASD_GPU: one host synchronisation per sample, parity with SimpleITK unpinned), a
+        (chains, structures) array per kept sample; otherwise the entry is a string saying that it was not computed."""
         if self.SGLD_params is None:
             self._SGLD_init()
         s = self.sampler
@@ -578,8 +579,8 @@ class Trainer:
         result = {'mean': mom['displacement_mean'], 'std_dev': mom['displacement_std'], 'im_mean': mom['im_mean'],
                   'im_std': mom['im_std'], 'n': mom['n'], 'DSC': dsc, 'no_non_diffeomorphic_voxels': folded,
                   'ASD': asd if with_ASD else 'unavailable: not requested (with_ASD=True computes the label-contour average '
-                                              'Hausdorff distance of reference utils/util.py:171-176 on the host with scipy instead of '
-                                              'SimpleITK; parity unpinned)'}
+                                              'Hausdorff distance of reference utils/util.py:171-176 per kept sample with the CUDA '
+                                              'distance transform kernels; parity with SimpleITK unpinned)'}
         if self.save_dir is not None and (not torch.distributed.is_initialized() or torch.distributed.get_rank() == 0):
             # MCMC_sample_{mean,std_dev}[_masked].vtk like the reference (trainer.py:457-460, logger/logger.py:110-131)
             from ..logger import save_displacement_mean_and_std_dev

@@ -135,6 +135,23 @@ def calc_DSC_GPU(no_samples, seg_fixed, seg_moving, structures_dict):
     return (2.0 * cnt[..., 2] / (cnt[..., 0] + cnt[..., 1])).float().numpy()
 
 
+@torch.no_grad()
+def calc_ASD_GPU(no_samples, seg_fixed, seg_moving, structures_dict, spacing):
+    """average surface distance per sample and structure (the reference's calc_metrics, utils/util.py:171-176), float64
+    (no_samples, structures), inf where a structure is empty: the label-contour / exact Euclidean distance transform kernels,
+    one host synchronisation per call and no volume copies.  Same definition as calc_ASD_host, which the tests compare it
+    with.  int16 CUDA segmentations only -- no PyTorch path."""
+    labels = [int(x) for x in structures_dict.values()]
+    a, b = seg_fixed[:no_samples], seg_moving[:no_samples].contiguous()
+    if not (a.is_cuda and b.is_cuda) or a.dtype != torch.int16 or b.dtype != torch.int16:
+        raise NotImplementedError('calc_ASD_GPU needs int16 CUDA segmentations: irsgmcmc_b200 has no CPU path')
+    if 0 in labels:
+        raise NotImplementedError('calc_ASD_GPU: label 0 is the background of the surface kernels')
+    a = a[:1].contiguous() if a.stride(0) == 0 else a.contiguous()
+    sp = [float(x) for x in np.asarray(spacing.cpu() if hasattr(spacing, 'cpu') else spacing, dtype=np.float64).reshape(-1)[:3]]
+    return ops.average_surface_distance(a, b, labels, sp).cpu().numpy()
+
+
 def _label_contour(mask):
     """ITK LabelContourImageFilter with its defaults on a binary image: a foreground voxel belongs to the contour when one of its
     six face neighbours is background (FullyConnectedOff); voxels on the image border count as touching background."""
@@ -175,17 +192,11 @@ def calc_ASD_host(seg_fixed_structure, seg_moving_structure, spacing=(1.0, 1.0, 
 
 @torch.no_grad()
 def calc_metrics(seg_fixed, seg_moving, structures_dict, spacing, GPU=True, no_samples=1):
-    """(ASD, DSC) per sample and structure like the reference's calc_metrics (:151-206).  DSC: the counting kernel
-    (calc_DSC_GPU; `GPU=False` is not offered -- there is no host Dice).  ASD: calc_ASD_host per sample and structure on the
-    host, as in the reference (parity unpinned, see there); needs scipy."""
+    """(ASD, DSC) per sample and structure like the reference's calc_metrics (:151-206), both from CUDA kernels: DSC from the
+    counting kernel (calc_DSC_GPU), ASD from the label-contour / distance transform kernels (calc_ASD_GPU; same definition
+    as the host restatement calc_ASD_host, parity with SimpleITK unpinned, see there).  `GPU=False` is not offered."""
     if not GPU:
         raise NotImplementedError('calc_metrics(GPU=False): the Dice scores come from the CUDA counting kernel only')
     DSC = calc_DSC_GPU(no_samples, seg_fixed, seg_moving, structures_dict)
-    a, b = seg_fixed[:no_samples].cpu().numpy(), seg_moving[:no_samples].cpu().numpy()
-    sp = spacing.numpy().tolist() if hasattr(spacing, 'numpy') else list(spacing)
-    ASD = np.zeros([no_samples, len(structures_dict)])
-    for idx in range(no_samples):
-        fa, mb = a[min(idx, a.shape[0] - 1)].squeeze(), b[idx].squeeze()
-        for j, label in enumerate(structures_dict.values()):
-            ASD[idx, j] = calc_ASD_host(fa == label, mb == label, sp)
+    ASD = calc_ASD_GPU(no_samples, seg_fixed, seg_moving, structures_dict, spacing)
     return ASD, DSC
