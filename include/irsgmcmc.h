@@ -203,6 +203,34 @@ int irs_welford_update(const float* sample, int n_new, long long n, double count
 int irs_welford_std(const float* m2, double count, float* std_out, long long n, void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------------ *
+ * Convergence diagnostics -- voxel-wise split R-hat (Gelman et al., BDA3 section 11.4; the reference has no check).
+ * The N kept samples of every chain are split into their first and last floor(N/2) (the middle one of an odd N is dropped):
+ * M = 2 x (chains) sequences of n = floor(N/2) draws, each with its own Welford (mean, M2) in fp32.
+ *   irs_split_welford_update: folds sample `count_before` + 1 of sequence (half, c) into mean / m2, for all C chains of this
+ *     GPU in one launch.  disp (C,3,V), im (C,1,V); mean / m2 (2, C, 4, V): [half][c][0..2] displacement, [3] warped image.
+ *     half in {0, 1}.
+ *   irs_split_rhat_sums: over the n_seq sequences (n_seq, E) of mean / m2 in index order, in fp64:
+ *     sums[0..E) = S1 = sum_j mean_j;  sums[E..2E) = SW = sum_j M2_j / (n - 1).  n >= 2.
+ *   irs_split_rhat_between: sb[e] = SB = sum_j (mean_j - s1[e] / M)^2 over the same n_seq sequences; s1 and M (>= 2) are the
+ *     totals over ALL sequences (all GPUs).
+ *   irs_split_rhat_finish: rhat (n_comp, V) floats (n_comp <= IRS_RHAT_MAX_COMPONENTS, E = n_comp V) from the totals SW and SB:
+ *     W = SW / M, var+ = (n - 1) / n W + SB / (M - 1), R-hat = sqrt(var+ / W); W = 0 gives 1 when SB = 0, else +inf.
+ *     summary (n_comp, 3) doubles: per component over the voxels where mask (V bytes) != 0, max R-hat (0 for an empty mask), the
+ *     number of voxels with R-hat > 1.01 and with R-hat > 1.1 -- block partials added in a fixed order, deterministic.
+ *     partials: IRS_RHAT_PARTIALS_DOUBLES doubles; counters: IRS_RHAT_MAX_COMPONENTS unsigned ints (left zero).
+ * With several GPUs: sums -> SUM all-reduce of (S1, SW) -> between -> SUM all-reduce of SB -> finish.
+ * ------------------------------------------------------------------------------------------------------------------ */
+#define IRS_RHAT_MAX_COMPONENTS 4
+#define IRS_RHAT_REDUCE_BLOCKS 256
+#define IRS_RHAT_PARTIALS_DOUBLES (IRS_RHAT_MAX_COMPONENTS * 3 * IRS_RHAT_REDUCE_BLOCKS)
+int irs_split_welford_update(const float* disp, const float* im, int C, long long V, int half, double count_before,
+                             float* mean, float* m2, void* stream);
+int irs_split_rhat_sums(const float* mean, const float* m2, int n_seq, long long E, int n, double* sums, void* stream);
+int irs_split_rhat_between(const float* mean, int n_seq, long long E, const double* s1, int M, double* sb, void* stream);
+int irs_split_rhat_finish(const double* sw, const double* sb, int M, int n, const unsigned char* mask, int n_comp,
+                          long long V, float* rhat, double* partials, unsigned int* counters, double* summary, void* stream);
+
+/* ------------------------------------------------------------------------------------------------------------------ *
  * The fused SGLD transition -- replaces Trainer._SGLD_transition, trainer/trainer.py:291-356, for all chains of this
  * GPU, including the sequential per-chain GMM Adam step (trainer.py:316-327, 68-77; optimizers/adam_rate_decay.py),
  * the regulariser's hyper-parameter Adam step (trainer.py:353-354) and the plain-SGD state update (trainer.py:351).

@@ -77,6 +77,9 @@ class ViBuffers(ctypes.Structure):
 # average surface distance scratch (include/irsgmcmc.h): IRS_ASD_MAX_BOXES counters, IRS_ASD_PARTIALS_DOUBLES partials
 ASD_MAX_BOXES, ASD_PARTIALS_DOUBLES = 48, 48 * 4 * 64
 
+# split R-hat (include/irsgmcmc.h): components per launch, reduction scratch
+RHAT_MAX_COMPONENTS, RHAT_PARTIALS_DOUBLES = 4, 4 * 3 * 256
+
 VI_STATE_SIZE, VI_STEP, VI_BETA_POW, VI_X, VI_SUMS, VI_ENTROPY = 16, 0, 1, 3, 4, 8
 
 # name -> (restype, argtypes); every symbol include/irsgmcmc.h declares
@@ -116,6 +119,10 @@ SYMBOLS = {
                                           _vp]),
     'irs_welford_update': (_i, [_vp, _i, _ll, _d, _vp, _vp, _vp]),
     'irs_welford_std': (_i, [_vp, _d, _vp, _ll, _vp]),
+    'irs_split_welford_update': (_i, [_vp, _vp, _i, _ll, _i, _d, _vp, _vp, _vp]),
+    'irs_split_rhat_sums': (_i, [_vp, _vp, _i, _ll, _i, _vp, _vp]),
+    'irs_split_rhat_between': (_i, [_vp, _i, _ll, _vp, _i, _vp, _vp]),
+    'irs_split_rhat_finish': (_i, [_vp, _vp, _i, _i, _vp, _i, _ll, _vp, _vp, _vp, _vp, _vp]),
     'irs_sgld_partials_doubles': (_sz, [ctypes.POINTER(SgldConfig)]),
     'irs_sgld_step': (_i, [ctypes.POINTER(SgldConfig), ctypes.POINTER(SgldBuffers), _vp]),
     'irs_sgld_step_profile': (_i, [ctypes.POINTER(SgldConfig), ctypes.POINTER(SgldBuffers), _vp, _vp]),

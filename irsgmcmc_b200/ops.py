@@ -313,6 +313,69 @@ def welford_std(m2, count):
     return out
 
 
+def split_welford_update(disp, im, half, count_before, mean, m2):
+    """fold the current sample of every chain into its split-R-hat sequence of half `half` (0: first floor(N/2) kept samples,
+    1: last floor(N/2)), which already holds `count_before` draws.  disp (C,3,D,H,W), im (C,1,D,H,W); mean / m2 (2,C,4,D,H,W)
+    fp32, updated in place."""
+    lib = _lib.load()
+    _lib.require_cuda(disp, im, mean, m2)
+    C, V = disp.shape[0], disp[0, 0].numel()
+    if disp.shape[:2] != (C, 3) or im.shape[:2] != (C, 1) or im[0, 0].numel() != V:
+        raise ValueError('disp must be (C,3,D,H,W) and im (C,1,D,H,W)')
+    if tuple(mean.shape[:3]) != (2, C, 4) or mean[0, 0, 0].numel() != V or m2.shape != mean.shape:
+        raise ValueError(f'mean / m2 must be (2, {C}, 4, D, H, W)')
+    for t in (disp, im, mean, m2):
+        _f32(t)
+    _lib.check(lib.irs_split_welford_update(_lib.ptr(disp), _lib.ptr(im), C, V, int(half), float(count_before),
+                                            _lib.ptr(mean), _lib.ptr(m2), _lib.stream()))
+
+
+def split_rhat(mean, m2, n, mask, group=None, distributed=True):
+    """
+    Split R-hat (BDA3 section 11.4) per element from per-sequence Welford moments: mean / m2 (n_seq, K, D, H, W) fp32, each
+    sequence of n >= 2 draws; mask (D,H,W) bool / uint8.  With torch.distributed initialised (and `distributed`), the
+    sequences of all ranks of `group` count (two SUM all-reduces of fp64 partial sums, parallel.split_rhat_totals).
+    Returns (rhat (K,D,H,W) fp32, summary (K,3) fp64 = per component over the mask: max R-hat, voxels > 1.01, voxels > 1.1,
+    M = total number of sequences).
+    """
+    from .parallel import split_rhat_totals
+    lib = _lib.load()
+    _lib.require_cuda(mean, m2, mask)
+    _f32(mean)
+    _f32(m2)
+    if mean.dim() != 5 or m2.shape != mean.shape:
+        raise ValueError('mean / m2 must be (n_seq, K, D, H, W)')
+    n_seq, K, (D, H, W) = mean.shape[0], mean.shape[1], mean.shape[2:]
+    if not 1 <= K <= _lib.RHAT_MAX_COMPONENTS or mask.numel() != D * H * W:
+        raise ValueError(f'K must be 1..{_lib.RHAT_MAX_COMPONENTS} and mask (D,H,W)')
+    if int(n) < 2:
+        raise ValueError('split R-hat needs at least 2 draws per sequence')
+    V = D * H * W
+    E, dev, st = K * V, mean.device, _lib.stream()
+    sums = torch.empty(2, E, device=dev, dtype=torch.float64)
+    _lib.check(lib.irs_split_rhat_sums(_lib.ptr(mean), _lib.ptr(m2), n_seq, E, int(n), _lib.ptr(sums), st))
+
+    def between(s1, M):
+        sb = torch.empty(E, device=dev, dtype=torch.float64)
+        _lib.check(lib.irs_split_rhat_between(_lib.ptr(mean), n_seq, E, _lib.ptr(s1), int(M), _lib.ptr(sb), _lib.stream()))
+        return sb
+
+    if distributed:
+        M, sums, sb = split_rhat_totals(n_seq, sums, between, group)
+    else:
+        M, sb = n_seq, between(sums[0], n_seq)
+    if M < 2:
+        raise ValueError('split R-hat needs at least 2 sequences')
+    rhat = torch.empty(K, D, H, W, device=dev, dtype=torch.float32)
+    summary = torch.empty(K, 3, device=dev, dtype=torch.float64)
+    partials = torch.empty(_lib.RHAT_PARTIALS_DOUBLES, device=dev, dtype=torch.float64)
+    counters = torch.empty(_lib.RHAT_MAX_COMPONENTS, device=dev, dtype=torch.int32)
+    m8 = mask.contiguous().view(torch.uint8) if mask.dtype == torch.bool else mask.contiguous()
+    _lib.check(lib.irs_split_rhat_finish(_lib.ptr(sums[1]), _lib.ptr(sb), int(M), int(n), _lib.ptr(m8), K, V, _lib.ptr(rhat),
+                                         _lib.ptr(partials), _lib.ptr(counters), _lib.ptr(summary), _lib.stream()))
+    return rhat, summary, M
+
+
 def log_det_jacobian(T, want_log_det=True):
     """log det J of a transformation (C,3,D,H,W) and the per-sample count of folded (NaN) voxels"""
     lib = _lib.load()

@@ -1,6 +1,7 @@
 """
-Multi-GPU: chains shard by rank with no per-iteration communication (SURVEY.md section 8e).  The only collective is the
-merge of the per-rank Welford posterior moments -- two sum all-reduces (NCCL over NVLink on GPUs; gloo in CPU tests).
+Multi-GPU: chains shard by rank with no per-iteration communication (SURVEY.md section 8e).  The collectives are the
+merge of the per-rank Welford posterior moments and, when convergence diagnostics are requested, the partial sums of the split
+R-hat -- two sum all-reduces each (NCCL over NVLink on GPUs; gloo in CPU tests).
 
 The reference has no distributed code at all; the quantity computed here is its calc_posterior_statistics
 (utils/util.py:114-120: mean and unbiased std over every kept sample of every chain).
@@ -28,6 +29,29 @@ def any_rank(flag, device=None, group=None):
     t = torch.tensor([1 if flag else 0], device=device if dist.get_backend(group) == 'nccl' else 'cpu', dtype=torch.int32)
     dist.all_reduce(t, op=dist.ReduceOp.MAX, group=group)
     return bool(t.item())
+
+
+def split_rhat_totals(n_seq_local, sums, between, group=None):
+    """
+    The two collective phases of the split R-hat (ops.split_rhat), in the pattern of merge_moments.
+      sums     (2, E) fp64: this rank's S1 = sum_j mean_j and SW = sum_j M2_j / (n - 1) over its n_seq_local sequences
+      between  callable (s1_total (E,) fp64, M) -> this rank's SB = sum_j (mean_j - s1_total / M)^2, (E,) fp64
+    Phase A sum-all-reduces (M, S1, SW) as one buffer (the sequence count rides in front, padded to 2 doubles), phase B the SB
+    partials.  Returns (M, sums (2, E), SB (E,)) -- the totals over all ranks, identical on every rank.  Pure torch on the
+    partial-sum tensors: NCCL on GPUs, gloo in CPU tests.  One host read (M) between the phases.
+    """
+    if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) == 1:
+        return n_seq_local, sums, between(sums[0], n_seq_local)
+    E = sums.shape[1]
+    buf = torch.empty(2 + 2 * E, device=sums.device, dtype=torch.float64)
+    buf[:2] = float(n_seq_local)
+    buf[2:].view(2, E).copy_(sums)
+    dist.all_reduce(buf, op=dist.ReduceOp.SUM, group=group)
+    M = int(round(float(buf[0].item())))
+    total = buf[2:].view(2, E)
+    sb = between(total[0], M)
+    dist.all_reduce(sb, op=dist.ReduceOp.SUM, group=group)
+    return M, total, sb
 
 
 def merge_moments(n_local, moments, group=None):

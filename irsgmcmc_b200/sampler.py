@@ -165,6 +165,9 @@ class SGLDSampler:
 
         self._lin = [torch.linspace(-1, 1, steps=n).to(dev) for n in (W, H, D)]  # utils/util.py:270-272 of the reference
 
+        # split-R-hat accumulators (enable_convergence_diagnostics): None while disabled
+        self._rhat = None
+
     # ------------------------------------------------------------------------------------------------------------------
     def _make_config(self):
         cfg = self.cfg
@@ -294,11 +297,15 @@ class SGLDSampler:
         """everything the chains carry between transitions, as host tensors: states, preconditioner, the shared mixture /
         regulariser parameters with their Adam moments and the Philox offset (`hyper`), the running posterior moments.
         A sampler restored from it continues bit-identically (the noise is a function of seed, chain, iteration)."""
-        return {'dims': tuple(self.dims), 'state_dims': tuple(self.state_dims), 'no_chains': self.C,
-                'chain_offset': self.chain_offset, 'seed': self.cfg.seed, 'iteration': self.iteration,
-                'v': self.v.cpu(), 'sigma': None if self.sigma is None else self.sigma.cpu(), 'hyper': self.hyper.cpu(),
-                'n_kept': self.n_kept, 'disp_mean': self.disp_mean.cpu(), 'disp_m2': self.disp_m2.cpu(),
-                'im_mean': self.im_mean.cpu(), 'im_m2': self.im_m2.cpu()}
+        sd = {'dims': tuple(self.dims), 'state_dims': tuple(self.state_dims), 'no_chains': self.C,
+              'chain_offset': self.chain_offset, 'seed': self.cfg.seed, 'iteration': self.iteration,
+              'v': self.v.cpu(), 'sigma': None if self.sigma is None else self.sigma.cpu(), 'hyper': self.hyper.cpu(),
+              'n_kept': self.n_kept, 'disp_mean': self.disp_mean.cpu(), 'disp_m2': self.disp_m2.cpu(),
+              'im_mean': self.im_mean.cpu(), 'im_m2': self.im_m2.cpu()}
+        if self._rhat is not None:   # convergence diagnostics enabled: their accumulators travel too
+            r = self._rhat
+            sd['rhat'] = {'N': r['N'], 'k': r['k'], 'mean': r['mean'].cpu(), 'm2': r['m2'].cpu()}
+        return sd
 
     @torch.no_grad()
     def load_state_dict(self, sd):
@@ -311,6 +318,15 @@ class SGLDSampler:
         self.iteration, self.n_kept = int(sd['iteration']), int(sd['n_kept'])
         for name in ('disp_mean', 'disp_m2', 'im_mean', 'im_m2'):
             getattr(self, name).copy_(sd[name])
+        # a checkpoint with diagnostics enables them here; one without leaves disabled diagnostics disabled and restarts
+        # enabled ones from zero kept samples
+        if 'rhat' in sd:
+            self.enable_convergence_diagnostics(sd['rhat']['N'])
+            self._rhat['k'] = int(sd['rhat']['k'])
+            self._rhat['mean'].copy_(sd['rhat']['mean'])
+            self._rhat['m2'].copy_(sd['rhat']['m2'])
+        elif self._rhat is not None:
+            self.enable_convergence_diagnostics(self._rhat['N'])
 
     def set_noise(self, eps=None, jitter_unit=None):
         """explicit N(0,1) / U[0,1) numbers (C,3,D,H,W) instead of Philox: exact noise-on parity tests"""
@@ -496,14 +512,28 @@ class SGLDSampler:
     # posterior moments
     # ------------------------------------------------------------------------------------------------------------------
     def accumulate(self):
-        """fold the current sample of every chain into the running moments (kept-sample rule: trainer.py:414-430)"""
+        """fold the current sample of every chain into the running moments (kept-sample rule: trainer.py:414-430) and, when
+        convergence diagnostics are enabled, into the chain's split-R-hat sequence"""
         n3, n1 = 3 * self.V, self.V
         st = _lib.stream()
+        if self._rhat is not None and self._rhat['k'] >= self._rhat['N']:
+            raise RuntimeError(f'convergence diagnostics were enabled for {self._rhat["N"]} kept samples per chain: this is '
+                               f'sample {self._rhat["k"] + 1} (enable_convergence_diagnostics again to start over)')
         _lib.check(self.lib.irs_welford_update(_lib.ptr(self.displacement), self.C, n3, float(self.n_kept),
                                                _lib.ptr(self.disp_mean), _lib.ptr(self.disp_m2), st))
         _lib.check(self.lib.irs_welford_update(_lib.ptr(self.im_warped), self.C, n1, float(self.n_kept),
                                                _lib.ptr(self.im_mean), _lib.ptr(self.im_m2), st))
         self.n_kept += self.C
+        r = self._rhat
+        if r is not None:
+            # kept sample k of N: the first floor(N/2) feed half 0, the last floor(N/2) half 1, the middle one of an odd N neither
+            k, N, n = r['k'], r['N'], r['N'] // 2
+            half, count = (0, k) if k < n else ((1, k - (N - n)) if k >= N - n else (None, None))
+            if half is not None:
+                _lib.check(self.lib.irs_split_welford_update(_lib.ptr(self.displacement), _lib.ptr(self.im_warped), self.C,
+                                                             self.V, half, float(count), _lib.ptr(r['mean']),
+                                                             _lib.ptr(r['m2']), st))
+            r['k'] = k + 1
 
     def posterior_moments(self, group=None):
         """
@@ -521,3 +551,68 @@ class SGLDSampler:
                 _lib.check(self.lib.irs_welford_std(_lib.ptr(m2), float(n), _lib.ptr(std), m2.numel(), _lib.stream()))
             out[key] = std
         return out
+
+    # ------------------------------------------------------------------------------------------------------------------
+    # convergence diagnostics (voxel-wise split R-hat)
+    # ------------------------------------------------------------------------------------------------------------------
+    @torch.no_grad()
+    def enable_convergence_diagnostics(self, n_kept_per_chain):
+        """
+        Allocate (or reset) the split-R-hat accumulators for the next `n_kept_per_chain` = N kept samples of every chain: a
+        Welford (mean, M2) of the displacement (3,V) and the warped image (1,V) for the first and for the last floor(N/2)
+        samples of each chain (the middle one of an odd N is dropped) -- 64 C V bytes of fp32, e.g. 8.6 GB for 64 chains at
+        128^3.  accumulate() then also updates them (one launch, no synchronisation; the pooled moments are unchanged) and
+        raises on sample N + 1; convergence_diagnostics() needs all N.
+        With hyper_mode='reference' the chains share the mixture / regulariser parameters they step in turn, so they are not
+        independent: R-hat is still computed, but its reading as a between-independent-chains check holds for 'per_chain' and
+        'frozen'.
+        """
+        N = int(n_kept_per_chain)
+        if N < 4:
+            raise ValueError('split R-hat needs at least 4 kept samples per chain (2 draws in each half)')
+        D, H, W = self.dims
+        if self._rhat is None or self._rhat['N'] != N:
+            self._rhat = None   # release the old pair first
+            mean = torch.zeros(2, self.C, 4, D, H, W, device=self.device, dtype=torch.float32)
+            self._rhat = {'N': N, 'k': 0, 'mean': mean, 'm2': torch.zeros_like(mean)}
+        else:
+            self._rhat['k'] = 0
+            self._rhat['mean'].zero_()
+            self._rhat['m2'].zero_()
+
+    def disable_convergence_diagnostics(self):
+        """free the split-R-hat accumulators; accumulate() goes back to the pooled moments alone"""
+        self._rhat = None
+
+    @property
+    def diagnostics_enabled(self):
+        return self._rhat is not None
+
+    @torch.no_grad()
+    def convergence_diagnostics(self, group=None):
+        """
+        Split R-hat (BDA3 section 11.4) over the kept samples of ALL chains of ALL ranks of `group` (two SUM all-reduces of
+        fp64 partial sums when torch.distributed is initialised): M = 2 x total chains sequences of n = floor(N/2) draws.
+        Returns {'displacement': (3,D,H,W), 'im': (1,D,H,W) fp32 device maps,
+                 'mask': {'displacement': {...}, 'im': {...}} over the fixed mask with, per component, 'max' (list), 'n_above_1.01'
+                         and 'n_above_1.1' (lists of voxel counts), 'n_voxels' (mask size),
+                 'n': draws per sequence, 'M': number of sequences}.
+        Raises unless enabled and all N kept samples have been accumulated.
+        """
+        r = self._rhat
+        if r is None:
+            raise RuntimeError('convergence diagnostics are not enabled (enable_convergence_diagnostics(N) before sampling)')
+        if r['k'] < r['N']:
+            raise RuntimeError(f'convergence diagnostics need all {r["N"]} kept samples per chain; {r["k"]} accumulated')
+        from . import ops
+        D, H, W = self.dims
+        n = r['N'] // 2
+        rhat, summary, M = ops.split_rhat(r['mean'].view(2 * self.C, 4, D, H, W), r['m2'].view(2 * self.C, 4, D, H, W), n,
+                                          self.mask.view(D, H, W), group=group)
+        s = summary.cpu()
+
+        def part(rows):
+            return {'max': [float(x) for x in s[rows, 0]], 'n_above_1.01': [int(x) for x in s[rows, 1]],
+                    'n_above_1.1': [int(x) for x in s[rows, 2]], 'n_voxels': int(self.n_mask)}
+        return {'displacement': rhat[:3], 'im': rhat[3:], 'mask': {'displacement': part(slice(0, 3)), 'im': part(slice(3, 4))},
+                'n': n, 'M': M}

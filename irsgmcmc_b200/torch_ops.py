@@ -18,6 +18,7 @@ which calls the adjoint op (the closed forms of SURVEY Appendix A, no scatter at
     GMM.log_pdf + autograd (model/loss.py:87-93)                          irsgmcmc::gmm_log_pdf, ::gmm_log_pdf_param_grads
     rescale_residuals + calc_VD_factor (utils/util.py:330-347,446-485)    irsgmcmc::vd_factor
     calc_posterior_statistics (utils/util.py:114-120)                     irsgmcmc::welford_update (in place), ::welford_std
+    (no reference counterpart: convergence check of the chains)           irsgmcmc::split_rhat
     calc_no_non_diffeomorphic_voxels (utils/util.py:209-212)              irsgmcmc::log_det_jacobian
     calc_DSC_GPU (utils/util.py:123-148)                                  irsgmcmc::dice_counts
     calc_metrics, ASD part (utils/util.py:171-176)                        irsgmcmc::average_surface_distance
@@ -368,6 +369,20 @@ def _(m2, count):
     return torch.empty_like(m2)
 
 
+@_op('split_rhat')
+def split_rhat(mean: Tensor, m2: Tensor, n: int, mask: Tensor) -> Tuple[Tensor, Tensor]:
+    """split R-hat of the n_seq sequences given (no collectives): per-sequence Welford mean / M2 (n_seq, K, D, H, W) fp32 of n
+    draws each, mask (D, H, W) -> (R-hat (K, D, H, W) fp32, summary (K, 3) fp64: max R-hat, voxels > 1.01, voxels > 1.1 over
+    the mask)"""
+    rhat, summary, _ = ops.split_rhat(mean.contiguous(), m2.contiguous(), n, mask.contiguous(), distributed=False)
+    return rhat, summary
+
+
+@split_rhat.register_fake
+def _(mean, m2, n, mask):
+    return mean.new_empty(mean.shape[1:]), mean.new_empty(mean.shape[1], 3, dtype=torch.float64)
+
+
 # ---- per-sample evaluation ----------------------------------------------------------------------------------------------------------
 @_op('log_det_jacobian')
 def log_det_jacobian(T: Tensor) -> Tuple[Tensor, Tensor]:
@@ -433,5 +448,5 @@ def _(v, hyper, stats, handle, n):
 
 OPS = ('warp3d', 'warp3d_bwd_grid', 'warp3d_nearest', 'svf_exp', 'svf_exp_bwd', 'sobolev_smooth', 'lcc_normalise',
        'lcc_normalise_bwd', 'reg_energy', 'reg_energy_grad', 'ffd', 'ffd_adjoint', 'langevin_proposal', 'gmm_log_pdf',
-       'gmm_log_pdf_param_grads', 'vd_factor', 'welford_update', 'welford_std', 'log_det_jacobian', 'dice_counts', 'average_surface_distance',
+       'gmm_log_pdf_param_grads', 'vd_factor', 'welford_update', 'welford_std', 'split_rhat', 'log_det_jacobian', 'dice_counts', 'average_surface_distance',
        'sgld_step')

@@ -68,10 +68,13 @@ def sampler_config_from_json(config):
 
 class Trainer:
     def __init__(self, config, fixed, moving, var_params_q_v=None, structures_dict=None, device=None,
-                 chain_offset=None, logger=None, save_dir=None, im_spacing=(1.0, 1.0, 1.0)):
+                 chain_offset=None, logger=None, save_dir=None, im_spacing=(1.0, 1.0, 1.0), sampler_config=None):
         """
         config: the reference's JSON config as a dict;  fixed / moving: {'im','mask','seg'} with shape (1,1,D,H,W)
         With torch.distributed initialised, `no_chains` is the TOTAL number of chains; this rank owns a contiguous shard.
+        sampler_config: an SGLDConfig used instead of the one derived from `config`, e.g. with hyper_mode='per_chain' for
+        independent chains.  The drop-in modules mirror ONE parameter set, so with 'per_chain' the Trainer runs without them
+        (_run_MCMC() / _SGLD_transition() with data_loss = reg_loss = None).
         """
         self.config = config
         tr = config['trainer']
@@ -103,8 +106,8 @@ class Trainer:
         self.device = device
         self.fixed, self.moving = fixed, moving
         self.var_params_q_v = var_params_q_v
-        self.sampler = SGLDSampler(fixed, moving, self.no_chains, sampler_config_from_json(config), device=device,
-                                   chain_offset=offset)
+        self.sampler = SGLDSampler(fixed, moving, self.no_chains, sampler_config or sampler_config_from_json(config),
+                                   device=device, chain_offset=offset)
         self.dims = self.sampler.dims
         self.no_voxels = int(np.prod(self.dims))
         self.SGLD_params = None
@@ -168,6 +171,8 @@ class Trainer:
     def _push_hyper(self, data_loss, reg_loss, optimizer_GMM=None, optimizer_reg=None, sampler=None):
         from .. import _lib as L
         s = sampler or self.sampler
+        if s.per_chain:
+            raise NotImplementedError("hyper_mode='per_chain' has a parameter set per chain: the drop-in modules cannot mirror it")
         K = s.cfg.no_components
         optimizer_GMM = optimizer_GMM if optimizer_GMM is not None else getattr(self, 'optimizer_GMM', None)
         optimizer_reg = optimizer_reg if optimizer_reg is not None else getattr(self, 'optimizer_reg', None)
@@ -193,6 +198,8 @@ class Trainer:
         host and is mirrored at the end of _run_MCMC / on request"""
         from .. import _lib as L
         s = sampler or self.sampler
+        if s.per_chain:
+            raise NotImplementedError("hyper_mode='per_chain' has a parameter set per chain: the drop-in modules cannot mirror it")
         K = s.cfg.no_components
         if with_optimizers:
             optimizer_GMM = optimizer_GMM if optimizer_GMM is not None else getattr(self, 'optimizer_GMM', None)
@@ -522,12 +529,24 @@ class Trainer:
         return loss_terms, out, aux
 
     # -- the loop around it (reference trainer.py:358-476) -------------------------------------------------------------
-    def _run_MCMC(self, data_loss=None, reg_loss=None, speed_test_iters=100, with_ASD=False):
+    def _run_MCMC(self, data_loss=None, reg_loss=None, speed_test_iters=100, with_ASD=False, with_R_hat=False):
         """burn-in + sampling; returns {'mean','std_dev', 'im_mean','im_std', 'n', 'DSC', 'ASD', 'no_non_diffeomorphic_voxels',
         'samples_per_sec'}; posterior statistics are over the kept samples of ALL ranks.  'ASD' (average surface distance,
         reference utils/util.py:171-176 through SimpleITK on the host): with_ASD=True computes it per kept sample on the device
         (utils.util.calc_metrics -> calc_ASD_GPU: one host synchronisation per sample, parity with SimpleITK unpinned), a
-        (chains, structures) array per kept sample; otherwise the entry is a string saying that it was not computed."""
+        (chains, structures) array per kept sample; otherwise the entry is a string saying that it was not computed.
+
+        with_R_hat=True adds 'R_hat', the convergence check of the chains (split R-hat, BDA3 section 11.4, over the N kept
+        samples of every chain of every rank: M = 2 x chains sequences of floor(N/2) draws):
+          'displacement' (3,D,H,W), 'im' (1,D,H,W)  voxel-wise R-hat maps (SGLDSampler.convergence_diagnostics)
+          'mask'    per component over the fixed mask: max R-hat and the voxel counts above 1.01 and 1.1
+          'traces'  {'data', 'reg', 'alpha', 'reg_energy'} -> {'R_hat', 'ESS'} of the per-chain scalars at the kept samples
+                    (utils.diagnostics.split_rhat / ess), 'n' and 'M'
+        With save_dir, MCMC_R_hat_displacement.vtk and MCMC_R_hat_im.nii.gz are written as well.  The per-chain accumulators
+        take 64 C V bytes while the run lasts.  In hyper_mode='reference' (the default) the chains share the mixture and
+        regulariser parameters that they step in turn, so they are not independent: R-hat is still computed, but its reading
+        as a check between independent chains holds for hyper_mode 'per_chain' / 'frozen' (Trainer(sampler_config=...)).
+        With with_R_hat=False nothing of this runs and the result is unchanged."""
         if self.SGLD_params is None:
             self._SGLD_init()
         s = self.sampler
@@ -539,6 +558,12 @@ class Trainer:
                 self._GMM_init()
         dsc, asd, folded = [], [], []
         total = self.no_iters_burn_in + self.no_samples_MCMC
+        if with_R_hat:
+            n_kept = sum(1 for i in range(1, total + 1) if self._is_kept(i))
+            s.enable_convergence_diagnostics(n_kept)
+            # per kept sample, this rank's rows of the stats (alpha, data, reg, reg energy): a device copy, no synchronisation
+            traces = torch.zeros(n_kept, self.no_chains, 4, device=s.device, dtype=torch.float64)
+            k_kept = 0
         from ..utils.diff_op import GradientOperator
         diff_op = GradientOperator()
         it = 0
@@ -552,6 +577,9 @@ class Trainer:
             it = nxt
             if self._is_kept(it):
                 s.accumulate()
+                if with_R_hat:
+                    traces[k_kept].copy_(s.stats[:, :4])
+                    k_kept += 1
                 T = s.transformation()
                 if self.structures_dict and s.moving_seg is not None and 'seg' in self.fixed:
                     seg_w = s.warp_segmentation(transformation=T)
@@ -581,6 +609,8 @@ class Trainer:
                   'ASD': asd if with_ASD else 'unavailable: not requested (with_ASD=True computes the label-contour average '
                                               'Hausdorff distance of reference utils/util.py:171-176 per kept sample with the CUDA '
                                               'distance transform kernels; parity with SimpleITK unpinned)'}
+        if with_R_hat:
+            result['R_hat'] = self._R_hat(traces)
         if self.save_dir is not None and (not torch.distributed.is_initialized() or torch.distributed.get_rank() == 0):
             # MCMC_sample_{mean,std_dev}[_masked].vtk like the reference (trainer.py:457-460, logger/logger.py:110-131)
             from ..logger import save_displacement_mean_and_std_dev
@@ -596,6 +626,31 @@ class Trainer:
             torch.cuda.synchronize()
             result['samples_per_sec'] = self.no_chains * speed_test_iters / (time.perf_counter() - t0)
         return result
+
+    def _R_hat(self, traces):
+        """the 'R_hat' entry of _run_MCMC(with_R_hat=True) from the filled accumulators and this rank's traces (N, C, 4); frees
+        the accumulators"""
+        from .. import _lib as L
+        from ..utils.diagnostics import ess, split_rhat
+        s = self.sampler
+        diag = s.convergence_diagnostics()
+        s.disable_convergence_diagnostics()
+        # all ranks' traces at their global chain offsets, gathered with one SUM all-reduce of a zero-padded buffer
+        allt = torch.zeros(traces.shape[0], self.no_chains_total, 4, device=traces.device, dtype=torch.float64)
+        allt[:, s.chain_offset:s.chain_offset + self.no_chains] = traces
+        if torch.distributed.is_available() and torch.distributed.is_initialized() and torch.distributed.get_world_size() > 1:
+            torch.distributed.all_reduce(allt, op=torch.distributed.ReduceOp.SUM)
+        allt = allt.cpu().numpy()
+        cols = {'data': L.STAT_DATA, 'reg': L.STAT_REG, 'alpha': L.STAT_ALPHA, 'reg_energy': L.STAT_ENERGY}
+        diag['traces'] = {name: {'R_hat': split_rhat(allt[:, :, j].T), 'ESS': ess(allt[:, :, j].T)} for name, j in cols.items()}
+        if self.save_dir is not None and (not torch.distributed.is_initialized() or torch.distributed.get_rank() == 0):
+            import os
+            from ..logger import save_field_to_disk, save_im_to_disk
+            os.makedirs(self.save_dir, exist_ok=True)
+            sp = [float(x) for x in self.im_spacing]
+            save_field_to_disk(diag['displacement'].cpu(), os.path.join(self.save_dir, 'MCMC_R_hat_displacement.vtk'), sp)
+            save_im_to_disk(diag['im'][0].cpu(), os.path.join(self.save_dir, 'MCMC_R_hat_im.nii.gz'), sp)
+        return diag
 
     def _is_kept(self, sample_no):
         """reference trainer.py:414-415"""
