@@ -231,6 +231,28 @@ int irs_split_rhat_finish(const double* sw, const double* sb, int M, int n, cons
                           long long V, float* rhat, double* partials, unsigned int* counters, double* summary, void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------------ *
+ * Posterior of the warped segmentation (the reference has none): a per-voxel histogram of labels over every accumulated
+ * segmentation, kept in integers so that it is exact and independent of how samples are batched or split over GPUs.
+ * labels_host: 1..32 distinct non-zero int16 values (0 in the list: IRS_ERR_UNSUPPORTED; duplicates: IRS_ERR_BAD_ARG); every
+ * other voxel value is the class "other", which is never stored (its count is n - sum_l counts[l][v]).
+ *   irs_label_counts_update: counts (n_labels, V) ints += [seg[c][v] == labels[l]] summed over the C segmentations (C, V).
+ *     Zero counts before the first update.  No atomics: one thread owns each counts element.
+ *   irs_label_posterior: from counts of n >= 1 segmentations,
+ *     prob (n_labels, V) floats = (float)counts / (float)n;
+ *     majority (V) shorts = the label of the largest count among the n_labels + 1 classes; ties go to "other" (written 0),
+ *       then to the earlier entry of labels_host;
+ *     entropy (V) floats = -sum_k p_k ln p_k over the n_labels + 1 classes in nats (0 ln 0 = 0);
+ *     summary (n_labels, 3) long longs, exact: S = sum_v counts[l][v], O = the same over the voxels where seg_fixed == labels[l]
+ *       (0 when seg_fixed is NULL), U = #{v : 0 < counts[l][v] < n}.  Integer atomics per block: deterministic.
+ * Nothing synchronises with the host; both are graph-capturable.
+ * ------------------------------------------------------------------------------------------------------------------ */
+int irs_label_counts_update(const short* seg, int C, long long V, const int* labels_host, int n_labels, int* counts,
+                            void* stream);
+int irs_label_posterior(const int* counts, const int* labels_host, int n_labels, long long n, long long V,
+                        const short* seg_fixed, float* prob, short* majority, float* entropy, long long* summary,
+                        void* stream);
+
+/* ------------------------------------------------------------------------------------------------------------------ *
  * The fused SGLD transition -- replaces Trainer._SGLD_transition, trainer/trainer.py:291-356, for all chains of this
  * GPU, including the sequential per-chain GMM Adam step (trainer.py:316-327, 68-77; optimizers/adam_rate_decay.py),
  * the regulariser's hyper-parameter Adam step (trainer.py:353-354) and the plain-SGD state update (trainer.py:351).

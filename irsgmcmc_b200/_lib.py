@@ -123,6 +123,8 @@ SYMBOLS = {
     'irs_split_rhat_sums': (_i, [_vp, _vp, _i, _ll, _i, _vp, _vp]),
     'irs_split_rhat_between': (_i, [_vp, _i, _ll, _vp, _i, _vp, _vp]),
     'irs_split_rhat_finish': (_i, [_vp, _vp, _i, _i, _vp, _i, _ll, _vp, _vp, _vp, _vp, _vp]),
+    'irs_label_counts_update': (_i, [_vp, _i, _ll, _vp, _i, _vp, _vp]),
+    'irs_label_posterior': (_i, [_vp, _vp, _i, _ll, _ll, _vp, _vp, _vp, _vp, _vp, _vp]),
     'irs_sgld_partials_doubles': (_sz, [ctypes.POINTER(SgldConfig)]),
     'irs_sgld_step': (_i, [ctypes.POINTER(SgldConfig), ctypes.POINTER(SgldBuffers), _vp]),
     'irs_sgld_step_profile': (_i, [ctypes.POINTER(SgldConfig), ctypes.POINTER(SgldBuffers), _vp, _vp]),

@@ -405,6 +405,63 @@ def dice_counts(seg_a, seg_b, labels):
     return counts
 
 
+def _label_array(labels):
+    import ctypes
+    labels = [int(x) for x in labels]
+    return (ctypes.c_int * len(labels))(*labels), len(labels)
+
+
+def label_counts_update(seg, labels, counts):
+    """add the C int16 segmentations seg (C, 1, D, H, W) into counts (L, D, H, W) int32 in place: counts[l][v] += number of
+    chains whose voxel v carries labels[l] (1..32 distinct non-zero values; any other value is the class "other", not stored)"""
+    lib = _lib.load()
+    _lib.require_cuda(seg, counts)
+    if seg.dtype != torch.int16:
+        raise NotImplementedError('int16 segmentations only')
+    if counts.dtype != torch.int32:
+        raise NotImplementedError('int32 counts only')
+    C, V = seg.shape[0], seg[0].numel()
+    lab, L = _label_array(labels)
+    if counts.shape[0] != L or counts[0].numel() != V:
+        raise ValueError(f'counts must be ({L}, D, H, W) for {L} labels over the {V} voxels of a segmentation')
+    _lib.check(lib.irs_label_counts_update(_lib.ptr(seg), C, V, lab, L, _lib.ptr(counts), _lib.stream()))
+
+
+def label_posterior(counts, n, labels, seg_fixed=None):
+    """
+    The posterior of a segmentation from the label counts (L, D, H, W) int32 of n accumulated segmentations:
+      prob     (L, D, H, W) fp32   (float)counts / (float)n
+      majority (1, 1, D, H, W) int16  the most frequent of the L + 1 classes; ties go to "other" (0), then to the earlier label
+      entropy  (1, D, H, W) fp32   -sum_k p_k ln p_k over the L + 1 classes (nats)
+      summary  (L, 3) int64        per label: S = sum of the counts, O = the same inside seg_fixed == label (0 without
+                                   seg_fixed), U = voxels with 0 < count < n
+    S / n is the expected volume in voxels, 2 O / (S + n |F|) the soft Dice of the probability map.  seg_fixed: int16 volume of
+    the same D, H, W, or None.
+    """
+    lib = _lib.load()
+    _lib.require_cuda(counts, seg_fixed)
+    if counts.dtype != torch.int32:
+        raise NotImplementedError('int32 counts only')
+    if seg_fixed is not None and seg_fixed.dtype != torch.int16:
+        raise NotImplementedError('int16 segmentations only')
+    if counts.dim() != 4:
+        raise ValueError('counts must be (L, D, H, W)')
+    lab, L = _label_array(labels)
+    (D, H, W), V = counts.shape[1:], counts[0].numel()
+    if counts.shape[0] != L:
+        raise ValueError(f'counts has {counts.shape[0]} rows for {L} labels')
+    if seg_fixed is not None and seg_fixed.numel() != V:
+        raise ValueError(f'seg_fixed must hold the {V} voxels of the counts')
+    dev = counts.device
+    prob = torch.empty(L, D, H, W, device=dev, dtype=torch.float32)
+    majority = torch.empty(1, 1, D, H, W, device=dev, dtype=torch.int16)
+    entropy = torch.empty(1, D, H, W, device=dev, dtype=torch.float32)
+    summary = torch.empty(L, 3, device=dev, dtype=torch.int64)
+    _lib.check(lib.irs_label_posterior(_lib.ptr(counts), lab, L, int(n), V, _lib.ptr(seg_fixed), _lib.ptr(prob),
+                                       _lib.ptr(majority), _lib.ptr(entropy), _lib.ptr(summary), _lib.stream()))
+    return prob, majority, entropy, summary
+
+
 def average_surface_distance(seg_a, seg_b, labels, spacing, workspace_bytes=512 << 20):
     """float64 (C, n_labels) average surface distance of the structures seg_a == l and seg_b[c] == l (the reference's
     LabelContour + average Hausdorff distance, utils/util.py:171-176): inf when either is empty.  int16 label volumes (C or

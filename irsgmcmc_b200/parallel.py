@@ -1,7 +1,8 @@
 """
 Multi-GPU: chains shard by rank with no per-iteration communication (SURVEY.md section 8e).  The collectives are the
 merge of the per-rank Welford posterior moments and, when convergence diagnostics are requested, the partial sums of the split
-R-hat -- two sum all-reduces each (NCCL over NVLink on GPUs; gloo in CPU tests).
+R-hat -- two sum all-reduces each (NCCL over NVLink on GPUs; gloo in CPU tests) -- and, for the segmentation posterior, one sum
+all-reduce of the integer label counts.
 
 The reference has no distributed code at all; the quantity computed here is its calc_posterior_statistics
 (utils/util.py:114-120: mean and unbiased std over every kept sample of every chain).
@@ -52,6 +53,23 @@ def split_rhat_totals(n_seq_local, sums, between, group=None):
     sb = between(total[0], M)
     dist.all_reduce(sb, op=dist.ReduceOp.SUM, group=group)
     return M, total, sb
+
+
+def merge_label_counts(n_local, counts, group=None):
+    """
+    The label counts of the segmentation posterior (ops.label_counts_update) summed over the ranks of `group`: one SUM
+    all-reduce of one int32 buffer, the number of accumulated segmentations riding in front (padded to 4 ints so that the
+    counts stay 16-byte aligned).  Integer sums: the result does not depend on how the chains are split over ranks.
+    Returns (n_total, counts_total) as new tensors, identical on every rank; the local counts are left as they are, so sampling
+    can go on after a query.  One host read (n_total).
+    """
+    if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) == 1:
+        return int(n_local), counts.clone()
+    buf = torch.empty(4 + counts.numel(), device=counts.device, dtype=torch.int32)
+    buf[:4] = int(n_local)
+    buf[4:].view_as(counts).copy_(counts)
+    dist.all_reduce(buf, op=dist.ReduceOp.SUM, group=group)
+    return int(buf[0].item()), buf[4:].view_as(counts)
 
 
 def merge_moments(n_local, moments, group=None):

@@ -167,6 +167,8 @@ class SGLDSampler:
 
         # split-R-hat accumulators (enable_convergence_diagnostics): None while disabled
         self._rhat = None
+        # label counts of the segmentation posterior (enable_segmentation_posterior): None while disabled
+        self._segpost = None
 
     # ------------------------------------------------------------------------------------------------------------------
     def _make_config(self):
@@ -305,6 +307,9 @@ class SGLDSampler:
         if self._rhat is not None:   # convergence diagnostics enabled: their accumulators travel too
             r = self._rhat
             sd['rhat'] = {'N': r['N'], 'k': r['k'], 'mean': r['mean'].cpu(), 'm2': r['m2'].cpu()}
+        if self._segpost is not None:   # segmentation posterior enabled: its label counts travel too
+            p = self._segpost
+            sd['segpost'] = {'labels': list(p['labels']), 'n': p['n'], 'counts': p['counts'].cpu()}
         return sd
 
     @torch.no_grad()
@@ -327,6 +332,13 @@ class SGLDSampler:
             self._rhat['m2'].copy_(sd['rhat']['m2'])
         elif self._rhat is not None:
             self.enable_convergence_diagnostics(self._rhat['N'])
+        # the same for the segmentation posterior: enabled with the checkpoint's labels and counts, or restarted from zero
+        if 'segpost' in sd:
+            self.enable_segmentation_posterior(sd['segpost']['labels'])
+            self._segpost['n'] = int(sd['segpost']['n'])
+            self._segpost['counts'].copy_(sd['segpost']['counts'])
+        elif self._segpost is not None:
+            self.enable_segmentation_posterior(self._segpost['labels'])
 
     def set_noise(self, eps=None, jitter_unit=None):
         """explicit N(0,1) / U[0,1) numbers (C,3,D,H,W) instead of Philox: exact noise-on parity tests"""
@@ -511,14 +523,25 @@ class SGLDSampler:
     # ------------------------------------------------------------------------------------------------------------------
     # posterior moments
     # ------------------------------------------------------------------------------------------------------------------
-    def accumulate(self):
-        """fold the current sample of every chain into the running moments (kept-sample rule: trainer.py:414-430) and, when
-        convergence diagnostics are enabled, into the chain's split-R-hat sequence"""
+    def accumulate(self, seg_warped=None):
+        """fold the current sample of every chain into the running moments (kept-sample rule: trainer.py:414-430), when
+        convergence diagnostics are enabled into the chain's split-R-hat sequence, and when the segmentation posterior is
+        enabled the warped moving segmentation of every chain into its label counts: `seg_warped` (C,1,D,H,W) int16 if the
+        caller has it already (warp_segmentation() of the current transformations), else warped here.  Without the
+        segmentation posterior `seg_warped` is not used."""
         n3, n1 = 3 * self.V, self.V
         st = _lib.stream()
         if self._rhat is not None and self._rhat['k'] >= self._rhat['N']:
             raise RuntimeError(f'convergence diagnostics were enabled for {self._rhat["N"]} kept samples per chain: this is '
                                f'sample {self._rhat["k"] + 1} (enable_convergence_diagnostics again to start over)')
+        p = self._segpost
+        if p is not None:
+            if seg_warped is None:
+                seg_warped = self.warp_segmentation()
+            if seg_warped.dtype != torch.int16 or tuple(seg_warped.shape) != (self.C, 1, *self.dims) or \
+                    not seg_warped.is_cuda or not seg_warped.is_contiguous():
+                raise ValueError(f'seg_warped must be a contiguous ({self.C}, 1, {", ".join(map(str, self.dims))}) int16 '
+                                 f'CUDA tensor')
         _lib.check(self.lib.irs_welford_update(_lib.ptr(self.displacement), self.C, n3, float(self.n_kept),
                                                _lib.ptr(self.disp_mean), _lib.ptr(self.disp_m2), st))
         _lib.check(self.lib.irs_welford_update(_lib.ptr(self.im_warped), self.C, n1, float(self.n_kept),
@@ -534,6 +557,10 @@ class SGLDSampler:
                                                              self.V, half, float(count), _lib.ptr(r['mean']),
                                                              _lib.ptr(r['m2']), st))
             r['k'] = k + 1
+        if p is not None:
+            _lib.check(self.lib.irs_label_counts_update(_lib.ptr(seg_warped), self.C, self.V, p['host_labels'],
+                                                        len(p['labels']), _lib.ptr(p['counts']), st))
+            p['n'] += self.C
 
     def posterior_moments(self, group=None):
         """
@@ -616,3 +643,67 @@ class SGLDSampler:
                     'n_above_1.1': [int(x) for x in s[rows, 2]], 'n_voxels': int(self.n_mask)}
         return {'displacement': rhat[:3], 'im': rhat[3:], 'mask': {'displacement': part(slice(0, 3)), 'im': part(slice(3, 4))},
                 'n': n, 'M': M}
+
+    # ------------------------------------------------------------------------------------------------------------------
+    # posterior of the warped segmentation (per-voxel label histogram)
+    # ------------------------------------------------------------------------------------------------------------------
+    @torch.no_grad()
+    def enable_segmentation_posterior(self, labels):
+        """
+        Allocate (or reset) the label counts of the segmentation posterior: (L, D, H, W) int32 for the L = len(labels) labels
+        (1..32 distinct non-zero int16 values; every other value of the segmentation is the class "other") -- 4 L V bytes
+        whatever the number of chains, e.g. 126 MB for 15 labels at 128^3, 1.0 GB at 256^3.  accumulate() then also adds the
+        warped moving segmentation of every chain (one launch, no synchronisation; moments, split R-hat and chain states are
+        unchanged) and segmentation_posterior() gives the label probabilities, the majority labels and the entropy.
+        Needs a moving segmentation (int16).
+        """
+        if self.moving_seg is None:
+            raise ValueError('the segmentation posterior needs a moving segmentation (moving["seg"])')
+        if self.moving_seg.dtype != torch.int16:
+            raise NotImplementedError('the segmentation posterior needs an int16 moving segmentation')
+        labels = [int(x) for x in labels]
+        if not 1 <= len(labels) <= 32 or len(set(labels)) != len(labels) or 0 in labels or \
+                not all(-32768 <= x <= 32767 for x in labels):
+            raise ValueError(f'the segmentation posterior takes 1..32 distinct non-zero int16 labels, got {labels}')
+        p = self._segpost
+        if p is None or p['labels'] != labels:
+            self._segpost = None   # release the old counts first
+            counts = torch.zeros(len(labels), *self.dims, device=self.device, dtype=torch.int32)
+            self._segpost = {'labels': labels, 'host_labels': (ctypes.c_int * len(labels))(*labels), 'n': 0, 'counts': counts}
+        else:
+            p['n'] = 0
+            p['counts'].zero_()
+
+    def disable_segmentation_posterior(self):
+        """free the label counts; accumulate() no longer touches the segmentations"""
+        self._segpost = None
+
+    @property
+    def segmentation_posterior_enabled(self):
+        return self._segpost is not None
+
+    @torch.no_grad()
+    def segmentation_posterior(self, seg_fixed=None, group=None):
+        """
+        The posterior of the warped moving segmentation over every segmentation accumulated by ALL ranks of `group` (one SUM
+        all-reduce of the integer counts when torch.distributed is initialised, parallel.merge_label_counts; the local counts are
+        kept, so sampling can continue).  seg_fixed: int16 (1,1,D,H,W) for the overlap sums, or None.
+        Returns {'labels': list, 'n': number of segmentations (kept samples x chains),
+                 'probability': (L,D,H,W) fp32, 'majority': (1,1,D,H,W) int16, 'entropy': (1,D,H,W) fp32 device tensors,
+                 'summary': (L,3) int64 device tensor, per label: S = sum of the counts (S / n = expected volume in voxels),
+                            O = the same inside seg_fixed == label (0 without seg_fixed; 2 O / (S + n |F|) = soft Dice),
+                            U = voxels with 0 < count < n}  (ops.label_posterior).
+        """
+        from . import ops
+        from .parallel import merge_label_counts
+        p = self._segpost
+        if p is None:
+            raise RuntimeError('the segmentation posterior is not enabled (enable_segmentation_posterior(labels) before sampling)')
+        n, counts = merge_label_counts(p['n'], p['counts'], group)
+        if n < 1:
+            raise RuntimeError('the segmentation posterior has no accumulated segmentation yet')
+        if seg_fixed is not None:
+            seg_fixed = seg_fixed.to(self.device).contiguous()
+        prob, majority, entropy, summary = ops.label_posterior(counts, n, p['labels'], seg_fixed)
+        return {'labels': list(p['labels']), 'n': n, 'probability': prob, 'majority': majority, 'entropy': entropy,
+                'summary': summary}

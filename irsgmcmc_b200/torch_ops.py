@@ -22,6 +22,7 @@ which calls the adjoint op (the closed forms of SURVEY Appendix A, no scatter at
     calc_no_non_diffeomorphic_voxels (utils/util.py:209-212)              irsgmcmc::log_det_jacobian
     calc_DSC_GPU (utils/util.py:123-148)                                  irsgmcmc::dice_counts
     calc_metrics, ASD part (utils/util.py:171-176)                        irsgmcmc::average_surface_distance
+    (no reference counterpart: posterior of the warped segmentation)      irsgmcmc::label_counts_update (in place), ::label_posterior
     Trainer._SGLD_transition (trainer/trainer.py:291-356)                 irsgmcmc::sgld_step (the fused transition, in place)
 
 The drop-in modules (utils/, model/) and the fused sampler use the same launchers; this module adds the dispatcher-visible
@@ -418,6 +419,33 @@ def _(seg_a, seg_b, labels, spacing):
     return seg_b.new_empty(seg_b.shape[0], len(labels), dtype=torch.float64)
 
 
+# ---- posterior of the warped segmentation ---------------------------------------------------------------------------------
+@torch.library.custom_op(f'{_NS}::label_counts_update', mutates_args=('counts',), device_types='cuda')
+def label_counts_update(seg: Tensor, labels: Sequence[int], counts: Tensor) -> None:
+    """counts (L, D, H, W) int32 += per label, the number of the C int16 segmentations seg (C, 1, D, H, W) carrying it"""
+    ops.label_counts_update(seg.contiguous(), list(labels), counts)
+
+
+@label_counts_update.register_fake
+def _(seg, labels, counts):
+    return None
+
+
+@_op('label_posterior')
+def label_posterior(counts: Tensor, n: int, labels: Sequence[int], seg_fixed: Optional[Tensor]) -> Tuple[Tensor, Tensor, Tensor,
+                                                                                                         Tensor]:
+    """(probability (L, D, H, W) fp32, majority label (1, 1, D, H, W) int16, entropy (1, D, H, W) fp32, summary (L, 3) int64)
+    from the label counts of n segmentations (ops.label_posterior)"""
+    return ops.label_posterior(counts.contiguous(), n, list(labels), None if seg_fixed is None else seg_fixed.contiguous())
+
+
+@label_posterior.register_fake
+def _(counts, n, labels, seg_fixed):
+    L, D, H, W = counts.shape
+    return (counts.new_empty(L, D, H, W, dtype=torch.float32), counts.new_empty(1, 1, D, H, W, dtype=torch.int16),
+            counts.new_empty(1, D, H, W, dtype=torch.float32), counts.new_empty(L, 3, dtype=torch.int64))
+
+
 # ---- the fused transition -------------------------------------------------------------------------------------------------------------
 _SAMPLERS = {}
 
@@ -449,4 +477,4 @@ def _(v, hyper, stats, handle, n):
 OPS = ('warp3d', 'warp3d_bwd_grid', 'warp3d_nearest', 'svf_exp', 'svf_exp_bwd', 'sobolev_smooth', 'lcc_normalise',
        'lcc_normalise_bwd', 'reg_energy', 'reg_energy_grad', 'ffd', 'ffd_adjoint', 'langevin_proposal', 'gmm_log_pdf',
        'gmm_log_pdf_param_grads', 'vd_factor', 'welford_update', 'welford_std', 'split_rhat', 'log_det_jacobian', 'dice_counts', 'average_surface_distance',
-       'sgld_step')
+       'label_counts_update', 'label_posterior', 'sgld_step')

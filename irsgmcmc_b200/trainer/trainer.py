@@ -408,7 +408,8 @@ class Trainer:
         return self.var_params_q_v, m, history
 
     @torch.no_grad()
-    def _test_VI(self, var_params_q_v=None, no_samples=None, modules=None, speed_test_samples=100, with_ASD=True):
+    def _test_VI(self, var_params_q_v=None, no_samples=None, modules=None, speed_test_samples=100, with_ASD=True,
+                 with_seg_posterior=False):
         """
         evaluation of the fitted q(v) (reference trainer.py:226-289): `no_samples_VI_test` draws from q(v) -> Sobolev smoothing ->
         transformation -> number of folded voxels + log det J, warped image and segmentation, ASD / DSC per structure, the sample on
@@ -417,6 +418,9 @@ class Trainer:
         host buffer for torch.std; here they are folded into Welford moments on the device (same unbiased result).
         Returns {'no_non_diffeomorphic_voxels': [S], 'DSC': (S, structures), 'ASD': (S, structures) | str, 'mean', 'std_dev' (3,D,H,W),
         'displacement_mu', 'im_moving_warped_mu', 'samples_per_sec'}.
+        with_seg_posterior=True (needs structures_dict, both segmentations and S >= 1, else ValueError) adds 'seg_posterior',
+        the posterior of the warped moving segmentation over the S draws (n = S), with the entries of _run_MCMC's; with
+        save_dir, VI_seg_majority.nii.gz and VI_seg_entropy.nii.gz.
         """
         from .. import ops
         from ..utils import SobolevGrad, calc_metrics
@@ -429,6 +433,12 @@ class Trainer:
         moving = {k: v.to(dev) for k, v in self.moving.items()}
         seg_fixed = self.fixed['seg'].to(dev) if 'seg' in self.fixed else None
         with_seg = bool(self.structures_dict) and seg_fixed is not None and 'seg' in moving
+        if with_seg_posterior:
+            if not with_seg or S < 1:
+                raise ValueError('with_seg_posterior=True needs structures_dict, fixed and moving segmentations and at least '
+                                 'one sample')
+            seg_labels = [int(x) for x in self.structures_dict.values()]
+            seg_counts = torch.zeros(len(seg_labels), *self.dims, device=dev, dtype=torch.int32)
         transformation_module, registration_module, diff_op = m['transformation_module'], m['registration_module'], m['reg_loss'].diff_op
 
         def register(v):
@@ -451,6 +461,8 @@ class Trainer:
                 else:
                     DSC = calc_DSC_GPU(1, seg_fixed, seg_moving_warped, self.structures_dict)
                 dsc.append(DSC[0])
+                if with_seg_posterior:
+                    ops.label_counts_update(seg_moving_warped.contiguous(), seg_labels, seg_counts)
             if self.save_dir is not None:
                 from ..logger import save_sample
                 save_sample(self.save_dir, self.im_spacing, test_sample_no, im_moving_warped, displacement, log_det_J, model='VI')
@@ -465,6 +477,11 @@ class Trainer:
         result = {'no_non_diffeomorphic_voxels': folded, 'DSC': np.asarray(dsc), 'mean': mean, 'std_dev': std_dev,
                   'ASD': np.asarray(asd) if (with_seg and with_ASD) else 'unavailable: no segmentations / structures, or with_ASD=False',
                   'displacement_mu': displacement_mu, 'im_moving_warped_mu': im_moving_warped_mu, 'n': count}
+        if with_seg_posterior:
+            prob, majority, entropy, summary = ops.label_posterior(seg_counts, S, seg_labels, seg_fixed.contiguous())
+            post = {'labels': seg_labels, 'n': S, 'probability': prob, 'majority': majority, 'entropy': entropy,
+                    'summary': summary}
+            result['seg_posterior'] = self._seg_posterior(post, with_ASD, 'VI')
         if speed_test_samples:   # reference trainer.py:275-289
             torch.cuda.synchronize()
             t0 = time.perf_counter()
@@ -529,7 +546,8 @@ class Trainer:
         return loss_terms, out, aux
 
     # -- the loop around it (reference trainer.py:358-476) -------------------------------------------------------------
-    def _run_MCMC(self, data_loss=None, reg_loss=None, speed_test_iters=100, with_ASD=False, with_R_hat=False):
+    def _run_MCMC(self, data_loss=None, reg_loss=None, speed_test_iters=100, with_ASD=False, with_R_hat=False,
+                  with_seg_posterior=False):
         """burn-in + sampling; returns {'mean','std_dev', 'im_mean','im_std', 'n', 'DSC', 'ASD', 'no_non_diffeomorphic_voxels',
         'samples_per_sec'}; posterior statistics are over the kept samples of ALL ranks.  'ASD' (average surface distance,
         reference utils/util.py:171-176 through SimpleITK on the host): with_ASD=True computes it per kept sample on the device
@@ -546,10 +564,22 @@ class Trainer:
         take 64 C V bytes while the run lasts.  In hyper_mode='reference' (the default) the chains share the mixture and
         regulariser parameters that they step in turn, so they are not independent: R-hat is still computed, but its reading
         as a check between independent chains holds for hyper_mode 'per_chain' / 'frozen' (Trainer(sampler_config=...)).
-        With with_R_hat=False nothing of this runs and the result is unchanged."""
+        With with_R_hat=False nothing of this runs and the result is unchanged.
+
+        with_seg_posterior=True (needs structures_dict and fixed and moving segmentations, else ValueError) adds
+        'seg_posterior', the posterior of the warped moving segmentation over every kept sample of every chain of every rank
+        (SGLDSampler.enable_segmentation_posterior over the structures' labels; the segmentation warped for the Dice scores is
+        folded into the label counts): the maps 'probability' (L,D,H,W), 'majority' (1,1,D,H,W) int16, 'entropy' (1,D,H,W),
+        'labels', 'n', 'summary' (L,3) int64, and 'structures' {name: {'expected_volume' (voxels), 'uncertain_voxels',
+        'soft_DSC', 'DSC_majority'[, 'ASD_majority' with with_ASD]}}.  With save_dir, MCMC_seg_majority.nii.gz and
+        MCMC_seg_entropy.nii.gz are written as well.  With with_seg_posterior=False nothing of this runs."""
         if self.SGLD_params is None:
             self._SGLD_init()
         s = self.sampler
+        if with_seg_posterior:
+            if not (self.structures_dict and s.moving_seg is not None and 'seg' in self.fixed):
+                raise ValueError('with_seg_posterior=True needs structures_dict and fixed and moving segmentations')
+            s.enable_segmentation_posterior(list(self.structures_dict.values()))
         if not self._gmm_pushed:
             if data_loss is not None or reg_loss is not None:
                 self._push_hyper(data_loss, reg_loss)
@@ -576,11 +606,8 @@ class Trainer:
             s.step(nxt - it)
             it = nxt
             if self._is_kept(it):
-                s.accumulate()
-                if with_R_hat:
-                    traces[k_kept].copy_(s.stats[:, :4])
-                    k_kept += 1
                 T = s.transformation()
+                seg_w = None
                 if self.structures_dict and s.moving_seg is not None and 'seg' in self.fixed:
                     seg_w = s.warp_segmentation(transformation=T)
                     seg_f = self.fixed['seg'].to(s.device).expand(self.no_chains, -1, -1, -1, -1)
@@ -588,6 +615,12 @@ class Trainer:
                     if with_ASD:
                         from ..utils.util import calc_metrics
                         asd.append(calc_metrics(seg_f, seg_w, self.structures_dict, self.im_spacing, no_samples=self.no_chains)[0])
+                # after the segmentation warp, so that the segmentation posterior reuses it; the transformation and the warp
+                # read what accumulate() reads and write nothing it reads, so the order changes no result
+                s.accumulate(seg_warped=seg_w)
+                if with_R_hat:
+                    traces[k_kept].copy_(s.stats[:, :4])
+                    k_kept += 1
                 n_folded, log_det_J = calc_no_non_diffeomorphic_voxels(T, diff_op)
                 folded.append(n_folded)
                 if self.save_dir is not None:
@@ -611,6 +644,10 @@ class Trainer:
                                               'distance transform kernels; parity with SimpleITK unpinned)'}
         if with_R_hat:
             result['R_hat'] = self._R_hat(traces)
+        if with_seg_posterior:
+            post = s.segmentation_posterior(seg_fixed=self.fixed['seg'])
+            s.disable_segmentation_posterior()
+            result['seg_posterior'] = self._seg_posterior(post, with_ASD, 'MCMC')
         if self.save_dir is not None and (not torch.distributed.is_initialized() or torch.distributed.get_rank() == 0):
             # MCMC_sample_{mean,std_dev}[_masked].vtk like the reference (trainer.py:457-460, logger/logger.py:110-131)
             from ..logger import save_displacement_mean_and_std_dev
@@ -651,6 +688,37 @@ class Trainer:
             save_field_to_disk(diag['displacement'].cpu(), os.path.join(self.save_dir, 'MCMC_R_hat_displacement.vtk'), sp)
             save_im_to_disk(diag['im'][0].cpu(), os.path.join(self.save_dir, 'MCMC_R_hat_im.nii.gz'), sp)
         return diag
+
+    def _seg_posterior(self, post, with_ASD, model):
+        """the 'seg_posterior' entry of _run_MCMC / _test_VI(with_seg_posterior=True) from the dict of
+        SGLDSampler.segmentation_posterior (computed with the fixed segmentation): per structure the expected volume S / n, the
+        uncertain voxels U, the soft Dice 2 O / (S + n |F|) of the probability map and the Dice (and ASD) of the majority
+        segmentation; {model}_seg_majority.nii.gz and {model}_seg_entropy.nii.gz in save_dir"""
+        from .. import ops
+        from ..utils.util import calc_ASD_GPU
+        n, labels, majority = post['n'], post['labels'], post['majority']
+        seg_f = self.fixed['seg'].to(majority.device).contiguous()
+        summary = post['summary'].cpu().numpy()
+        fixed_sizes = ops.dice_counts(seg_f, seg_f, labels)[0, :, 0].cpu().numpy()   # |F_l|
+        dsc = calc_DSC_GPU(1, seg_f, majority, self.structures_dict)[0]
+        asd = calc_ASD_GPU(1, seg_f, majority, self.structures_dict, self.im_spacing)[0] if with_ASD else None
+        structures = {}
+        for j, name in enumerate(self.structures_dict):
+            S, O, U = (int(x) for x in summary[j])
+            den = S + n * int(fixed_sizes[j])
+            structures[name] = {'expected_volume': S / n, 'uncertain_voxels': U,
+                                'soft_DSC': 2.0 * O / den if den else float('nan'), 'DSC_majority': float(dsc[j])}
+            if with_ASD:
+                structures[name]['ASD_majority'] = float(asd[j])
+        post['structures'] = structures
+        if self.save_dir is not None and (not torch.distributed.is_initialized() or torch.distributed.get_rank() == 0):
+            import os
+            from ..logger import save_im_to_disk
+            os.makedirs(self.save_dir, exist_ok=True)
+            sp = [float(x) for x in self.im_spacing]
+            save_im_to_disk(majority[0, 0].cpu(), os.path.join(self.save_dir, f'{model}_seg_majority.nii.gz'), sp)
+            save_im_to_disk(post['entropy'][0].cpu(), os.path.join(self.save_dir, f'{model}_seg_entropy.nii.gz'), sp)
+        return post
 
     def _is_kept(self, sample_no):
         """reference trainer.py:414-415"""
