@@ -1,7 +1,6 @@
 // irs_data.cu -- data term: LCC normalisation as separable box filters over shared-memory tiles with halos, its adjoint,
 // the Gaussian-mixture log-density with warp-shuffle reductions, virtual decimation.
 // (reference model/loss.py:87-114, utils/util.py:330-347,446-485, trainer/trainer.py:68-77,316-327)
-#include <cstdlib>
 #include <type_traits>
 
 #include "irs_kernels.cuh"
@@ -180,10 +179,6 @@ box_march_kernel(const float* __restrict__ in0, const float* __restrict__ in1, c
 }
 
 static int box_seg_len(IrsDims d, int C) {
-    if (const char* e = getenv("IRS_BOX_SEG")) {   // development override
-        const int v = atoi(e);
-        if (v >= 1) return v < d.D ? v : d.D;
-    }
     // enough CTAs for ~2 waves of the 148 x 8 resident slots, segments no shorter than 8 planes (halo 2S per segment)
     const long long tiles = (long long)((d.W + TX - 1) / TX) * ((d.H + TY - 1) / TY) * C;
     int len = d.D;
@@ -766,14 +761,9 @@ masked_moments_kernel(const float* __restrict__ z, const unsigned char* __restri
 }  // namespace
 
 int irs_data_blocks(IrsDims d) {
-    static int cap = 0;   // development override
-    if (cap == 0) {
-        cap = -1;
-        if (const char* e = getenv("IRS_DATA_BLOCKS")) { const int v = atoi(e); if (v >= 1) cap = v; }
-    }
     // 4 CTAs per SM x 148 SMs: enough loads in flight, short final reduction; 2 per SM up to 128^3, where the final
     // reduction over the blocks is a visible part of these latency-bound kernels (measured 48 vs 51 us for the mixture step)
-    const int limit = cap > 0 ? cap : (d.V() <= 128ll * 128 * 128 ? 296 : 592);
+    const int limit = d.V() <= 128ll * 128 * 128 ? 296 : 592;
     long long b = (d.V() + 255) / 256;
     return (int)(b < limit ? b : limit);
 }

@@ -102,6 +102,9 @@ int irs_launch_langevin(const float* v, const float* sigma, long long sigma_cs, 
 int irs_launch_smooth3(const float* in, float* work, float* out, const IrsTaps& taps, int C, IrsDims d,
                        cudaStream_t st);
 // out = S * (v + coef sigma eps); work: (C,3,V) scratch
+// irs_langevin_fused: whether the state grid d and the tap count let irs_launch_langevin_smooth3 fuse the noise with the x / y
+// passes (two launches instead of four); it also needs 16-byte aligned fields and sigma_cs % 4 == 0
+bool irs_langevin_fused(IrsDims d, int n_taps);
 int irs_launch_langevin_smooth3(const float* v, const float* sigma, long long sigma_cs, float coef, IrsRng rng, float* work,
                                 float* out, const IrsTaps& taps, int C, IrsDims d, cudaStream_t st);
 int irs_launch_reg_energy(const float* v, double* energy, long long energy_stride, double* partials,

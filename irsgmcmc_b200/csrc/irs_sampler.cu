@@ -5,7 +5,6 @@
 // factors, mixture / regulariser hyper-parameters and their Adam state, the Philox offset) stays in device memory, so
 // the sequence has no host synchronisation and can be captured in a CUDA graph and replayed.
 #include <cstdint>
-#include <cstdlib>
 
 #include "irs_kernels.cuh"
 
@@ -135,22 +134,12 @@ int check_config(const irs_sgld_config* c) {
 }
 
 inline bool has_ffd(const irs_sgld_config* c) { return c->ffd_cps[0] > 0; }
-// mirrors the choice of irs_launch_langevin_smooth3 (the state grid: the control grid with the FFD); pointer alignment is assumed
-inline bool langevin_fused(const irs_sgld_config* c) {
-    static int env = -1;
-    if (env < 0) { const char* e = getenv("IRS_LANGEVIN_FUSED"); env = (e && atoi(e) == 0) ? 0 : 1; }
-    const int W = has_ffd(c) ? c->ffd_grid[2] : c->W;
-    return env == 1 && W % 4 == 0 && (c->n_taps == 3 || c->n_taps == 5 || c->n_taps == 7);
-}
 // one persistent launch for the mixture step of all chains (irs_launch_gmm_chain_walk) instead of two launches per chain.
 // Always for the chain-parallel hyper modes.  In the reference mode (chains in order on the shared mixture) the walk wins where
 // a chain is small and the two launches are pure latency (measured, 64 chains: 64^3 1.45 vs 1.77 ms; 128^3 3.13 vs 2.56 ms --
-// there one CTA per SM under-fills the machine), hence the volume threshold.  IRS_GMM_WALK=0 / 1 forces a side (development).
+// there one CTA per SM under-fills the machine), hence the volume threshold.
 inline bool gmm_walk_enabled(const irs_sgld_config* c) {
-    static int env = -2;
-    if (env == -2) { const char* e = getenv("IRS_GMM_WALK"); env = e ? (atoi(e) != 0 ? 1 : 0) : -1; }
     if (c->hyper_mode != IRS_HYPER_REFERENCE) return true;
-    if (env >= 0) return env == 1;
     return (long long)c->D * c->H * c->W <= 96LL * 96 * 96;
 }
 // the grid the chain state lives on: the control grid with the FFD, the image grid otherwise
@@ -173,8 +162,9 @@ extern "C" size_t irs_sgld_partials_doubles(const irs_sgld_config* cfg) {
 
 extern "C" int irs_sgld_launches_per_step(const irs_sgld_config* c) {
     if (check_config(c) != IRS_OK) return -1;
-    int n = 1;                                   // langevin (fused with the x / y smoothing when the field can be vectorised)
-    n += c->n_taps > 0 ? (langevin_fused(c) ? 1 : 3) : 0;   // Sobolev: z pass only / z, y, x
+    int n = 1;                                   // langevin (fused with the x / y smoothing when the field can be vectorised;
+                                                 // pointer alignment is assumed)
+    n += c->n_taps > 0 ? (irs_langevin_fused(state_dims(c), c->n_taps) ? 1 : 3) : 0;   // Sobolev: z pass only / z, y, x
     n += (c->W % 4 == 0 && !has_ffd(c)) ? 0 : 1; // regulariser energy (an epilogue of the first squaring step otherwise)
     n += has_ffd(c) ? 6 : 0;                     // B-spline FFD: three axis passes forward, three for the adjoint
     n += c->svf_steps;                           // scaling and squaring

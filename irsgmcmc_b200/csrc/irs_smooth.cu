@@ -1,7 +1,6 @@
 // irs_smooth.cu -- Langevin proposal, Sobolev smoothing, diffusion regulariser, preconditioned SGD update
 // (reference utils/functions.py:76-109, utils/util.py:48-58,394-404, utils/diff_op.py:78-96, model/loss.py:152-161,
 //  trainer/trainer.py:351)
-#include <cstdlib>
 #include <mutex>
 
 #include "irs_kernels.cuh"
@@ -188,8 +187,8 @@ langevin_vec_kernel(const float* __restrict__ v, const float* __restrict__ sigma
 // out.  The z pass that follows is the only other pass: 12 + 12 (+ halo) read, 12 written here, 12 + 12 there, instead of four
 // passes of 24 B.  Separable smoothing passes commute (replicate padding acts per axis), so x, y, z instead of the reference's
 // z, y, x changes the result at rounding level only (checked against the oracle at 1e-5 like before).
-template <int NT, int THREADS, int MINB>
-__global__ void __launch_bounds__(THREADS, MINB)
+template <int NT>
+__global__ void __launch_bounds__(512, 2)
 langevin_xy_kernel(const float* __restrict__ v, const float* __restrict__ sigma, long long sigma_cs, float coef, IrsRng rng,
                    float* __restrict__ out, IrsTaps taps, int TY, IrsDims d) {
     extern __shared__ __align__(16) float S[];   // [3][R][W], R = TY + 2 s
@@ -285,15 +284,11 @@ template <int NT>
 static int launch_langevin_xy_nt(const float* v, const float* sigma, long long sigma_cs, float coef, const IrsRng& rng,
                                  float* work, float* out, const IrsTaps& taps, int C, IrsDims d, cudaStream_t st) {
     constexpr int s = (NT - 1) / 2;
-    static int ty_env = -1, t_env = -1;
-    if (ty_env < 0) { const char* e = getenv("IRS_LANGEVIN_TY"); ty_env = e ? atoi(e) : 0; }
-    if (t_env < 0) { const char* e = getenv("IRS_LANGEVIN_T"); t_env = e ? atoi(e) : 0; }
-    int TY = ty_env > 0 ? ty_env : 32;
+    int TY = 32;
     while (TY > 8 && (size_t)3 * (TY + 2 * s) * d.W * 4 > 100 * 1024) TY -= 8;
     if (TY > d.H) TY = d.H;
     const size_t smem = (size_t)3 * (TY + 2 * s) * d.W * 4;
     if (smem > 200 * 1024) return IRS_ERR_UNSUPPORTED;
-    const bool small_cta = t_env == 256;
     static std::mutex mu;
     static bool ready[64] = {};
     {
@@ -301,16 +296,13 @@ static int launch_langevin_xy_nt(const float* v, const float* sigma, long long s
         int dev = 0;
         cudaGetDevice(&dev);
         if (!ready[dev & 63]) {
-            cudaError_t e = cudaFuncSetAttribute(langevin_xy_kernel<NT, 512, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-            if (e == cudaSuccess)
-                e = cudaFuncSetAttribute(langevin_xy_kernel<NT, 256, 4>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+            cudaError_t e = cudaFuncSetAttribute(langevin_xy_kernel<NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
             if (e != cudaSuccess) return (int)e;
             ready[dev & 63] = true;
         }
     }
     dim3 grid((unsigned)(((d.H + TY - 1) / TY) * d.D), C);
-    if (small_cta) langevin_xy_kernel<NT, 256, 4><<<grid, 256, smem, st>>>(v, sigma, sigma_cs, coef, rng, work, taps, TY, d);
-    else langevin_xy_kernel<NT, 512, 2><<<grid, 512, smem, st>>>(v, sigma, sigma_cs, coef, rng, work, taps, TY, d);
+    langevin_xy_kernel<NT><<<grid, 512, smem, st>>>(v, sigma, sigma_cs, coef, rng, work, taps, TY, d);
     dim3 vgrid((unsigned)((d.V() / 4 + 255) / 256), C * 3);
     smooth_axis_vec_kernel<2, NT><<<vgrid, 256, 0, st>>>(work, out, taps, d);
     return (int)cudaGetLastError();
@@ -583,14 +575,16 @@ int irs_launch_smooth3(const float* in, float* work, float* out, const IrsTaps& 
     return (int)cudaGetLastError();
 }
 
+bool irs_langevin_fused(IrsDims d, int n_taps) {   // the last term: the smallest tile (8 rows + halo) fits in 200 KB
+    return d.W % 4 == 0 && (n_taps == 3 || n_taps == 5 || n_taps == 7) && (size_t)3 * (8 + n_taps - 1) * d.W * 4 <= 200 * 1024;
+}
+
 // Langevin proposal + separable smoothing: two kernels (noise + x + y on shared-memory rows, then z) when the field can be
-// vectorised, the four-pass sequence otherwise.  IRS_LANGEVIN_FUSED=0 keeps the four passes (development switch).
+// vectorised, the four-pass sequence otherwise.
 int irs_launch_langevin_smooth3(const float* v, const float* sigma, long long sigma_cs, float coef, IrsRng rng, float* work,
                                 float* out, const IrsTaps& taps, int C, IrsDims d, cudaStream_t st) {
-    static int fused = -1;
-    if (fused < 0) { const char* e = getenv("IRS_LANGEVIN_FUSED"); fused = (e && atoi(e) == 0) ? 0 : 1; }
-    if (fused && vec_ok(d, v, sigma, out, rng.explicit_values) && vec_ok(d, work) && (sigma_cs % 4) == 0 &&
-        (taps.n == 3 || taps.n == 5 || taps.n == 7) && (size_t)3 * (8 + taps.n - 1) * d.W * 4 <= 200 * 1024) {
+    if (irs_langevin_fused(d, taps.n) && vec_ok(d, v, sigma, out, rng.explicit_values) && vec_ok(d, work) &&
+        (sigma_cs % 4) == 0) {
         switch (taps.n) {
             case 3: return launch_langevin_xy_nt<3>(v, sigma, sigma_cs, coef, rng, work, out, taps, C, d, st);
             case 5: return launch_langevin_xy_nt<5>(v, sigma, sigma_cs, coef, rng, work, out, taps, C, d, st);

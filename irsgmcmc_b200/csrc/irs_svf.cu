@@ -14,14 +14,12 @@
 //
 // Kernels in this file, fastest first; the choice between them is made on the device from max|u_k| (no host sync):
 //   svf_step_fwd_tma_kernel    forward step, TMA plane ring (max|u| < 1 bound; otherwise its in-kernel ring fallback)
-//   svf_step_bwd_tma2_kernel   adjoint step, TMA rings + per-source records, two targets per thread (the default)
-//   svf_step_bwd_tma_kernel    the same with one target per thread (IRS_BWD_NT=1)
+//   svf_step_bwd_tma2_kernel   adjoint step, TMA rings + per-source records, two targets per thread
 //   svf_step_fwd_tile_kernel / svf_step_bwd_tile_kernel   shared-memory rings fed by ordinary loads: row pitches the TMA
 //                              unit cannot address (W % 4 != 0), and steps with 1 <= max|u| < 2 inside the TMA kernels
 //   irs_body_svf_fwd / irs_body_svf_bwd, svf_step_bwd_scatter_kernel   global gathers / atomic scatter for larger radii
 #include <cstdlib>
 #include <mutex>
-#include <type_traits>
 
 #include "irs_kernels.cuh"
 #include "irs_bodies.cuh"
@@ -271,10 +269,6 @@ __device__ __forceinline__ float2 fmul2(float2 a, float2 b) {
 // scalar x pair (+ pair): ptxas folds the duplicated scalar into the .F32 broadcast operand of FFMA2 / FMUL2
 __device__ __forceinline__ float2 ffma2s(float s, float2 b, float2 c) { return ffma2(make_float2(s, s), b, c); }
 __device__ __forceinline__ float2 fmul2s(float s, float2 b) { return fmul2(make_float2(s, s), b); }
-
-#ifndef IRS_BWD_V2
-#define IRS_BWD_V2 1   // adjoint consumer: straight-line path for gradient-carrying neighbourhoods, z components of the two
-#endif                 // targets packed (FFMA2), cheaper row flags (0 = the round-1 consumer, kept for A/B timing)
 
 // position term of the adjoint: sum_c g_c * grad trilinear[u_c](p).  Interpolation is linear in the corner values, so
 // the three components are combined at the eight corners first (w = g . u) and ONE gradient is interpolated.
@@ -712,12 +706,8 @@ __device__ __forceinline__ float svf_fwd_tma_body(const CUtensorMap* tmap, const
 // Row pitch of the forward step's plane boxes.  64 floats (a multiple of the 32 banks): all rows alias the same banks, so lanes whose
 // cells lie in different rows do not collide as long as neighbouring lanes pick the same column offset -- measured 0.2146 -> 0.2112 ms
 // for the 12 steps on the benchmark's rank-0 draw and 0.2498 -> 0.2357 ms on a typical draw, although the unit moves 60 % more bytes
-// per plane than with the tight pitch of 40 (IRS_FWD_BW=40 rebuilds that variant).  The adjoint keeps 40: at 64 its two rings no
-// longer fit twice per SM.
-#ifndef IRS_FWD_BW
-#define IRS_FWD_BW 64
-#endif
-constexpr int FWD_BW = IRS_FWD_BW;
+// per plane than with the tight pitch of 40.  The adjoint keeps 40: at 64 its two rings no longer fit twice per SM.
+constexpr int FWD_BW = 64;
 constexpr size_t svf_fwd_tma_smem() { return sizeof(float) * TMA_NS * TmaRing<FWD_BW>::SS + 8 * TMA_NS; }
 
 // out-of-line fallbacks of the TMA forward kernel: their register pressure stays out of the main path
@@ -732,7 +722,8 @@ constexpr size_t svf_fwd_tile_smem_compact(int R) {
 
 // maxabs_prev = max |u_{k-1}| of the previous step (nullptr for the first): |u_k| <= 2 max |u_{k-1}|, so the TMA ring is
 // taken when that bound is below three voxels (see `small` below), the wider non-TMA ring otherwise
-// CTAS = resident CTAs per SM the kernel is compiled for (register cap 65536 / 256 / CTAS).  ENERGY (first step only):
+// Compiled for 5 resident CTAs per SM (register cap 65536 / 256 / 5): measured at 128^3, 4 -> 0.212 ms, 5 -> 0.200 ms,
+// 6 -> 0.208 ms for the 12 forward steps.  ENERGY (first step only):
 // also reduces the regulariser energy of the input field per chain -- block sums in double, partials[blockIdx.x], the
 // last block of the chain adds them in block order (deterministic) -> energy[chain * energy_stride].
 struct IrsEnergyOut {
@@ -742,8 +733,8 @@ struct IrsEnergyOut {
     unsigned int* counters;  // one per chain, zero on entry, reset on exit
 };
 
-template <int CTAS, bool ENERGY>
-__global__ void __launch_bounds__(TILE_T, CTAS)
+template <bool ENERGY>
+__global__ void __launch_bounds__(TILE_T, 5)
 svf_step_fwd_tma_kernel(const __grid_constant__ CUtensorMap tmap, const float* __restrict__ in_all, float in_scale,
                         float* __restrict__ out_all, const float* __restrict__ maxabs_prev, float* __restrict__ maxabs,
                         int seg_len, IrsDims d, IrsEnergyOut eo) {
@@ -781,266 +772,17 @@ svf_step_fwd_tma_kernel(const __grid_constant__ CUtensorMap tmap, const float* _
 // ---- adjoint step ------------------------------------------------------------------------------------------------------
 // Per source plane s the CTA first turns every source voxel of the tile + halo into a RECORD
 //     { cx, cy, g0, g1 } { g2, wz_0, wz_1, wz_2 }                 two 128-bit shared-memory words (in two arrays)
-// where (cx, cy, cz) = clamp(s + u(s)) - s is the source's sub-voxel offset, g = dL/du_{k+1}(s), and wz_b is its hat
-// weight onto the target plane whose index is congruent to b modulo 3 (planes s-1, s, s+1 in rotating order).  A target
-// then needs, per in-plane neighbour, two LDS.128, two weight ops, four products and six FMAs (three of them packed) -- the
-// z weights and the border clamps are paid once per source instead of nine times.  The nine accumulators (3 target
-// planes x 3 components) never move: the loop is unrolled by three and the plane that completes is selected at compile
-// time.  (A 12-float record holding the nine products wz_b * g_c saves four instructions per neighbour but costs a third
+// where (cx, cy, cz) = clamp(s + u(s)) - s is the source's sub-voxel offset, g = dL/du_{k+1}(s), and wz_0..2 are its hat
+// weights onto the target planes s-1, s and s+1.  A target then needs, per in-plane neighbour, two LDS.128, two weight ops
+// and the products with the record -- the z weights and the border clamps are paid once per source instead of nine times.
+// (A 12-float record holding the nine products wz_b * g_c saves four instructions per neighbour but costs a third
 // LDS.128: measured shared-memory bound, 61 % of the LSU data pipe vs 50 % issue.)
+// The tile is 32 x 16: thread (lx, ly) owns the targets in rows 2 ly and 2 ly + 1, whose neighbourhoods share two of their
+// three source rows -- against one target per thread, 12 record loads for two targets instead of 18, half the barriers and
+// TMA issues per voxel, a smaller halo share (34 x 18 records for 512 targets).  128 registers, 2 CTAs per SM.
 constexpr int REC_F = 8;    // floats per record
 constexpr int BWD_NG = 3;   // ring slots of the incoming gradient: plane s and two in flight (slot = plane mod 3, static)
-
-struct BwdAcc {
-    float2 xy[3];   // components x, y of bank b (packed: updated with FFMA2)
-    float z[3];     // component z of bank b
-    __device__ __forceinline__ void clear() {
-#pragma unroll
-        for (int i = 0; i < 3; ++i) { xy[i] = make_float2(0.f, 0.f); z[i] = 0.f; }
-    }
-};
-
-template <int OX>
-__device__ __forceinline__ float hat_small(float c) {   // |c| < 1; weight of a source at offset OX onto the target column
-    return OX < 0 ? fmaxf(c, 0.f) : (OX > 0 ? fmaxf(-c, 0.f) : 1.f - fabsf(c));
-}
-
-struct BwdTmaCtx {
-    const CUtensorMap *tmap_u, *tmap_g;
-    float *U, *G, *REC;
-    int* row_nz;          // [3][TMA_EY]: "this source row has a non-zero gradient", per plane modulo 3
-    uint64_t *bar_u, *bar_g;
-    float in_scale, out_scale;
-    IrsDims d;
-    int x0t, y0t, zs, ze, chain;
-    float* g;
-};
-
-template <int BW>
-__device__ __forceinline__ void svf_bwd_tma_body(const BwdTmaCtx& c) {
-    using RG = TmaRing<BW>;
-    const int tid = threadIdx.x;
-    const IrsDims d = c.d;
-    const int lx = tid % TILE_X, ly = tid / TILE_X, x = c.x0t + lx, y = c.y0t + ly;
-    const bool active = x < d.W && y < d.H;
-    const int lc = (ly + 1) * BW + lx + TMA_XO;     // own voxel inside a plane box
-    const int lr = (ly + 1) * TMA_EX + lx + 1;      // own record
-    const float xf = (float)x, yf = (float)y;
-    const float xmax = (float)(d.W - 1), ymax = (float)(d.H - 1), zmax = (float)(d.D - 1);
-    const int Vi = (int)d.V(), HW = d.H * d.W;
-    const int zs = c.zs, ze = c.ze;
-    const int s_first = zs - 1, n_it = (ze - zs) + 2;   // source planes zs-1 .. ze
-    // ring sequence numbers: U plane p -> p - (zs - 2);  G plane p -> p - (zs - 1)
-    const int n_u = n_it + 2, n_g = n_it;
-
-    // the (up to two) records this thread produces per plane
-    int rec_e[2], rec_po[2], rec_row[2];
-    float rec_lox[2], rec_hix[2], rec_loy[2], rec_hiy[2];
-#pragma unroll
-    for (int k = 0; k < 2; ++k) {
-        const int e = tid + k * TILE_T;
-        const int ey = e / TMA_EX, ex = e - ey * TMA_EX;
-        rec_e[k] = e < TMA_EX * TMA_EY ? e : -1;
-        rec_po[k] = ey * BW + ex + (TMA_XO - 1);
-        rec_row[k] = ey;
-        const float gx = (float)(c.x0t - 1 + ex), gy = (float)(c.y0t - 1 + ey);
-        rec_lox[k] = -gx; rec_hix[k] = xmax - gx; rec_loy[k] = -gy; rec_hiy[k] = ymax - gy;
-    }
-
-    if (tid == 0) {
-#pragma unroll
-        for (int i = 0; i < TMA_NS; ++i) irs_mbar_init(&c.bar_u[i], 1);
-#pragma unroll
-        for (int i = 0; i < BWD_NG; ++i) irs_mbar_init(&c.bar_g[i], 1);
-        irs_mbar_fence_init();
-    }
-    if (tid < 3 * TMA_EY) c.row_nz[tid] = 0;
-    __syncthreads();
-    if (tid == 0) {
-        for (int q = 0; q < TMA_NS && q < n_u; ++q) {
-            irs_mbar_expect_tx(&c.bar_u[q], RG::BYTES);
-            irs_tma_load_plane(c.U + q * RG::SS, c.tmap_u, &c.bar_u[q], c.x0t - TMA_XO, c.y0t - 1, zs - 2 + q, 3 * c.chain);
-        }
-        for (int q = 0; q < BWD_NG && q < n_g; ++q) {
-            irs_mbar_expect_tx(&c.bar_g[q], RG::BYTES);
-            irs_tma_load_plane(c.G + q * RG::SS, c.tmap_g, &c.bar_g[q], c.x0t - TMA_XO, c.y0t - 1, zs - 1 + q, 3 * c.chain);
-        }
-    }
-
-    // Records of source plane s_first + itp (its U and G planes must have landed) into record buffer itp & 1 and row
-    // flags itp mod 3.  MP = itp mod 3: target plane s -> bank MP, s+1 -> bank MP+1, s-1 -> bank MP+2 (mod 3).
-    auto produce = [&](auto m_tag, int itp) {
-        constexpr int MP = decltype(m_tag)::value;
-        constexpr int B0 = MP, BP = (MP + 1) % 3, BM = (MP + 2) % 3;
-        const int s = s_first + itp;
-        if (s < 0 || s >= d.D) return;   // nobody reads the records of a plane outside the volume
-        const float* Us = c.U + ((itp + 1) & 3) * RG::SS;
-        const float* Gs = c.G + MP * RG::SS;
-        float4* rec = reinterpret_cast<float4*>(c.REC) + (itp & 1) * (2 * TMA_EX * TMA_EY);
-        const float sf = (float)s;
-#pragma unroll
-        for (int k = 0; k < 2; ++k) {
-            if (rec_e[k] < 0) continue;
-            const int po = rec_po[k];
-            const float g0 = Gs[po], g1 = Gs[RG::CS + po], g2 = Gs[2 * RG::CS + po];
-            const float cx = irs_clampf(Us[po] * c.in_scale, rec_lox[k], rec_hix[k]);
-            const float cy = irs_clampf(Us[RG::CS + po] * c.in_scale, rec_loy[k], rec_hiy[k]);
-            const float cz = irs_clampf(Us[2 * RG::CS + po] * c.in_scale, -sf, zmax - sf);
-            const float wm = fmaxf(-cz, 0.f), w0 = 1.f - fabsf(cz), wp = fmaxf(cz, 0.f);
-            float wb[3];
-            wb[B0] = w0; wb[BP] = wp; wb[BM] = wm;
-            float4* r = rec + rec_e[k];   // two arrays of float4: conflict-free LDS.128
-            r[0] = make_float4(cx, cy, g0, g1);
-            r[TMA_EX * TMA_EY] = make_float4(g2, wb[0], wb[1], wb[2]);
-            if (g0 != 0.f || g1 != 0.f || g2 != 0.f) c.row_nz[MP * TMA_EY + rec_row[k]] = 1;
-        }
-    };
-
-    BwdAcc acc;
-    acc.clear();
-    int gi = ((s_first - 1) * d.H + y) * d.W + x;   // index of target (x, y, s-1)
-    irs_mbar_wait(&c.bar_u[0], 0);
-    irs_mbar_wait(&c.bar_u[1], 0);
-    irs_mbar_wait(&c.bar_g[0], 0);
-    produce(std::integral_constant<int, 0>{}, 0);
-    __syncthreads();
-    if (tid == 0 && BWD_NG < n_g) {   // G plane s_first has been turned into records: its slot takes sequence number 3
-        irs_mbar_expect_tx(&c.bar_g[0], RG::BYTES);
-        irs_tma_load_plane(c.G, c.tmap_g, &c.bar_g[0], c.x0t - TMA_XO, c.y0t - 1, zs - 1 + BWD_NG, 3 * c.chain);
-    }
-
-    // one source plane; M = (s - s_first) mod 3
-    auto iteration = [&](auto m_tag, int it) {
-        constexpr int M = decltype(m_tag)::value;
-        constexpr int B0 = M, BP = (M + 1) % 3, BM = (M + 2) % 3;
-        const int s = s_first + it;
-        irs_mbar_wait(&c.bar_u[(it + 2) & 3], ((it + 2) >> 2) & 1);   // U plane s+1
-        if (tid < TMA_EY) c.row_nz[BM * TMA_EY + tid] = 0;            // flags of plane s+2: last read in the previous iteration
-        if (it + 1 < n_it) {
-            irs_mbar_wait(&c.bar_g[BP], ((it + 1) / 3) & 1);          // G plane s+1 (ring of 3: slot = (it + 1) mod 3)
-            produce(std::integral_constant<int, BP>{}, it + 1);      // records of the NEXT plane: one barrier per plane
-        }
-        const float* Us = c.U + ((it + 1) & 3) * RG::SS;              // U plane s
-        const float4* rec = reinterpret_cast<const float4*>(c.REC) + (it & 1) * (2 * TMA_EX * TMA_EY);
-        if (active && s >= 0 && s < d.D) {
-            // ---- interpolation transpose: 9 in-plane neighbours x 3 target planes ----
-            const int* nz = c.row_nz + M * TMA_EY + ly;
-            float g0 = 0.f, g1 = 0.f, g2 = 0.f;   // the target's own incoming gradient (from its record)
-            auto source_row = [&](auto oy_tag) {
-                constexpr int OY = decltype(oy_tag)::value;
-                auto source = [&](auto ox_tag) {
-                    constexpr int OX = decltype(ox_tag)::value;
-                    const float4* r = rec + (lr + OY * TMA_EX + OX);
-                    const float4 r0 = r[0], r1 = r[TMA_EX * TMA_EY];
-                    const float w = hat_small<OX>(r0.x) * hat_small<OY>(r0.y);
-                    const float w0 = w * r1.y, w1 = w * r1.z, w2 = w * r1.w;
-                    const float2 g01 = make_float2(r0.z, r0.w);
-                    acc.xy[0] = ffma2(make_float2(w0, w0), g01, acc.xy[0]); acc.z[0] = fmaf(w0, r1.x, acc.z[0]);
-                    acc.xy[1] = ffma2(make_float2(w1, w1), g01, acc.xy[1]); acc.z[1] = fmaf(w1, r1.x, acc.z[1]);
-                    acc.xy[2] = ffma2(make_float2(w2, w2), g01, acc.xy[2]); acc.z[2] = fmaf(w2, r1.x, acc.z[2]);
-                    if (OX == 0 && OY == 0) { g0 = r0.z; g1 = r0.w; g2 = r1.x; }
-                };
-                if (nz[OY + 1] != 0) {   // a source row without gradient contributes nothing (warp-uniform)
-                    source(std::integral_constant<int, -1>{});
-                    source(std::integral_constant<int, 0>{});
-                    source(std::integral_constant<int, 1>{});
-                }
-            };
-            source_row(std::integral_constant<int, -1>{});
-            source_row(std::integral_constant<int, 0>{});
-            source_row(std::integral_constant<int, 1>{});
-            // ---- direct + position term of target (x, y, s) ----
-            if (s >= zs && s < ze && nz[1] != 0) {
-                float px = xf + Us[lc] * c.in_scale, py = yf + Us[RG::CS + lc] * c.in_scale,
-                      pz = (float)s + Us[2 * RG::CS + lc] * c.in_scale;
-                const float mx = irs_inside(px, d.W) * c.in_scale, my = irs_inside(py, d.H) * c.in_scale,
-                            mz = irs_inside(pz, d.D) * c.in_scale;
-                px = irs_clampf(px, 0.f, xmax); py = irs_clampf(py, 0.f, ymax); pz = irs_clampf(pz, 0.f, zmax);
-                int i000, sz;
-                float fx, fy, fz, jx, jy, jz;
-                tma_ring_cell<BW>(px, py, pz, c.x0t, c.y0t, s, it + 1, i000, sz, fx, fy, fz);
-                ring_interp_grad_dot<BW>(c.U, RG::CS, i000, sz, g0, g1, g2, fx, fy, fz, jx, jy, jz);
-                acc.xy[B0].x += g0 + mx * jx;
-                acc.xy[B0].y += g1 + my * jy;
-                acc.z[B0] += g2 + mz * jz;
-            }
-        }
-        // ---- target plane s-1 is complete ----
-        if (active && s - 1 >= zs && s - 1 < ze) {
-            c.g[gi] = acc.xy[BM].x * c.out_scale;
-            c.g[Vi + gi] = acc.xy[BM].y * c.out_scale;
-            c.g[2 * Vi + gi] = acc.z[BM] * c.out_scale;
-        }
-        acc.xy[BM] = make_float2(0.f, 0.f);
-        acc.z[BM] = 0.f;
-        gi += HW;
-        __syncthreads();   // U plane s-1, G plane s+1 and the records of plane s are free; those of plane s+1 are complete
-        if (tid == 0) {
-            if (it + 4 < n_u) {
-                irs_mbar_expect_tx(&c.bar_u[it & 3], RG::BYTES);
-                irs_tma_load_plane(c.U + (it & 3) * RG::SS, c.tmap_u, &c.bar_u[it & 3], c.x0t - TMA_XO, c.y0t - 1,
-                                   zs + 2 + it, 3 * c.chain);
-            }
-            if (it + 1 + BWD_NG < n_g) {   // G plane s+1 (sequence number it + 1, slot BP) was consumed by produce()
-                irs_mbar_expect_tx(&c.bar_g[BP], RG::BYTES);
-                irs_tma_load_plane(c.G + BP * RG::SS, c.tmap_g, &c.bar_g[BP], c.x0t - TMA_XO, c.y0t - 1, zs + 3 + it,
-                                   3 * c.chain);
-            }
-        }
-    };
-
-    for (int it = 0; it < n_it; it += 3) {
-        iteration(std::integral_constant<int, 0>{}, it);
-        if (it + 1 < n_it) iteration(std::integral_constant<int, 1>{}, it + 1);
-        if (it + 2 < n_it) iteration(std::integral_constant<int, 2>{}, it + 2);
-    }
-}
-
-constexpr int BWD_BW = 40;
-constexpr size_t svf_bwd_tma_smem() {
-    return sizeof(float) * ((TMA_NS + BWD_NG) * TmaRing<BWD_BW>::SS + 2 * TMA_EX * TMA_EY * REC_F) + 8 * (TMA_NS + BWD_NG) +
-           4 * 3 * TMA_EY + 8;
-}
-
-__global__ void __launch_bounds__(TILE_T, 4)
-svf_step_bwd_tma_kernel(const __grid_constant__ CUtensorMap tmap_u, const __grid_constant__ CUtensorMap tmap_g,
-                        const float* __restrict__ in, float in_scale, const float* __restrict__ gp_all,
-                        float* __restrict__ g_all, const float* __restrict__ maxabs, int radius_max, float out_scale,
-                        int seg_len, IrsDims d, IrsCells cm) {
-    extern __shared__ __align__(128) float smem[];
-    irs_pdl_wait();
-    irs_pdl_launch_dependents();
-    const int R = svf_gather_radius(__ldg(maxabs));
-    const long long V = d.V();
-    const size_t off = (size_t)blockIdx.y * 3 * V;
-    const int tiles_x = (d.W + TILE_X - 1) / TILE_X, tiles_y = (d.H + TILE_Y - 1) / TILE_Y;
-    const int bx = blockIdx.x % tiles_x, by = (blockIdx.x / tiles_x) % tiles_y, bz = blockIdx.x / (tiles_x * tiles_y);
-    const int x0t = bx * TILE_X, y0t = by * TILE_Y, zs = bz * seg_len, ze = min(zs + seg_len, d.D);
-    const int Rl = svf_local_radius(R, radius_max, cm, blockIdx.y, x0t, y0t, TILE_Y, zs, ze);
-    if (Rl == 1 && Rl <= radius_max) {
-        using RG = TmaRing<BWD_BW>;
-        BwdTmaCtx c;
-        c.tmap_u = &tmap_u; c.tmap_g = &tmap_g;
-        c.U = smem;
-        c.G = smem + TMA_NS * RG::SS;
-        c.REC = smem + (TMA_NS + BWD_NG) * RG::SS;
-        c.bar_u = reinterpret_cast<uint64_t*>(c.REC + 2 * TMA_EX * TMA_EY * REC_F);
-        c.bar_g = c.bar_u + TMA_NS;
-        c.row_nz = reinterpret_cast<int*>(c.bar_g + BWD_NG);
-        c.in_scale = in_scale; c.out_scale = out_scale; c.d = d;
-        c.x0t = x0t; c.y0t = y0t; c.zs = zs; c.ze = ze; c.chain = blockIdx.y;
-        c.g = g_all + off;
-        svf_bwd_tma_body<BWD_BW>(c);
-    } else {
-        svf_bwd_tile_dispatch_cold(R, in + off, in_scale, gp_all + off, g_all + off, radius_max, out_scale, d, x0t, y0t, zs, ze,
-                                   smem);
-    }
-}
-
-// ---- adjoint step, two targets per thread ----------------------------------------------------------------------------------
-// Same algorithm on a 32 x 16 tile: thread (lx, ly) owns the targets in rows 2 ly and 2 ly + 1, whose neighbourhoods share
-// two of their three source rows -- 12 record loads for two targets instead of 18, half the barriers and TMA issues per
-// voxel, a smaller halo share (34 x 18 records for 512 targets).  128 registers, 2 CTAs per SM.
+constexpr int BWD_BW = 40;  // row pitch of the plane boxes (why not 64: see FWD_BW)
 constexpr int B2_TY = 16, B2_EY = B2_TY + 2, B2_NR = TMA_EX * B2_EY;                  // 612 records per plane
 constexpr int B2_CS = B2_EY * BWD_BW;                                               // component stride of a plane box
 constexpr uint32_t B2_BYTES = 3u * B2_CS * 4u;
@@ -1049,7 +791,19 @@ constexpr size_t svf_bwd_tma2_smem() {
     return sizeof(float) * ((TMA_NS + BWD_NG) * B2_SS + 2 * B2_NR * REC_F) + 8 * (TMA_NS + BWD_NG) + 4 * 3 * B2_EY + 8;
 }
 
-__device__ __forceinline__ float hat_small_rt(float c, int o) {   // hat_small with the offset as a (constant-folded) argument
+struct BwdTmaCtx {
+    const CUtensorMap *tmap_u, *tmap_g;
+    float *U, *G, *REC;
+    int* row_nz;          // [3][B2_EY]: "this source row has a non-zero gradient", per plane modulo 3
+    uint64_t *bar_u, *bar_g;
+    float in_scale, out_scale;
+    IrsDims d;
+    int x0t, y0t, zs, ze, chain;
+    float* g;
+};
+
+// |c| < 1: hat weight of a source at in-plane offset o (-1, 0, 1; constant-folded) onto the target column
+__device__ __forceinline__ float hat_small_rt(float c, int o) {
     return o < 0 ? fmaxf(c, 0.f) : (o > 0 ? fmaxf(-c, 0.f) : 1.f - fabsf(c));
 }
 
@@ -1126,16 +880,11 @@ __device__ __forceinline__ void svf_bwd_tma2_body(const BwdTmaCtx& c) {
             float4* r = rec + rec_e[k];
             r[0] = make_float4(cx, cy, g0, g1);
             r[B2_NR] = make_float4(g2, wm, w0, wp);
-#if IRS_BWD_V2
             if (((__float_as_uint(g0) | __float_as_uint(g1) | __float_as_uint(g2)) << 1) != 0u)   // any non-zero (+-0 are zero)
                 c.row_nz[MP * B2_EY + rec_row[k]] = 1;
-#else
-            if (g0 != 0.f || g1 != 0.f || g2 != 0.f) c.row_nz[MP * B2_EY + rec_row[k]] = 1;
-#endif
         }
     };
 
-#if IRS_BWD_V2
     // Accumulators: XY[j][b] = components (x, y) of target j in bank b; ZZ[b] = component z of targets (0, 1) in bank b.
     // A record of the two source rows that both targets see costs 3 FMUL2 + 9 FFMA2 for its 18 products (the z components of
     // the two targets share one packed FMA); bank 0 = target plane s-1, 1 = s, 2 = s+1, rotated by register moves per plane.
@@ -1259,112 +1008,6 @@ __device__ __forceinline__ void svf_bwd_tma2_body(const BwdTmaCtx& c) {
         }
     }
 }
-#else
-    BwdAcc acc[2];
-    acc[0].clear(); acc[1].clear();
-    int gi = ((s_first - 1) * d.H + y0) * d.W + x;   // index of target 0 in plane s-1 (target 1: + W)
-    irs_mbar_wait(&c.bar_u[0], 0);
-    irs_mbar_wait(&c.bar_u[1], 0);
-    irs_mbar_wait(&c.bar_g[0], 0);
-    produce(0);
-    __syncthreads();
-    if (tid == 0 && BWD_NG < n_g) {
-        irs_mbar_expect_tx(&c.bar_g[0], B2_BYTES);
-        irs_tma_load_plane(c.G, c.tmap_g, &c.bar_g[0], c.x0t - TMA_XO, c.y0t - 1, zs - 1 + BWD_NG, 3 * c.chain);
-    }
-
-    for (int it = 0; it < n_it; ++it) {
-        constexpr int B0 = 1, BM = 0;   // accumulator 0 = target plane s-1, 1 = s, 2 = s+1
-        const int M = it % 3, BP = (it + 1) % 3, BMf = (it + 2) % 3;   // ring slots (gradient planes, row flags)
-        const int s = s_first + it;
-        irs_mbar_wait(&c.bar_u[(it + 2) & 3], ((it + 2) >> 2) & 1);
-        if (tid < B2_EY) c.row_nz[BMf * B2_EY + tid] = 0;
-        if (it + 1 < n_it) {
-            irs_mbar_wait(&c.bar_g[BP], ((it + 1) / 3) & 1);
-            produce(it + 1);
-        }
-        const float* Us = c.U + ((it + 1) & 3) * SS;
-        const float4* rec = reinterpret_cast<const float4*>(c.REC) + (it & 1) * (2 * B2_NR);
-        if ((act[0] || act[1]) && s >= 0 && s < d.D) {
-            const int* nz = c.row_nz + M * B2_EY + ty0;   // flags of record rows ty0 .. ty0 + 3
-            float gown[2][3] = {{0.f, 0.f, 0.f}, {0.f, 0.f, 0.f}};
-            // record row rr (0..3) of this thread's neighbourhood: oy = rr - 1 for target 0, rr - 2 for target 1
-#pragma unroll
-            for (int rr = 0; rr < 4; ++rr) {
-                if (nz[rr] == 0) continue;   // warp-uniform: the row holds no gradient
-#pragma unroll
-                for (int ox = -1; ox <= 1; ++ox) {
-                    const float4* r = rec + (lr0 + (rr - 1) * TMA_EX + ox);
-                    const float4 r0 = r[0], r1 = r[B2_NR];
-                    const float wx = hat_small_rt(r0.x, ox);
-                    const float2 g01 = make_float2(r0.z, r0.w);
-#pragma unroll
-                    for (int j = 0; j < 2; ++j) {
-                        const int oy = rr - 1 - j;
-                        if (oy < -1 || oy > 1) continue;
-                        const float w = wx * hat_small_rt(r0.y, oy);
-                        const float w0 = w * r1.y, w1 = w * r1.z, w2 = w * r1.w;
-                        acc[j].xy[0] = ffma2(make_float2(w0, w0), g01, acc[j].xy[0]); acc[j].z[0] = fmaf(w0, r1.x, acc[j].z[0]);
-                        acc[j].xy[1] = ffma2(make_float2(w1, w1), g01, acc[j].xy[1]); acc[j].z[1] = fmaf(w1, r1.x, acc[j].z[1]);
-                        acc[j].xy[2] = ffma2(make_float2(w2, w2), g01, acc[j].xy[2]); acc[j].z[2] = fmaf(w2, r1.x, acc[j].z[2]);
-                        if (ox == 0 && oy == 0) { gown[j][0] = r0.z; gown[j][1] = r0.w; gown[j][2] = r1.x; }
-                    }
-                }
-            }
-            // ---- direct + position terms ----
-            if (s >= zs && s < ze) {
-#pragma unroll
-                for (int j = 0; j < 2; ++j) {
-                    if (!act[j] || nz[1 + j] == 0) continue;
-                    const int lc = lc0 + j * BW;
-                    const float g0 = gown[j][0], g1 = gown[j][1], g2 = gown[j][2];
-                    float px = xf + Us[lc] * c.in_scale, py = (float)(y0 + j) + Us[CS + lc] * c.in_scale,
-                          pz = (float)s + Us[2 * CS + lc] * c.in_scale;
-                    const float mx = irs_inside(px, d.W) * c.in_scale, my = irs_inside(py, d.H) * c.in_scale,
-                                mz = irs_inside(pz, d.D) * c.in_scale;
-                    px = irs_clampf(px, 0.f, xmax); py = irs_clampf(py, 0.f, ymax); pz = irs_clampf(pz, 0.f, zmax);
-                    const float fx0 = floorf(px), fy0 = floorf(py), fz0 = floorf(pz);
-                    const float fx = px - fx0, fy = py - fy0, fz = pz - fz0;
-                    const int ix = (int)fx0, iy = (int)fy0, iz = (int)fz0;
-                    const int s0 = (it + 1 + (iz - s)) & (TMA_NS - 1), s1 = (s0 + 1) & (TMA_NS - 1);
-                    const int i000 = s0 * SS + (iy - (c.y0t - 1)) * BW + (ix - (c.x0t - TMA_XO));
-                    float jx, jy, jz;
-                    ring_interp_grad_dot<BW>(c.U, CS, i000, (s1 - s0) * SS, g0, g1, g2, fx, fy, fz, jx, jy, jz);
-                    acc[j].xy[B0].x += g0 + mx * jx;
-                    acc[j].xy[B0].y += g1 + my * jy;
-                    acc[j].z[B0] += g2 + mz * jz;
-                }
-            }
-        }
-        // ---- target plane s-1 is complete ----
-#pragma unroll
-        for (int j = 0; j < 2; ++j) {
-            if (act[j] && s - 1 >= zs && s - 1 < ze) {
-                const int o = gi + j * d.W;
-                c.g[o] = acc[j].xy[BM].x * c.out_scale;
-                c.g[Vi + o] = acc[j].xy[BM].y * c.out_scale;
-                c.g[2 * Vi + o] = acc[j].z[BM] * c.out_scale;
-            }
-            acc[j].xy[0] = acc[j].xy[1]; acc[j].z[0] = acc[j].z[1];
-            acc[j].xy[1] = acc[j].xy[2]; acc[j].z[1] = acc[j].z[2];
-            acc[j].xy[2] = make_float2(0.f, 0.f); acc[j].z[2] = 0.f;
-        }
-        gi += HW;
-        __syncthreads();
-        if (tid == 0) {
-            if (it + 4 < n_u) {
-                irs_mbar_expect_tx(&c.bar_u[it & 3], B2_BYTES);
-                irs_tma_load_plane(c.U + (it & 3) * SS, c.tmap_u, &c.bar_u[it & 3], c.x0t - TMA_XO, c.y0t - 1, zs + 2 + it,
-                                   3 * c.chain);
-            }
-            if (it + 1 + BWD_NG < n_g) {
-                irs_mbar_expect_tx(&c.bar_g[BP], B2_BYTES);
-                irs_tma_load_plane(c.G + BP * SS, c.tmap_g, &c.bar_g[BP], c.x0t - TMA_XO, c.y0t - 1, zs + 3 + it, 3 * c.chain);
-            }
-        }
-    }
-}
-#endif
 
 __global__ void __launch_bounds__(TILE_T, 2)
 svf_step_bwd_tma2_kernel(const __grid_constant__ CUtensorMap tmap_u, const __grid_constant__ CUtensorMap tmap_g,
@@ -1417,7 +1060,7 @@ constexpr size_t svf_fwd_tile_smem(int R) {
 // the hardware scheduler even the SMs out; measured at 128^3, one chain: 10 (adjoint) / 8 (forward) planes beat 15.
 static int svf_seg_len(IrsDims d, int C, int slots, int halo, const char* env_name = "IRS_SVF_SEG", bool dynamic = false,
                        int tile_y = TILE_Y) {
-    if (const char* e = getenv(env_name)) {   // development override
+    if (const char* e = getenv(env_name)) {   // test hook: forces segment boundaries; read at every launch
         const int v = atoi(e);
         if (v >= 1) return v < d.D ? v : d.D;
     }
@@ -1466,10 +1109,8 @@ svf_outputs_kernel(const float* __restrict__ u_all, const float* __restrict__ li
 // the resident-CTA counts come from that device's occupancy calculator.  A process that drives several GPUs (one sampler per
 // device) must not reuse the first device's state, so everything is cached PER DEVICE behind a mutex.
 struct SvfDeviceState {
-    bool fwd_tma_ready = false, bwd_tile_ready = false, bwd_tma_ready = false, bwd_tma2_ready = false;
-    int fwd_ctas = 0;
+    bool fwd_tma_ready = false, bwd_tile_ready = false, bwd_tma2_ready = false;
     int slots_fwd_tma = 0, slots_fwd_tile = 0, slots_bwd_tile = 0, slots_bwd_tma = 0;
-    int two = -1;
 };
 constexpr int kMaxDevices = 64;
 SvfDeviceState g_svf_dev[kMaxDevices];
@@ -1523,21 +1164,12 @@ int irs_launch_svf_fwd(const float* v, float* hist, float* maxabs, int n_steps, 
     const bool tma = irs_tma_field_ok(v, d.W) && irs_tma_field_ok(hist, d.W) && (F % 4) == 0;
     if (tma) {
         const size_t smem = zmax(svf_fwd_tma_smem(), svf_fwd_tile_smem_compact(RF));
-        using Kern = void (*)(CUtensorMap, const float*, float, float*, const float*, float*, int, IrsDims, IrsEnergyOut);
-        Kern kern = nullptr, kern_e = nullptr;
+        auto* const kern = svf_step_fwd_tma_kernel<false>;
+        auto* const kern_e = svf_step_fwd_tma_kernel<true>;
         int slots = 0;
         {
             std::lock_guard<std::mutex> lock(g_svf_mu);
             SvfDeviceState& ds = svf_device_state();
-            if (ds.fwd_ctas == 0) {
-                ds.fwd_ctas = 5;   // measured at 128^3: 4 -> 0.212 ms, 5 -> 0.200 ms, 6 -> 0.208 ms for the 12 forward steps
-                if (const char* ev = getenv("IRS_FWD_CTAS")) ds.fwd_ctas = atoi(ev);   // development override
-            }
-            const int ctas = ds.fwd_ctas;
-            kern = ctas <= 4 ? (Kern)svf_step_fwd_tma_kernel<4, false>
-                             : (ctas == 5 ? (Kern)svf_step_fwd_tma_kernel<5, false> : (Kern)svf_step_fwd_tma_kernel<6, false>);
-            kern_e = ctas <= 4 ? (Kern)svf_step_fwd_tma_kernel<4, true>
-                               : (ctas == 5 ? (Kern)svf_step_fwd_tma_kernel<5, true> : (Kern)svf_step_fwd_tma_kernel<6, true>);
             if (!ds.fwd_tma_ready) {
                 e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
                 if (e != cudaSuccess) return (int)e;
@@ -1598,14 +1230,12 @@ int irs_launch_svf_bwd(const float* v, const float* hist, const float* maxabs, f
     const size_t F = (size_t)C * 3 * d.V();
     const float scale0 = 1.0f / (float)(1 << n_steps);
     const size_t smem = svf_bwd_tile_smem(2);
-    const int tiles = ((d.W + TILE_X - 1) / TILE_X) * ((d.H + TILE_Y - 1) / TILE_Y);
     const long long vblocks = (d.V() + 255) / 256;
     dim3 vgrid((unsigned)(vblocks < 1184 ? vblocks : 1184), 1);   // persistent: see svf_step_bwd_scatter_kernel
     const bool tma = irs_tma_field_ok(v, d.W) && irs_tma_field_ok(hist, d.W) && irs_tma_field_ok(g_u, d.W) &&
                      irs_tma_field_ok(g_work, d.W) && (F % 4) == 0;
-    const size_t smem_tma = zmax(svf_bwd_tma_smem(), smem);
-    const size_t smem_tma2 = zmax(svf_bwd_tma2_smem(), smem);
-    int slots = 0, slots_tma = 0, two = 1;
+    const size_t smem_tma = zmax(svf_bwd_tma2_smem(), smem);
+    int slots = 0, slots_tma = 0;
     {
         std::lock_guard<std::mutex> lock(g_svf_mu);
         SvfDeviceState& ds = svf_device_state();
@@ -1615,29 +1245,19 @@ int irs_launch_svf_bwd(const float* v, const float* hist, const float* maxabs, f
             ds.slots_bwd_tile = resident_ctas(svf_step_bwd_tile_kernel, smem);
             ds.bwd_tile_ready = true;
         }
-        if (ds.two < 0)   // two targets per thread (32 x 16 tiles) unless IRS_BWD_NT=1 (development switch)
-            ds.two = (getenv("IRS_BWD_NT") && atoi(getenv("IRS_BWD_NT")) == 1) ? 0 : 1;
-        two = ds.two;
-        if (tma && two == 1 && !ds.bwd_tma2_ready) {
-            cudaError_t e = cudaFuncSetAttribute(svf_step_bwd_tma2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_tma2);
+        if (tma && !ds.bwd_tma2_ready) {
+            cudaError_t e = cudaFuncSetAttribute(svf_step_bwd_tma2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_tma);
             if (e != cudaSuccess) return (int)e;
-            ds.slots_bwd_tma = resident_ctas(svf_step_bwd_tma2_kernel, smem_tma2);
+            ds.slots_bwd_tma = resident_ctas(svf_step_bwd_tma2_kernel, smem_tma);
             ds.bwd_tma2_ready = true;
-        }
-        if (tma && two == 0 && !ds.bwd_tma_ready) {
-            cudaError_t e = cudaFuncSetAttribute(svf_step_bwd_tma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_tma);
-            if (e != cudaSuccess) return (int)e;
-            ds.slots_bwd_tma = resident_ctas(svf_step_bwd_tma_kernel, smem_tma);
-            ds.bwd_tma_ready = true;
         }
         slots = ds.slots_bwd_tile;
         slots_tma = ds.slots_bwd_tma;
     }
-    const bool tma2 = tma && two == 1;
-    const int seg_len = tma ? svf_seg_len(d, C, slots_tma, 4, "IRS_SVF_SEG_BWD", true, tma2 ? B2_TY : TILE_Y) : svf_seg_len(d, C, slots, 6);
-    const int nseg = (d.D + seg_len - 1) / seg_len;
-    const int tiles2 = ((d.W + TILE_X - 1) / TILE_X) * ((d.H + B2_TY - 1) / B2_TY);
-    dim3 tgrid((tma2 ? tiles2 : tiles) * nseg, C);
+    const int tile_y = tma ? B2_TY : TILE_Y;
+    const int seg_len = tma ? svf_seg_len(d, C, slots_tma, 4, "IRS_SVF_SEG_BWD", true, tile_y) : svf_seg_len(d, C, slots, 6);
+    const int tiles = ((d.W + TILE_X - 1) / TILE_X) * ((d.H + tile_y - 1) / tile_y);
+    dim3 tgrid(tiles * ((d.D + seg_len - 1) / seg_len), C);
     // ping-pong between g_work and the caller's g_u buffer (g_u is only read by the first adjoint step)
     const float* gp = g_u;
     cudaError_t le = cudaSuccess;
@@ -1655,16 +1275,11 @@ int irs_launch_svf_bwd(const float* v, const float* hist, const float* maxabs, f
         const int radius_max_k = companion ? gather_radius_max : 0x7fffffff;
         if (tma) {
             CUtensorMap map_u, map_g;
-            const int bh = tma2 ? B2_EY : TMA_EY;
-            if (irs_tma_encode_field(&map_u, in, 3 * C, d.D, d.H, d.W, BWD_BW, bh) != 0 ||
-                irs_tma_encode_field(&map_g, gp, 3 * C, d.D, d.H, d.W, BWD_BW, bh) != 0)
+            if (irs_tma_encode_field(&map_u, in, 3 * C, d.D, d.H, d.W, BWD_BW, B2_EY) != 0 ||
+                irs_tma_encode_field(&map_g, gp, 3 * C, d.D, d.H, d.W, BWD_BW, B2_EY) != 0)
                 return IRS_ERR_UNSUPPORTED;
-            if (tma2)
-                le = irs_launch_pdl(svf_step_bwd_tma2_kernel, tgrid, dim3(TILE_T), smem_tma2, st, map_u, map_g, in, in_scale,
-                                    gp, out, maxabs + k, radius_max_k, in_scale, seg_len, d, cm);
-            else
-                le = irs_launch_pdl(svf_step_bwd_tma_kernel, tgrid, dim3(TILE_T), smem_tma, st, map_u, map_g, in, in_scale, gp,
-                                    out, maxabs + k, radius_max_k, in_scale, seg_len, d, cm);
+            le = irs_launch_pdl(svf_step_bwd_tma2_kernel, tgrid, dim3(TILE_T), smem_tma, st, map_u, map_g, in, in_scale, gp,
+                                out, maxabs + k, radius_max_k, in_scale, seg_len, d, cm);
         } else {
             le = irs_launch_pdl(svf_step_bwd_tile_kernel, tgrid, dim3(TILE_T), smem, st, in, in_scale, gp, out, maxabs + k,
                                 radius_max_k, in_scale, seg_len, d, cm);

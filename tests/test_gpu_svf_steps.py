@@ -7,10 +7,6 @@ Forward: the input of step k is the kernel's own hist[k - 1], so each step is ch
 Adjoint: ops.svf_exp_bwd reads only v, hist[0 .. n-2] and the maxabs block, so a test builds them itself with one
 non-zero step input U at step k.  A step whose input is zero maps g to exactly 2 g, hence g_v = 2^(n-1) 2^-n A_U^T g.
 """
-import os
-import subprocess
-import sys
-
 import pytest
 import torch
 
@@ -19,7 +15,6 @@ from tests.util import smooth_field
 
 pytestmark = pytest.mark.gpu
 DEV = 'cuda:0'
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
 @pytest.fixture(scope='module')
@@ -268,24 +263,3 @@ def test_composite_twelve_steps(ops, n, C):
         g_v = ops.svf_exp_bwd(v, hist, maxabs, g, radius_max)
         expect_within(g_v, ref, bound, f'composite n={n} C={C} radius_max={radius_max}')
 
-
-# ---- development kernels that ship in the library ---------------------------------------------------------------------------
-CHILD_SUBSET = ('(test_forward_steps and (n40 or n16)) or test_forward_threshold_inputs or '
-                '(test_adjoint_step and not rings and not forced and (12_11 or 1_0 or 12_8))')
-
-
-@pytest.mark.parametrize('env', [{'IRS_BWD_NT': '1'}, {'IRS_FWD_CTAS': '4'}, {'IRS_FWD_CTAS': '6'}],
-                         ids=['IRS_BWD_NT=1', 'IRS_FWD_CTAS=4', 'IRS_FWD_CTAS=6'])
-def test_development_kernels(env):
-    """the one-target adjoint and the other forward occupancies are chosen once per device and process, so a subset of
-    this file runs in a child pytest process with each setting; the child has exited when this test returns"""
-    if os.environ.get('IRS_SVF_STEPS_CHILD'):
-        pytest.skip('inside the child process')
-    cmd = [sys.executable] + (['-s'] if sys.flags.no_user_site else []) + \
-          ['-m', 'pytest', '-q', '-p', 'no:cacheprovider', '-m', 'gpu', os.path.abspath(__file__), '-k', CHILD_SUBSET]
-    res = subprocess.run(cmd, cwd=ROOT, env={**os.environ, **env, 'IRS_SVF_STEPS_CHILD': '1'}, capture_output=True, text=True,
-                         timeout=1800)
-    tail = res.stdout[-3000:] + res.stderr[-2000:]
-    print(tail)
-    assert res.returncode == 0, tail
-    assert ' passed' in res.stdout and ' failed' not in res.stdout
