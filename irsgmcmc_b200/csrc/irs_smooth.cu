@@ -184,7 +184,8 @@ langevin_vec_kernel(const float* __restrict__ v, const float* __restrict__ sigma
 // of s rows on either side goes to shared memory (the halo rows regenerate their Philox numbers -- a voxel's noise is a pure
 // function of (seed, chain, iteration, voxel) -- 2 s / TY more generator work, against a whole pass over the field saved),
 // is smoothed along x in place (one float4 per thread per round, neighbours read before anybody writes) and along y on the way
-// out.  The z pass that follows is the only other pass: 12 + 12 (+ halo) read, 12 written here, 12 + 12 there, instead of four
+// out (a round of the in-place x pass takes whole rows, so that every unit reads neighbours no other round has written).  The
+// z pass that follows is the only other pass: 12 + 12 (+ halo) read, 12 written here, 12 + 12 there, instead of four
 // passes of 24 B.  Separable smoothing passes commute (replicate padding acts per axis), so x, y, z instead of the reference's
 // z, y, x changes the result at rounding level only (checked against the oracle at 1e-5 like before).
 template <int NT>
@@ -232,10 +233,12 @@ langevin_xy_kernel(const float* __restrict__ v, const float* __restrict__ sigma,
         for (int ch = 0; ch < 3; ++ch) *reinterpret_cast<float4*>(S + ch * CS + r * W + 4 * x4) = a[ch];
     }
     __syncthreads();
-    // ---- x pass, in place: every thread reads the three aligned float4 of its unit, then all write ----
-    for (int base = 0; base < units; base += blockDim.x) {
+    // ---- x pass, in place: every thread reads the three aligned float4 of its unit, then all write.  A round covers whole
+    // rows (irs_langevin_fused keeps W4 <= 512), so no unit reads a neighbour that an earlier round already smoothed ----
+    const int round_units = (blockDim.x / W4) * W4;
+    for (int base = 0; base < units; base += round_units) {
         const int u = base + threadIdx.x;
-        const bool valid = u < units;
+        const bool valid = threadIdx.x < round_units && u < units;
         float4 o[3];
         if (valid) {
             const int r = u / W4, x4 = u - r * W4;
@@ -575,8 +578,11 @@ int irs_launch_smooth3(const float* in, float* work, float* out, const IrsTaps& 
     return (int)cudaGetLastError();
 }
 
-bool irs_langevin_fused(IrsDims d, int n_taps) {   // the last term: the smallest tile (8 rows + halo) fits in 200 KB
-    return d.W % 4 == 0 && (n_taps == 3 || n_taps == 5 || n_taps == 7) && (size_t)3 * (8 + n_taps - 1) * d.W * 4 <= 200 * 1024;
+// the smallest tile (8 rows + halo) fits in 200 KB, and a round of the x pass (512 threads, one float4 each) holds at least
+// one whole row (implied by the first condition today: W <= 1706; stated so that a larger tile budget cannot make it spin)
+bool irs_langevin_fused(IrsDims d, int n_taps) {
+    return d.W % 4 == 0 && (n_taps == 3 || n_taps == 5 || n_taps == 7) && (size_t)3 * (8 + n_taps - 1) * d.W * 4 <= 200 * 1024 &&
+           d.W / 4 <= 512;
 }
 
 // Langevin proposal + separable smoothing: two kernels (noise + x + y on shared-memory rows, then z) when the field can be
