@@ -253,6 +253,37 @@ int irs_label_posterior(const int* counts, const int* labels_host, int n_labels,
                         void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------------ *
+ * Posterior of the Jacobian determinant (the reference computes log det J per sample, utils/util.py:72-91,209-212, and
+ * aggregates nothing).  ld(c, v) = what irs_log_det_jacobian writes for sample c at voxel v; the sample is finite at v when
+ * ld is finite (det > 0) and folded otherwise: det < 0 (NaN, the reference's folding), det == 0 (-inf), NaN or inf input.
+ * Without an exact zero or an overflow, "folded" is the reference's NaN count.  Accumulators per voxel (12 bytes, whatever
+ * the number of samples): folds (V) ints = folded samples; mean, m2 (V) floats = Welford of ld over the n_v = n - folds
+ * finite samples, the recurrence of irs_welford_update with the running count starting at count_before - folds.  Zero them
+ * before the first update; with no fold anywhere mean / m2 equal irs_welford_update on the stacked log det volumes bit for bit.
+ *   irs_jacobian_update: folds the C transformations T (C,3,D,H,W) into the accumulators (one launch); count_before = samples
+ *     accumulated so far, count_before + C <= 2^24.  sample_stats (C,4) doubles per sample over the voxels where mask (V
+ *     bytes) != 0: finite voxels, folded voxels, sum ld, sum ld^2 over the finite ones (counts by integer atomics, sums by
+ *     block partials added in a fixed order).  partials: IRS_JACOBIAN_PARTIALS_DOUBLES(C) doubles; counters: C + 1 unsigned
+ *     long longs, zero on the first call and left zero.
+ *   irs_jacobian_posterior: from the accumulators of n (1..2^24) samples, p_fold = (float)folds / (float)n; mean_out = mean,
+ *     NaN where n_v = 0; std_out = sqrt(m2 / (n_v - 1)), NaN where n_v < 2 (all (V) floats).  summary: IRS_JACOBIAN_SUMMARY_WORDS
+ *     8-byte words over the mask voxels: [0] sum folds, [1] #{folds > 0}, [2] #{2 folds > n}, [3] #{n_v >= 1}, [4] #{n_v >= 2},
+ *     [7] mask voxels as long longs (exact, integer atomics); [5] mean of mean_out over the voxels of [3], [6] mean of std_out
+ *     over those of [4] as doubles (NaN for none; fixed-order block partials).  partials: IRS_JACOBIAN_PARTIALS_DOUBLES(1)
+ *     doubles; counters: 1 unsigned long long.
+ * Deterministic, no host synchronisation, graph-capturable.
+ * ------------------------------------------------------------------------------------------------------------------ */
+#define IRS_JACOBIAN_REDUCE_BLOCKS 1184
+#define IRS_JACOBIAN_PARTIALS_DOUBLES(C) (2 * (size_t)(C) * IRS_JACOBIAN_REDUCE_BLOCKS)
+#define IRS_JACOBIAN_SUMMARY_WORDS 8
+int irs_jacobian_update(const float* T, const unsigned char* mask, int C, int D, int H, int W, double count_before,
+                        int* folds, float* mean, float* m2, double* sample_stats, double* partials,
+                        unsigned long long* counters, void* stream);
+int irs_jacobian_posterior(const int* folds, const float* mean, const float* m2, long long n, long long V,
+                           const unsigned char* mask, float* p_fold, float* mean_out, float* std_out, double* partials,
+                           unsigned long long* counters, long long* summary, void* stream);
+
+/* ------------------------------------------------------------------------------------------------------------------ *
  * The fused SGLD transition -- replaces Trainer._SGLD_transition, trainer/trainer.py:291-356, for all chains of this
  * GPU, including the sequential per-chain GMM Adam step (trainer.py:316-327, 68-77; optimizers/adam_rate_decay.py),
  * the regulariser's hyper-parameter Adam step (trainer.py:353-354) and the plain-SGD state update (trainer.py:351).

@@ -55,6 +55,15 @@ __device__ __forceinline__ float irs_jitter_normalised(float u01, float alpha, i
     return __fdiv_rn(__fmul_rn(noise, 2.0f), (float)(n - 1));
 }
 
+// log det J from the nine scaled forward differences J[j][comp] = d T_comp / d x_j: the 3x3 determinant written out with
+// the same six products in the same order as the reference (utils/util.py:72-91), then logf.  log_det_j_kernel
+// (irs_metrics.cu) and the Jacobian posterior (irs_jacobian.cu) both call it, so they compute the same bits.
+__device__ __forceinline__ float irs_log_det_3x3(const float (&J)[3][3]) {
+    const float det = J[0][0] * J[1][1] * J[2][2] + J[0][1] * J[1][2] * J[2][0] + J[0][2] * J[1][0] * J[2][1] -
+                      J[2][0] * J[1][1] * J[0][2] - J[2][1] * J[1][2] * J[0][0] - J[2][2] * J[1][0] * J[0][1];
+    return logf(det);
+}
+
 // up to 32 segmentation labels of one per-sample evaluation launch (Dice counts, surface distance)
 struct LabelList {
     int n;

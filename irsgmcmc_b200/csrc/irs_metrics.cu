@@ -26,10 +26,8 @@ log_det_j_kernel(const float* __restrict__ T_all, float* __restrict__ log_det, i
             J[1][ch] = (__ldg(f + iy + sy) - __ldg(f + iy)) * ky;
             J[2][ch] = (__ldg(f + iz + sz) - __ldg(f + iz)) * kz;
         }
-        // nabla_x = J[.][0], nabla_y = J[.][1], nabla_z = J[.][2]; same six products and order as the reference
-        const float det = J[0][0] * J[1][1] * J[2][2] + J[0][1] * J[1][2] * J[2][0] + J[0][2] * J[1][0] * J[2][1] -
-                          J[2][0] * J[1][1] * J[0][2] - J[2][1] * J[1][2] * J[0][0] - J[2][2] * J[1][0] * J[0][1];
-        const float ld = logf(det);
+        // nabla_x = J[.][0], nabla_y = J[.][1], nabla_z = J[.][2]
+        const float ld = irs_log_det_3x3(J);
         if (log_det != nullptr) log_det[(size_t)c * V + i] = ld;
         folded += (ld != ld) ? 1 : 0;   // NaN: negative determinant
     }

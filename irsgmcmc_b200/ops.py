@@ -514,3 +514,86 @@ def average_surface_distance(seg_a, seg_b, labels, spacing, workspace_bytes=512 
                 _lib.ptr(ws), ws.numel(), _lib.ptr(partials), _lib.ptr(counters), _lib.ptr(asd), C, D, H, W, _lib.stream()))
         out[:, l0:l0 + n] = asd
     return out
+
+
+def _mask_u8(mask, V):
+    if mask.numel() != V:
+        raise ValueError(f'mask must hold the {V} voxels of the volume')
+    if mask.dtype == torch.bool:
+        return mask.contiguous().view(torch.uint8)
+    if mask.dtype != torch.uint8:
+        raise NotImplementedError('bool / uint8 masks only')
+    return mask.contiguous()
+
+
+def jacobian_scratch(C, device):
+    """(partials, counters) of irs_jacobian_update for C chains (also enough for irs_jacobian_posterior); the counters start at
+    zero and every call leaves them zero, so a caller may keep the pair for all its updates"""
+    partials = torch.empty(2 * C * _lib.JACOBIAN_REDUCE_BLOCKS, device=device, dtype=torch.float64)
+    return partials, torch.zeros(C + 1, device=device, dtype=torch.int64)
+
+
+def jacobian_update(T, mask, count_before, folds, mean, m2, scratch=None):
+    """
+    Fold the log det J of the C transformations T (C,3,D,H,W) into the Jacobian-posterior accumulators of `count_before` earlier
+    samples, in place: folds (D,H,W) int32 = folded samples (log det J not finite: det <= 0, NaN or inf), mean / m2 (D,H,W) fp32
+    = Welford of log det J over the finite samples.  mask (D,H,W) bool / uint8.  Returns the (C,4) fp64 device tensor of this
+    sample over the mask, per chain: finite voxels, folded voxels, sum of log det J and of its square over the finite voxels.
+    scratch: jacobian_scratch(C, device), or None for a fresh pair.
+    """
+    lib = _lib.load()
+    _lib.require_cuda(T, mask, folds, mean, m2)
+    _f32(T, mean, m2)
+    C, D, H, W = _dims(T)
+    V = D * H * W
+    if T.shape[1] != 3:
+        raise ValueError('T must be (C,3,D,H,W)')
+    if folds.dtype != torch.int32:
+        raise NotImplementedError('int32 folds only')
+    if folds.numel() != V or mean.numel() != V or m2.numel() != V:
+        raise ValueError(f'folds, mean and m2 must hold the {V} voxels of T')
+    m8 = _mask_u8(mask, V)
+    partials, counters = jacobian_scratch(C, T.device) if scratch is None else scratch
+    if partials.numel() < 2 * C * _lib.JACOBIAN_REDUCE_BLOCKS or counters.numel() < C + 1:
+        raise ValueError(f'scratch too small for {C} chains')
+    stats = torch.empty(C, 4, device=T.device, dtype=torch.float64)
+    _lib.check(lib.irs_jacobian_update(_lib.ptr(T), _lib.ptr(m8), C, D, H, W, float(count_before), _lib.ptr(folds),
+                                       _lib.ptr(mean), _lib.ptr(m2), _lib.ptr(stats), _lib.ptr(partials), _lib.ptr(counters),
+                                       _lib.stream()))
+    return stats
+
+
+def jacobian_posterior(folds, mean, m2, n, mask):
+    """
+    The Jacobian posterior from the accumulators of n samples (ops.jacobian_update):
+      p_fold   (D,H,W) fp32  (float)folds / (float)n
+      mean     (D,H,W) fp32  mean of log det J over the n_v = n - folds finite samples, NaN where n_v = 0
+      std      (D,H,W) fp32  sqrt(m2 / (n_v - 1)), unbiased like torch.std, NaN where n_v < 2
+      summary  dict over the voxels of mask: 'sum_folds' (exact; / n = expected number of folded voxels), 'voxels_ever_folded'
+               (folds > 0), 'voxels_folded_in_majority' (2 folds > n), 'voxels_finite' (n_v >= 1), 'voxels_finite_2'
+               (n_v >= 2), 'mask_voxels', 'mean_log_det_J' (mean of the mean map over n_v >= 1), 'mean_std_log_det_J' (mean
+               of the std map over n_v >= 2) -- one host read
+    """
+    lib = _lib.load()
+    _lib.require_cuda(folds, mean, m2, mask)
+    _f32(mean, m2)
+    if folds.dtype != torch.int32:
+        raise NotImplementedError('int32 folds only')
+    V = folds.numel()
+    if mean.numel() != V or m2.numel() != V:
+        raise ValueError('folds, mean and m2 must have the same number of voxels')
+    m8 = _mask_u8(mask, V)
+    dev = folds.device
+    p_fold, mean_out, std_out = (torch.empty(folds.shape, device=dev, dtype=torch.float32) for _ in range(3))
+    partials, counters = jacobian_scratch(1, dev)
+    summary = torch.empty(_lib.JACOBIAN_SUMMARY_WORDS, device=dev, dtype=torch.int64)
+    _lib.check(lib.irs_jacobian_posterior(_lib.ptr(folds), _lib.ptr(mean), _lib.ptr(m2), int(n), V, _lib.ptr(m8),
+                                          _lib.ptr(p_fold), _lib.ptr(mean_out), _lib.ptr(std_out), _lib.ptr(partials),
+                                          _lib.ptr(counters), _lib.ptr(summary), _lib.stream()))
+    s = summary.cpu()
+    words = [int(x) for x in s]
+    means = s[5:7].view(torch.float64).tolist()
+    summ = {'sum_folds': words[0], 'voxels_ever_folded': words[1], 'voxels_folded_in_majority': words[2],
+            'voxels_finite': words[3], 'voxels_finite_2': words[4], 'mask_voxels': words[7],
+            'mean_log_det_J': means[0], 'mean_std_log_det_J': means[1]}
+    return p_fold, mean_out, std_out, summ

@@ -1,8 +1,8 @@
 """
 Multi-GPU: chains shard by rank with no per-iteration communication (SURVEY.md section 8e).  The collectives are the
 merge of the per-rank Welford posterior moments and, when convergence diagnostics are requested, the partial sums of the split
-R-hat -- two sum all-reduces each (NCCL over NVLink on GPUs; gloo in CPU tests) -- and, for the segmentation posterior, one sum
-all-reduce of the integer label counts.
+R-hat -- two sum all-reduces each (NCCL over NVLink on GPUs; gloo in CPU tests) --, for the segmentation posterior, one sum
+all-reduce of the integer label counts, and for the Jacobian posterior two sum all-reduces of its per-voxel Welford moments.
 
 The reference has no distributed code at all; the quantity computed here is its calc_posterior_statistics
 (utils/util.py:114-120: mean and unbiased std over every kept sample of every chain).
@@ -70,6 +70,37 @@ def merge_label_counts(n_local, counts, group=None):
     buf[4:].view_as(counts).copy_(counts)
     dist.all_reduce(buf, op=dist.ReduceOp.SUM, group=group)
     return int(buf[0].item()), buf[4:].view_as(counts)
+
+
+def merge_jacobian_moments(n_local, folds, mean, m2, group=None):
+    """
+    The accumulators of the Jacobian posterior (ops.jacobian_update) over the ranks of `group`: Chan's merge with the per-voxel
+    count n_v = n - folds of finite samples,
+        n_v = sum_r n_v,r ;  mean = sum_r n_v,r mean_r / n_v ;  M2 = sum_r [ M2_r + n_v,r (mean_r - mean)^2 ]
+    in two SUM all-reduces of fp32 buffers in the style of merge_moments: the first carries n in front (padded to 4 floats),
+    n_v and n_v mean, the second the M2 terms.  Integer counts are exact in fp32 below 2^24 samples, so the folds come back
+    exactly as n - sum n_v; mean is 0 where no rank has a finite sample.  Returns (n_total, folds, mean, m2) as new tensors,
+    identical on every rank; the local accumulators are kept, so sampling can continue.  One host read (n_total).
+    """
+    if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) == 1:
+        return int(n_local), folds.clone(), mean.clone(), m2.clone()
+    V = folds.numel()
+    nv_local = (int(n_local) - folds).to(torch.float32)
+    buf = torch.empty(4 + 2 * V, device=mean.device, dtype=torch.float32)
+    buf[:4] = float(n_local)
+    nv, s = buf[4:4 + V].view_as(mean), buf[4 + V:].view_as(mean)
+    nv.copy_(nv_local.view_as(mean))
+    torch.mul(mean, nv, out=s)
+    dist.all_reduce(buf, op=dist.ReduceOp.SUM, group=group)
+    n_total = int(round(float(buf[0].item())))
+    if n_total >= 1 << 24:
+        raise ValueError(f'{n_total} samples: the Jacobian posterior counts are exact below 2^24')
+    mean_t = torch.where(nv > 0, s / nv.clamp(min=1.0), torch.zeros_like(s))
+    d = mean - mean_t
+    m2_t = torch.addcmul(m2, d, d * nv_local.view_as(mean))
+    dist.all_reduce(m2_t, op=dist.ReduceOp.SUM, group=group)
+    folds_t = (n_total - nv.to(torch.int32)).view_as(folds)
+    return n_total, folds_t, mean_t, m2_t
 
 
 def merge_moments(n_local, moments, group=None):

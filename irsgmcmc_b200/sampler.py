@@ -169,6 +169,8 @@ class SGLDSampler:
         self._rhat = None
         # label counts of the segmentation posterior (enable_segmentation_posterior): None while disabled
         self._segpost = None
+        # accumulators of the Jacobian posterior (enable_jacobian_posterior): None while disabled
+        self._jacpost = None
 
     # ------------------------------------------------------------------------------------------------------------------
     def _make_config(self):
@@ -310,6 +312,9 @@ class SGLDSampler:
         if self._segpost is not None:   # segmentation posterior enabled: its label counts travel too
             p = self._segpost
             sd['segpost'] = {'labels': list(p['labels']), 'n': p['n'], 'counts': p['counts'].cpu()}
+        if self._jacpost is not None:   # Jacobian posterior enabled: its accumulators travel too
+            j = self._jacpost
+            sd['jacpost'] = {'n': j['n'], 'folds': j['folds'].cpu(), 'mean': j['mean'].cpu(), 'm2': j['m2'].cpu()}
         return sd
 
     @torch.no_grad()
@@ -339,6 +344,14 @@ class SGLDSampler:
             self._segpost['counts'].copy_(sd['segpost']['counts'])
         elif self._segpost is not None:
             self.enable_segmentation_posterior(self._segpost['labels'])
+        # and for the Jacobian posterior
+        if 'jacpost' in sd:
+            self.enable_jacobian_posterior()
+            self._jacpost['n'] = int(sd['jacpost']['n'])
+            for name in ('folds', 'mean', 'm2'):
+                self._jacpost[name].copy_(sd['jacpost'][name])
+        elif self._jacpost is not None:
+            self.enable_jacobian_posterior()
 
     def set_noise(self, eps=None, jitter_unit=None):
         """explicit N(0,1) / U[0,1) numbers (C,3,D,H,W) instead of Philox: exact noise-on parity tests"""
@@ -523,12 +536,15 @@ class SGLDSampler:
     # ------------------------------------------------------------------------------------------------------------------
     # posterior moments
     # ------------------------------------------------------------------------------------------------------------------
-    def accumulate(self, seg_warped=None):
+    def accumulate(self, seg_warped=None, transformation=None):
         """fold the current sample of every chain into the running moments (kept-sample rule: trainer.py:414-430), when
         convergence diagnostics are enabled into the chain's split-R-hat sequence, and when the segmentation posterior is
         enabled the warped moving segmentation of every chain into its label counts: `seg_warped` (C,1,D,H,W) int16 if the
         caller has it already (warp_segmentation() of the current transformations), else warped here.  Without the
-        segmentation posterior `seg_warped` is not used."""
+        segmentation posterior `seg_warped` is not used.  When the Jacobian posterior is enabled, log det J of every chain's
+        transformation is folded into its accumulators and last_jacobian_stats is overwritten: `transformation` (C,3,D,H,W)
+        fp32 if the caller has it already (transformation() of the current state), else computed here.  Without the Jacobian
+        posterior `transformation` is not used."""
         n3, n1 = 3 * self.V, self.V
         st = _lib.stream()
         if self._rhat is not None and self._rhat['k'] >= self._rhat['N']:
@@ -541,6 +557,14 @@ class SGLDSampler:
             if seg_warped.dtype != torch.int16 or tuple(seg_warped.shape) != (self.C, 1, *self.dims) or \
                     not seg_warped.is_cuda or not seg_warped.is_contiguous():
                 raise ValueError(f'seg_warped must be a contiguous ({self.C}, 1, {", ".join(map(str, self.dims))}) int16 '
+                                 f'CUDA tensor')
+        j = self._jacpost
+        if j is not None:
+            if transformation is None:
+                transformation = self.transformation()
+            if transformation.dtype != torch.float32 or tuple(transformation.shape) != (self.C, 3, *self.dims) or \
+                    not transformation.is_cuda or not transformation.is_contiguous():
+                raise ValueError(f'transformation must be a contiguous ({self.C}, 3, {", ".join(map(str, self.dims))}) fp32 '
                                  f'CUDA tensor')
         _lib.check(self.lib.irs_welford_update(_lib.ptr(self.displacement), self.C, n3, float(self.n_kept),
                                                _lib.ptr(self.disp_mean), _lib.ptr(self.disp_m2), st))
@@ -561,6 +585,13 @@ class SGLDSampler:
             _lib.check(self.lib.irs_label_counts_update(_lib.ptr(seg_warped), self.C, self.V, p['host_labels'],
                                                         len(p['labels']), _lib.ptr(p['counts']), st))
             p['n'] += self.C
+        if j is not None:
+            D, H, W = self.dims
+            _lib.check(self.lib.irs_jacobian_update(_lib.ptr(transformation), _lib.ptr(self.mask), self.C, D, H, W,
+                                                    float(j['n']), _lib.ptr(j['folds']), _lib.ptr(j['mean']),
+                                                    _lib.ptr(j['m2']), _lib.ptr(j['stats']), _lib.ptr(j['partials']),
+                                                    _lib.ptr(j['counters']), st))
+            j['n'] += self.C
 
     def posterior_moments(self, group=None):
         """
@@ -707,3 +738,67 @@ class SGLDSampler:
         prob, majority, entropy, summary = ops.label_posterior(counts, n, p['labels'], seg_fixed)
         return {'labels': list(p['labels']), 'n': n, 'probability': prob, 'majority': majority, 'entropy': entropy,
                 'summary': summary}
+
+    # ------------------------------------------------------------------------------------------------------------------
+    # posterior of the Jacobian determinant (folding probability, mean and std of log det J)
+    # ------------------------------------------------------------------------------------------------------------------
+    @torch.no_grad()
+    def enable_jacobian_posterior(self):
+        """
+        Allocate (or reset) the accumulators of the Jacobian posterior: per voxel the number of folded samples (int32) and
+        the Welford mean / M2 (fp32) of log det J over the finite samples -- 12 V bytes whatever the number of chains, 25 MB
+        at 128^3, 201 MB at 256^3.  accumulate() then also folds log det J of every chain's transformation into them (one
+        launch, no synchronisation; moments, split R-hat, label counts and chain states are unchanged) and keeps the per-chain
+        sums of that sample over the mask in last_jacobian_stats; jacobian_posterior() gives the maps and summaries.
+        """
+        j = self._jacpost
+        if j is None:
+            from . import ops
+            partials, counters = ops.jacobian_scratch(self.C, self.device)
+            z = dict(device=self.device, dtype=torch.float32)
+            self._jacpost = {'n': 0, 'folds': torch.zeros(*self.dims, device=self.device, dtype=torch.int32),
+                             'mean': torch.zeros(*self.dims, **z), 'm2': torch.zeros(*self.dims, **z),
+                             'stats': torch.zeros(self.C, 4, device=self.device, dtype=torch.float64),
+                             'partials': partials, 'counters': counters}
+        else:
+            j['n'] = 0
+            for name in ('folds', 'mean', 'm2', 'stats'):
+                j[name].zero_()
+
+    def disable_jacobian_posterior(self):
+        """free the accumulators; accumulate() no longer computes log det J"""
+        self._jacpost = None
+
+    @property
+    def jacobian_posterior_enabled(self):
+        return self._jacpost is not None
+
+    @property
+    def last_jacobian_stats(self):
+        """(C,4) fp64 device tensor of the latest accumulated sample, per chain over the fixed mask: finite voxels, folded
+        voxels, sum of log det J and of its square over the finite voxels (overwritten by every accumulate(); copy it to keep
+        it).  The population std of log det J over the finite mask voxels, SDlogJ, is sqrt(s2 / n - (s / n)^2).  Registration
+        challenges that report SDlogJ clip det J at 1e-9 instead of leaving the non-positive voxels out."""
+        if self._jacpost is None:
+            raise RuntimeError('the Jacobian posterior is not enabled (enable_jacobian_posterior() before sampling)')
+        return self._jacpost['stats']
+
+    @torch.no_grad()
+    def jacobian_posterior(self, group=None):
+        """
+        The Jacobian posterior over every sample accumulated by ALL ranks of `group` (parallel.merge_jacobian_moments, two SUM
+        all-reduces when torch.distributed is initialised; the local accumulators are kept, so sampling can continue).
+        Returns {'n': samples (kept samples x chains), 'fold_probability', 'log_det_J_mean', 'log_det_J_std': (D,H,W) fp32
+                 device maps (ops.jacobian_posterior: NaN mean where every sample folds, NaN std with fewer than two finite
+                 samples), 'summary': the mask summary of ops.jacobian_posterior}.
+        """
+        from . import ops
+        from .parallel import merge_jacobian_moments
+        j = self._jacpost
+        if j is None:
+            raise RuntimeError('the Jacobian posterior is not enabled (enable_jacobian_posterior() before sampling)')
+        n, folds, mean, m2 = merge_jacobian_moments(j['n'], j['folds'], j['mean'], j['m2'], group)
+        if n < 1:
+            raise RuntimeError('the Jacobian posterior has no accumulated sample yet')
+        p_fold, mean_out, std_out, summary = ops.jacobian_posterior(folds, mean, m2, n, self.mask.view(self.dims))
+        return {'n': n, 'fold_probability': p_fold, 'log_det_J_mean': mean_out, 'log_det_J_std': std_out, 'summary': summary}

@@ -409,7 +409,7 @@ class Trainer:
 
     @torch.no_grad()
     def _test_VI(self, var_params_q_v=None, no_samples=None, modules=None, speed_test_samples=100, with_ASD=True,
-                 with_seg_posterior=False):
+                 with_seg_posterior=False, with_jacobian_posterior=False):
         """
         evaluation of the fitted q(v) (reference trainer.py:226-289): `no_samples_VI_test` draws from q(v) -> Sobolev smoothing ->
         transformation -> number of folded voxels + log det J, warped image and segmentation, ASD / DSC per structure, the sample on
@@ -421,6 +421,9 @@ class Trainer:
         with_seg_posterior=True (needs structures_dict, both segmentations and S >= 1, else ValueError) adds 'seg_posterior',
         the posterior of the warped moving segmentation over the S draws (n = S), with the entries of _run_MCMC's; with
         save_dir, VI_seg_majority.nii.gz and VI_seg_entropy.nii.gz.
+        with_jacobian_posterior=True (S >= 1, else ValueError) adds 'jacobian_posterior', the posterior of log det J over the
+        S draws with the entries of _run_MCMC's ('SDlogJ' and 'folded_fraction' are (S, 1)); with save_dir,
+        VI_log_det_J_mean.nii.gz, VI_log_det_J_std_dev.nii.gz and VI_fold_probability.nii.gz.
         """
         from .. import ops
         from ..utils import SobolevGrad, calc_metrics
@@ -439,6 +442,13 @@ class Trainer:
                                  'one sample')
             seg_labels = [int(x) for x in self.structures_dict.values()]
             seg_counts = torch.zeros(len(seg_labels), *self.dims, device=dev, dtype=torch.int32)
+        if with_jacobian_posterior:
+            if S < 1:
+                raise ValueError('with_jacobian_posterior=True needs at least one sample')
+            jac = {'folds': torch.zeros(*self.dims, device=dev, dtype=torch.int32),
+                   'mean': torch.zeros(*self.dims, device=dev), 'm2': torch.zeros(*self.dims, device=dev),
+                   'mask': self.fixed['mask'].to(dev).view(*self.dims), 'scratch': ops.jacobian_scratch(1, dev)}
+            jac_traces = torch.zeros(S, 1, 4, device=dev, dtype=torch.float64)
         transformation_module, registration_module, diff_op = m['transformation_module'], m['registration_module'], m['reg_loss'].diff_op
 
         def register(v):
@@ -453,6 +463,9 @@ class Trainer:
             count = ops.welford_update(displacement.contiguous(), count, mean, m2)
             n_folded, log_det_J = calc_no_non_diffeomorphic_voxels(transformation, diff_op)
             folded.append(int(n_folded[0]))
+            if with_jacobian_posterior:
+                jac_traces[test_sample_no - 1] = ops.jacobian_update(transformation.contiguous(), jac['mask'], test_sample_no - 1,
+                                                                     jac['folds'], jac['mean'], jac['m2'], jac['scratch'])
             if with_seg:
                 seg_moving_warped = registration_module(moving['seg'], transformation)
                 if with_ASD:
@@ -482,6 +495,10 @@ class Trainer:
             post = {'labels': seg_labels, 'n': S, 'probability': prob, 'majority': majority, 'entropy': entropy,
                     'summary': summary}
             result['seg_posterior'] = self._seg_posterior(post, with_ASD, 'VI')
+        if with_jacobian_posterior:
+            p_fold, mean_ld, std_ld, summary = ops.jacobian_posterior(jac['folds'], jac['mean'], jac['m2'], S, jac['mask'])
+            post = {'n': S, 'fold_probability': p_fold, 'log_det_J_mean': mean_ld, 'log_det_J_std': std_ld, 'summary': summary}
+            result['jacobian_posterior'] = self._jacobian_posterior(post, jac_traces, 'VI', gather=False)
         if speed_test_samples:   # reference trainer.py:275-289
             torch.cuda.synchronize()
             t0 = time.perf_counter()
@@ -547,7 +564,7 @@ class Trainer:
 
     # -- the loop around it (reference trainer.py:358-476) -------------------------------------------------------------
     def _run_MCMC(self, data_loss=None, reg_loss=None, speed_test_iters=100, with_ASD=False, with_R_hat=False,
-                  with_seg_posterior=False):
+                  with_seg_posterior=False, with_jacobian_posterior=False):
         """burn-in + sampling; returns {'mean','std_dev', 'im_mean','im_std', 'n', 'DSC', 'ASD', 'no_non_diffeomorphic_voxels',
         'samples_per_sec'}; posterior statistics are over the kept samples of ALL ranks.  'ASD' (average surface distance,
         reference utils/util.py:171-176 through SimpleITK on the host): with_ASD=True computes it per kept sample on the device
@@ -572,7 +589,17 @@ class Trainer:
         folded into the label counts): the maps 'probability' (L,D,H,W), 'majority' (1,1,D,H,W) int16, 'entropy' (1,D,H,W),
         'labels', 'n', 'summary' (L,3) int64, and 'structures' {name: {'expected_volume' (voxels), 'uncertain_voxels',
         'soft_DSC', 'DSC_majority'[, 'ASD_majority' with with_ASD]}}.  With save_dir, MCMC_seg_majority.nii.gz and
-        MCMC_seg_entropy.nii.gz are written as well.  With with_seg_posterior=False nothing of this runs."""
+        MCMC_seg_entropy.nii.gz are written as well.  With with_seg_posterior=False nothing of this runs.
+
+        with_jacobian_posterior=True adds 'jacobian_posterior', the posterior of log det J of the transformation over every kept
+        sample of every chain of every rank (SGLDSampler.enable_jacobian_posterior; a sample is folded at a voxel where log det
+        J is not finite): the maps 'fold_probability', 'log_det_J_mean', 'log_det_J_std' (D,H,W), 'n', and over the fixed mask
+        'expected_folded_voxels' (sum of the folding probabilities), 'voxels_ever_folded', 'voxels_folded_in_majority',
+        'mean_log_det_J', 'mean_std_log_det_J', plus per kept sample and chain (all ranks' chains) 'SDlogJ', the population std
+        of log det J over the finite mask voxels, and 'folded_fraction', the folded share of the mask, as (kept samples,
+        chains) arrays.  Registration challenges that report SDlogJ clip det J at 1e-9 instead of leaving the non-positive
+        voxels out.  With save_dir, MCMC_log_det_J_mean.nii.gz, MCMC_log_det_J_std_dev.nii.gz and
+        MCMC_fold_probability.nii.gz are written as well.  With with_jacobian_posterior=False nothing of this runs."""
         if self.SGLD_params is None:
             self._SGLD_init()
         s = self.sampler
@@ -580,6 +607,8 @@ class Trainer:
             if not (self.structures_dict and s.moving_seg is not None and 'seg' in self.fixed):
                 raise ValueError('with_seg_posterior=True needs structures_dict and fixed and moving segmentations')
             s.enable_segmentation_posterior(list(self.structures_dict.values()))
+        if with_jacobian_posterior:
+            s.enable_jacobian_posterior()
         if not self._gmm_pushed:
             if data_loss is not None or reg_loss is not None:
                 self._push_hyper(data_loss, reg_loss)
@@ -594,6 +623,11 @@ class Trainer:
             # per kept sample, this rank's rows of the stats (alpha, data, reg, reg energy): a device copy, no synchronisation
             traces = torch.zeros(n_kept, self.no_chains, 4, device=s.device, dtype=torch.float64)
             k_kept = 0
+        if with_jacobian_posterior:
+            # per kept sample, this rank's rows of the Jacobian sums over the mask: a device copy, no synchronisation
+            jac_traces = torch.zeros(sum(1 for i in range(1, total + 1) if self._is_kept(i)), self.no_chains, 4,
+                                     device=s.device, dtype=torch.float64)
+            k_jac = 0
         from ..utils.diff_op import GradientOperator
         diff_op = GradientOperator()
         it = 0
@@ -617,10 +651,13 @@ class Trainer:
                         asd.append(calc_metrics(seg_f, seg_w, self.structures_dict, self.im_spacing, no_samples=self.no_chains)[0])
                 # after the segmentation warp, so that the segmentation posterior reuses it; the transformation and the warp
                 # read what accumulate() reads and write nothing it reads, so the order changes no result
-                s.accumulate(seg_warped=seg_w)
+                s.accumulate(seg_warped=seg_w, transformation=T)
                 if with_R_hat:
                     traces[k_kept].copy_(s.stats[:, :4])
                     k_kept += 1
+                if with_jacobian_posterior:
+                    jac_traces[k_jac].copy_(s.last_jacobian_stats)
+                    k_jac += 1
                 n_folded, log_det_J = calc_no_non_diffeomorphic_voxels(T, diff_op)
                 folded.append(n_folded)
                 if self.save_dir is not None:
@@ -648,6 +685,10 @@ class Trainer:
             post = s.segmentation_posterior(seg_fixed=self.fixed['seg'])
             s.disable_segmentation_posterior()
             result['seg_posterior'] = self._seg_posterior(post, with_ASD, 'MCMC')
+        if with_jacobian_posterior:
+            post = s.jacobian_posterior()
+            s.disable_jacobian_posterior()
+            result['jacobian_posterior'] = self._jacobian_posterior(post, jac_traces, 'MCMC')
         if self.save_dir is not None and (not torch.distributed.is_initialized() or torch.distributed.get_rank() == 0):
             # MCMC_sample_{mean,std_dev}[_masked].vtk like the reference (trainer.py:457-460, logger/logger.py:110-131)
             from ..logger import save_displacement_mean_and_std_dev
@@ -718,6 +759,40 @@ class Trainer:
             sp = [float(x) for x in self.im_spacing]
             save_im_to_disk(majority[0, 0].cpu(), os.path.join(self.save_dir, f'{model}_seg_majority.nii.gz'), sp)
             save_im_to_disk(post['entropy'][0].cpu(), os.path.join(self.save_dir, f'{model}_seg_entropy.nii.gz'), sp)
+        return post
+
+    def _jacobian_posterior(self, post, traces, model, gather=True):
+        """the 'jacobian_posterior' entry of _run_MCMC / _test_VI(with_jacobian_posterior=True) from the dict of
+        SGLDSampler.jacobian_posterior and this rank's per-sample rows (N, C, 4) = (finite, folded, sum ld, sum ld^2) over the
+        mask; with gather, all ranks' rows at their global chain offsets (one SUM all-reduce of a zero-padded buffer, as the
+        R-hat traces).  {model}_log_det_J_mean.nii.gz, {model}_log_det_J_std_dev.nii.gz and {model}_fold_probability.nii.gz
+        in save_dir"""
+        if gather:
+            s = self.sampler
+            allt = torch.zeros(traces.shape[0], self.no_chains_total, 4, device=traces.device, dtype=torch.float64)
+            allt[:, s.chain_offset:s.chain_offset + self.no_chains] = traces
+            if torch.distributed.is_available() and torch.distributed.is_initialized() and \
+                    torch.distributed.get_world_size() > 1:
+                torch.distributed.all_reduce(allt, op=torch.distributed.ReduceOp.SUM)
+            traces = allt
+        t = traces.cpu().numpy()
+        finite, fold, s1, s2 = t[..., 0], t[..., 1], t[..., 2], t[..., 3]
+        with np.errstate(divide='ignore', invalid='ignore'):
+            m = s1 / finite
+            post['SDlogJ'] = np.sqrt(np.maximum(s2 / finite - m * m, 0.0))   # population std; NaN without a finite voxel
+            post['folded_fraction'] = fold / (finite + fold)
+        summ = post['summary']
+        post['expected_folded_voxels'] = summ['sum_folds'] / post['n']
+        for key in ('voxels_ever_folded', 'voxels_folded_in_majority', 'mean_log_det_J', 'mean_std_log_det_J'):
+            post[key] = summ[key]
+        if self.save_dir is not None and (not torch.distributed.is_initialized() or torch.distributed.get_rank() == 0):
+            import os
+            from ..logger import save_im_to_disk
+            os.makedirs(self.save_dir, exist_ok=True)
+            sp = [float(x) for x in self.im_spacing]
+            for key, name in (('log_det_J_mean', 'log_det_J_mean'), ('log_det_J_std', 'log_det_J_std_dev'),
+                              ('fold_probability', 'fold_probability')):
+                save_im_to_disk(post[key].cpu(), os.path.join(self.save_dir, f'{model}_{name}.nii.gz'), sp)
         return post
 
     def _is_kept(self, sample_no):
