@@ -168,6 +168,70 @@ void emul_reg_hyper_step(double* hyper, const double* cfg_d, int C, double* stat
     irs_reg_hyper_step(hyper, cfg, C, stats);
 }
 
+// the warp of the fused step (csrc/irs_warp.cu warp_vox_fwd_kernel<true>): position_from_u's arithmetic with explicit
+// jitter r (C,3,V; nullptr: none), then irs_inside, the clamp, irs_cell and irs_interp_grad
+void emul_warp_vox(const float* img, const float* u, const float* r, float alpha, float* out, float* grad, int C, int D,
+                   int H, int W) {
+    IrsDims d{D, H, W};
+    const long long V = d.V();
+    for (int c = 0; c < C; ++c)
+        for (long long i = 0; i < V; ++i) {
+            int x, y, z;
+            irs_voxel_xyz(i, d, x, y, z);
+            const float* uc = u + (size_t)c * 3 * V;
+            float px = (float)x + uc[i], py = (float)y + uc[V + i], pz = (float)z + uc[2 * V + i];
+            if (r != nullptr) {
+                const float* rc = r + (size_t)c * 3 * V;
+                px += alpha - 2.0f * alpha * rc[i];
+                py += alpha - 2.0f * alpha * rc[V + i];
+                pz += alpha - 2.0f * alpha * rc[2 * V + i];
+            }
+            const float mx = irs_inside(px, W), my = irs_inside(py, H), mz = irs_inside(pz, D);
+            const IrsCell cell = irs_cell(irs_clampf(px, 0.f, (float)(W - 1)), irs_clampf(py, 0.f, (float)(H - 1)),
+                                          irs_clampf(pz, 0.f, (float)(D - 1)), d);
+            float dx, dy, dz;
+            out[(size_t)c * V + i] = irs_interp_grad(cell, [&](int k) { return img[k]; }, dx, dy, dz);
+            float* g = grad + (size_t)c * 3 * V;
+            g[i] = dx * mx; g[V + i] = dy * my; g[2 * V + i] = dz * mz;
+        }
+}
+
+// one voxel of gmm_grad_kernel: irs_gmm_eval_t<kk> (kk = 4 or IRS_MAX_K) with a table of lw[8], prec[8]; g = alpha z wprec
+// and log p on the mask, 0 off it
+void emul_gmm_grad(const float* z, const unsigned char* mask, const float* table, int K, int kk, float alpha, float* g,
+                   float* lp, long long n) {
+    IrsGmm gm;
+    gm.K = K;
+    for (int k = 0; k < IRS_MAX_K; ++k) { gm.lw[k] = table[k]; gm.prec[k] = table[IRS_MAX_K + k]; }
+    for (long long i = 0; i < n; ++i) {
+        float rho[IRS_MAX_K], wp;
+        const float l = kk == 4 ? irs_gmm_eval_t<4>(gm, z[i], rho, wp) : irs_gmm_eval_t<IRS_MAX_K>(gm, z[i], rho, wp);
+        g[i] = mask[i] ? alpha * z[i] * wp : 0.f;
+        lp[i] = mask[i] ? l : 0.f;
+    }
+}
+
+// sgd_update_kernel for one chain (3,D,H,W): grad_v = sigma^2 (g_css + k dE/dcss), v -= tau grad_v (sigma nullptr: 1)
+void emul_sgd_update(float* v, const float* sigma, const float* css, const float* g_css, float k, float tau, float* grad_v,
+                     int D, int H, int W) {
+    IrsDims d{D, H, W};
+    const long long V = d.V(), sy = W, sz = (long long)W * H;
+    for (int ch = 0; ch < 3; ++ch)
+        for (long long i = 0; i < V; ++i) {
+            int x, y, z;
+            irs_voxel_xyz(i, d, x, y, z);
+            const size_t o = (size_t)ch * V + i;
+            const float* f = css + (size_t)ch * V;
+            const float ge = irs_diff_energy_grad(x > 0 ? f[i - 1] : 0.f, f[i], x < W - 1 ? f[i + 1] : 0.f, x, W)
+                           + irs_diff_energy_grad(y > 0 ? f[i - sy] : 0.f, f[i], y < H - 1 ? f[i + sy] : 0.f, y, H)
+                           + irs_diff_energy_grad(z > 0 ? f[i - sz] : 0.f, f[i], z < D - 1 ? f[i + sz] : 0.f, z, D);
+            const float sg = sigma ? sigma[o] : 1.f;
+            const float g = sg * sg * (g_css[o] + k * ge);
+            grad_v[o] = g;
+            v[o] -= tau * g;
+        }
+}
+
 void emul_normal3(unsigned long long seed, int n, int chain, unsigned long long iter, float* out) {
     for (int i = 0; i < n; ++i) irs_normal3(seed, (uint32_t)i, (uint32_t)chain, iter, out + 3 * (size_t)i);
 }
