@@ -192,6 +192,25 @@ int irs_average_surface_distance(const short* seg_a, long long a_chain_stride, c
                                  int pair_end, float* workspace, long long workspace_floats, double* partials,
                                  unsigned int* counters, double* asd, int C, int D, int H, int W, void* stream);
 
+/* Hausdorff distance and its percentile, with the average surface distance of the same distance transform.  For the pair
+ * (A, B) above, d_AB = the distances from the contour voxels of A to the contour of B (a multiset), d_BA the same from B to A:
+ *   hd[p]   = max(max d_AB, max d_BA)                        (ITK HausdorffDistanceImageFilter on the contour images)
+ *   hd_q[p] = max(P_q(d_AB), P_q(d_BA)), P_q = numpy.percentile(x, q), method 'linear': s sorted, h = (n - 1) (q / 100) in
+ *             fp64, s[n - 1] when h >= n - 1, else s[i] + (s[i+1] - s[i]) g for g = h - i < 0.5 (i = floor(h)) and
+ *             s[i+1] - (s[i+1] - s[i]) (1 - g) otherwise -- every element counts once, not weighted by surface area
+ *   asd[p]  = bit-identical to irs_average_surface_distance
+ * inf when A or B is empty, 0 when A == B.  The order statistics are selected on the fp32 squared distances (exact for unit and
+ * dyadic spacings), then square-rooted and interpolated in fp64.  percentile in [0, 100] (else IRS_ERR_BAD_ARG, NaN included);
+ * workspace >= 2 * (box voxels) + |A| + |B| floats (boxes[6], boxes[7]) summed over the non-empty pairs of the range, else
+ * IRS_ERR_WORKSPACE; partials IRS_ASD_PARTIALS_DOUBLES doubles; counters IRS_SD_COUNTERS unsigned.  Deterministic: integer
+ * atomics only, results independent of the batching of the pairs; no host synchronisation. */
+#define IRS_SD_COUNTERS (3 * IRS_ASD_MAX_BOXES)
+int irs_surface_distances(const short* seg_a, long long a_chain_stride, const short* seg_b, const int* labels_host,
+                          int n_labels, const int* boxes_host, const float* spacing_host, double percentile, int pair_begin,
+                          int pair_end, float* workspace, long long workspace_floats, double* partials,
+                          unsigned int* counters, double* asd, double* hd, double* hd_q, int C, int D, int H, int W,
+                          void* stream);
+
 /* ------------------------------------------------------------------------------------------------------------------ *
  * Posterior moments -- replaces calc_posterior_statistics (utils/util.py:114-120) without the host-side sample buffer:
  * Welford running (count, mean, M2) over samples; count is a host-side number.

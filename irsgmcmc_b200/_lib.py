@@ -76,6 +76,8 @@ class ViBuffers(ctypes.Structure):
 
 # average surface distance scratch (include/irsgmcmc.h): IRS_ASD_MAX_BOXES counters, IRS_ASD_PARTIALS_DOUBLES partials
 ASD_MAX_BOXES, ASD_PARTIALS_DOUBLES = 48, 48 * 4 * 64
+# Hausdorff distance (include/irsgmcmc.h): IRS_SD_COUNTERS counters (the ASD tickets and the two list lengths per box)
+SD_COUNTERS = 3 * ASD_MAX_BOXES
 
 # split R-hat (include/irsgmcmc.h): components per launch, reduction scratch
 RHAT_MAX_COMPONENTS, RHAT_PARTIALS_DOUBLES = 4, 4 * 3 * 256
@@ -120,6 +122,8 @@ SYMBOLS = {
     'irs_surface_boxes': (_i, [_vp, _ll, _vp, _vp, _i, _vp, _i, _i, _i, _i, _vp]),
     'irs_average_surface_distance': (_i, [_vp, _ll, _vp, _vp, _i, _vp, _vp, _i, _i, _vp, _ll, _vp, _vp, _vp, _i, _i, _i, _i,
                                           _vp]),
+    'irs_surface_distances': (_i, [_vp, _ll, _vp, _vp, _i, _vp, _vp, _d, _i, _i, _vp, _ll, _vp, _vp, _vp, _vp, _vp, _i, _i, _i,
+                                   _i, _vp]),
     'irs_welford_update': (_i, [_vp, _i, _ll, _d, _vp, _vp, _vp]),
     'irs_welford_std': (_i, [_vp, _d, _vp, _ll, _vp]),
     'irs_split_welford_update': (_i, [_vp, _vp, _i, _ll, _i, _d, _vp, _vp, _vp]),

@@ -3,7 +3,10 @@
 //   box pass     bounding box of A u B and |A|, |B| for every (sample, label) in one pass over the volumes
 //   three passes the exact separable Euclidean distance transform over every box (W, then H, then D), both directions at once:
 //                channel 0 = squared distance to the contour of B, channel 1 = to the contour of A
-//   reduction    the two directed means over the contour voxels, block partials summed in a fixed order (no float atomics)
+//   reduction    the two directed means over the contour voxels, block partials summed in a fixed order (no float atomics);
+//                for the Hausdorff distance it also appends every contour voxel's squared distance to a list per (pair, direction)
+//   selection    (Hausdorff distance only) one CTA per list: maximum and the percentile's ranks by an MSB-first radix select
+//                over the fp32 bit patterns (irs_select.cuh)
 // Contour (ITK LabelContourImageFilter, FullyConnectedOff): a voxel of the set with one of its 6 face neighbours outside the set,
 // where outside the volume counts as outside.  The box holds every voxel of A and B, so "outside the box" is "outside the set",
 // and an exact transform over the box is exact for every contour voxel: no margin is needed.
@@ -12,6 +15,7 @@
 
 #include "irs_kernels.cuh"
 #include "irs_edt.cuh"
+#include "irs_select.cuh"
 
 namespace {
 
@@ -86,6 +90,7 @@ struct AsdBox {
     long long off;            // first float of the box in the workspace: channel 0 then channel 1, each (nd, nh, nw)
     int c, label, pair;       // sample, label value, index into asd[]
     int z0, y0, x0, nd, nh, nw;
+    int cap_a;                // Hausdorff lists after the two channels: |A| floats (contour of A), then |B| floats
 };
 
 struct AsdGroup {
@@ -180,9 +185,24 @@ edt_envelope_kernel(float* __restrict__ ws, const __grid_constant__ AsdGroup G, 
 // ASD = (mean over the contour of A of the distance to the contour of B + the same from B to A) / 2.  A voxel is on the
 // contour of B exactly when its channel-0 distance is 0 (spacings are positive), and likewise for A: the flags need no
 // second look at the volumes.  Per box: reduce_blocks() blocks, each a fixed-order partial; the last to arrive adds them up.
+// LISTS (Hausdorff distance): every contour voxel of A also appends its squared distance to the contour of B to the box's list
+// AB, and the same from B to A; the slots come from one integer atomicAdd per warp, so the list order varies from run to run
+// while the sums (each thread's sequence of voxels is the same in both variants) and every order statistic do not.
+__device__ __forceinline__ void list_append(bool on, float key, float* list, unsigned int* count, int lane) {
+    const unsigned m = __ballot_sync(0xffffffffu, on);
+    if (m == 0u) return;
+    const int leader = __ffs(m) - 1;
+    unsigned base = 0u;
+    if (lane == leader) base = atomicAdd(count, (unsigned)__popc(m));
+    base = __shfl_sync(0xffffffffu, base, leader);
+    if (on) list[base + __popc(m & ((1u << lane) - 1u))] = key;
+}
+
+template <bool LISTS>
 __global__ void __launch_bounds__(256)
-asd_reduce_kernel(const float* __restrict__ ws, const __grid_constant__ AsdGroup G, double* __restrict__ partials,
-                  unsigned int* __restrict__ counters, double* __restrict__ asd) {
+asd_reduce_kernel(float* __restrict__ ws, const __grid_constant__ AsdGroup G, double* __restrict__ partials,
+                  unsigned int* __restrict__ counters, double* __restrict__ asd, double* __restrict__ hd,
+                  double* __restrict__ hd_q) {
     __shared__ double sh[4 * 8];
     __shared__ bool last;
     const AsdBox& B = G.b[blockIdx.y];
@@ -191,13 +211,31 @@ asd_reduce_kernel(const float* __restrict__ ws, const __grid_constant__ AsdGroup
     if ((int)blockIdx.x >= nb) return;
     const float* d0 = ws + B.off;
     const float* d1 = d0 + nvox;
-    double v[4] = {0.0, 0.0, 0.0, 0.0};   // sum over cA of d(., cB), |cA|, sum over cB of d(., cA), |cB|
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < nvox; i += (long long)nb * blockDim.x) {
-        const float a = d0[i], b = d1[i];
-        if (b == 0.0f) { v[0] += sqrt((double)a); v[1] += 1.0; }
-        if (a == 0.0f) { v[2] += sqrt((double)b); v[3] += 1.0; }
-    }
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    double v[4] = {0.0, 0.0, 0.0, 0.0};   // sum over cA of d(., cB), |cA|, sum over cB of d(., cA), |cB|
+    if (LISTS) {
+        float* list_ab = ws + B.off + 2 * nvox;
+        float* list_ba = list_ab + B.cap_a;
+        unsigned int* n_ab = counters + IRS_ASD_MAX_BOXES + blockIdx.y;
+        unsigned int* n_ba = n_ab + IRS_ASD_MAX_BOXES;
+        // warp-uniform trip count for the warp-wide slot allocation; each thread visits the voxels of the loop below
+        for (long long base = (long long)blockIdx.x * blockDim.x + (threadIdx.x - lane); base < nvox;
+             base += (long long)nb * blockDim.x) {
+            const long long i = base + lane;
+            float a = 1.0f, b = 1.0f;
+            if (i < nvox) { a = d0[i]; b = d1[i]; }
+            if (b == 0.0f) { v[0] += sqrt((double)a); v[1] += 1.0; }
+            if (a == 0.0f) { v[2] += sqrt((double)b); v[3] += 1.0; }
+            list_append(b == 0.0f, a, list_ab, n_ab, lane);
+            list_append(a == 0.0f, b, list_ba, n_ba, lane);
+        }
+    } else {
+        for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < nvox; i += (long long)nb * blockDim.x) {
+            const float a = d0[i], b = d1[i];
+            if (b == 0.0f) { v[0] += sqrt((double)a); v[1] += 1.0; }
+            if (a == 0.0f) { v[2] += sqrt((double)b); v[3] += 1.0; }
+        }
+    }
 #pragma unroll
     for (int k = 0; k < 4; ++k) {
         const double s = irs_warp_sum(v[k]);
@@ -224,7 +262,93 @@ asd_reduce_kernel(const float* __restrict__ ws, const __grid_constant__ AsdGroup
         tot[k] = s;
     }
     asd[B.pair] = 0.5 * (tot[0] / tot[1] + tot[2] / tot[3]);
+    if (LISTS) hd[B.pair] = hd_q[B.pair] = 0.0;   // the selection raises them with integer maxima
     counters[blockIdx.y] = 0u;
+}
+
+// Hausdorff distance: one CTA per (box, direction) list of n squared distances (blockIdx.x = 0: contour of A to B, 1: B to A).
+// Four MSB-first passes of IRS_SELECT_BITS bits find the key at rank i of the percentile (shared-memory histograms, lanes with
+// the same digit merged into one integer atomicAdd); rank i + 1 is that key again when more than i + 1 keys are <= it, else the
+// smallest key above it (one more pass, a block minimum).  The first pass also takes the list's maximum.  The two directions
+// meet in integer atomicMax on the fp64 bit patterns of the non-negative results: HD = max of the maxima, HD_q = max of the
+// directed percentiles, independent of which CTA comes first.  The list's count is reset for the next launch group.
+constexpr int kSelectThreads = 512;
+
+__global__ void __launch_bounds__(kSelectThreads)
+hd_select_kernel(const float* __restrict__ ws, const __grid_constant__ AsdGroup G, unsigned int* __restrict__ counters,
+                 double q, double* __restrict__ hd, double* __restrict__ hd_q) {
+    __shared__ unsigned int hist[IRS_SELECT_BINS];
+    __shared__ unsigned int sh_bin, sh_r, sh_eq, sh_max, sh_min;
+    const AsdBox& B = G.b[blockIdx.y];
+    const int dir = blockIdx.x, t = threadIdx.x, lane = t & 31, warp = t >> 5;
+    const long long nvox = box_voxels(B);
+    const unsigned int* keys = reinterpret_cast<const unsigned int*>(ws + B.off + 2 * nvox + (dir ? B.cap_a : 0));
+    unsigned int* count = counters + IRS_ASD_MAX_BOXES * (1 + dir) + blockIdx.y;
+    const unsigned int n = __ldcg(count);
+    if (n == 0u) return;   // not reached: a non-empty set has a contour
+    const IrsPercentileRank pr = irs_percentile_rank(n, q);
+    if (t == 0) { sh_max = 0u; sh_min = 0xffffffffu; }
+    unsigned int prefix = 0u, mask = 0u, r = pr.i, mx = 0u;
+    for (int shift = 32 - IRS_SELECT_BITS; shift >= 0; shift -= IRS_SELECT_BITS) {
+        for (int k = t; k < IRS_SELECT_BINS; k += kSelectThreads) hist[k] = 0u;
+        __syncthreads();
+        for (unsigned int base = t - lane; base < n; base += kSelectThreads) {   // warp-uniform: lanes merge below
+            const unsigned int k = base + lane;
+            int bin = -1;
+            if (k < n) {
+                const unsigned int v = __ldcg(keys + k);
+                if (shift == 32 - IRS_SELECT_BITS) mx = max(mx, v);
+                if ((v & mask) == prefix) bin = (int)((v >> shift) & (IRS_SELECT_BINS - 1));
+            }
+            const unsigned peers = __match_any_sync(0xffffffffu, bin);
+            if (bin >= 0 && lane == __ffs(peers) - 1) atomicAdd(hist + bin, (unsigned)__popc(peers));
+        }
+        __syncthreads();
+        if (warp == 0) {   // lane l owns bins [8 l, 8 l + 8): the lane where the cumulative count passes r walks its bins
+            constexpr int per = IRS_SELECT_BINS / 32;
+            unsigned int s = 0u;
+#pragma unroll
+            for (int k = 0; k < per; ++k) s += hist[lane * per + k];
+            unsigned int incl = s;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const unsigned int u = __shfl_up_sync(0xffffffffu, incl, o);
+                if (lane >= o) incl += u;
+            }
+            const unsigned int excl = incl - s;
+            if (excl <= r && r < incl) {
+                unsigned int rr = r - excl;
+                const int bin = lane * per + irs_select_bin(hist + lane * per, per, &rr);
+                sh_bin = (unsigned)bin;
+                sh_r = rr;
+                sh_eq = hist[bin];
+            }
+        }
+        __syncthreads();
+        prefix |= sh_bin << shift;
+        mask |= (unsigned int)(IRS_SELECT_BINS - 1) << shift;
+        r = sh_r;
+    }
+    mx = __reduce_max_sync(0xffffffffu, mx);
+    if (lane == 0) atomicMax(&sh_max, mx);
+    const bool above = !pr.last && pr.i + 1 >= pr.i - r + sh_eq;   // keys <= rank i's key: (i - r) below it, sh_eq equal to it
+    if (above) {
+        unsigned int m = 0xffffffffu;
+        for (unsigned int k = t; k < n; k += kSelectThreads) {
+            const unsigned int v = __ldcg(keys + k);
+            if (v > prefix) m = min(m, v);
+        }
+        m = __reduce_min_sync(0xffffffffu, m);
+        if (lane == 0) atomicMin(&sh_min, m);
+    }
+    __syncthreads();
+    if (t != 0) return;
+    const unsigned int next = above ? sh_min : prefix;
+    const double p = irs_percentile_value(__uint_as_float(prefix), __uint_as_float(next), pr);
+    const double h = sqrt((double)__uint_as_float(sh_max));
+    atomicMax(reinterpret_cast<unsigned long long*>(hd_q + B.pair), (unsigned long long)__double_as_longlong(p));
+    atomicMax(reinterpret_cast<unsigned long long*>(hd + B.pair), (unsigned long long)__double_as_longlong(h));
+    *count = 0u;
 }
 
 __global__ void fill_kernel(double* __restrict__ x, int n, double value) {
@@ -234,8 +358,15 @@ __global__ void fill_kernel(double* __restrict__ x, int n, double value) {
 
 bool bad_spacing(float s) { return !(s > 0.0f) || !(s * s >= FLT_MIN) || !(s * s <= FLT_MAX); }
 
+// the Hausdorff outputs of irs_surface_distances; hd == nullptr: the average surface distance alone
+struct HdOut {
+    double q;
+    double* hd;
+    double* hd_q;
+};
+
 int launch_group(const short* seg_a, long long a_cs, const short* seg_b, IrsDims d, const AsdGroup& G, const float* w,
-                 float* ws, double* partials, unsigned int* counters, double* asd, cudaStream_t st) {
+                 float* ws, double* partials, unsigned int* counters, double* asd, const HdOut& hd, cudaStream_t st) {
     if (G.n == 0) return IRS_OK;
     const long long rows = G.line0[0][G.n];
     edt_rows_kernel<<<(unsigned)((rows + 127) / 128), 128, 0, st>>>(seg_a, a_cs, seg_b, d, G, ws, w[0]);
@@ -260,9 +391,83 @@ int launch_group(const short* seg_a, long long a_cs, const short* seg_b, IrsDims
     }
     int nb = 1;
     for (int k = 0; k < G.n; ++k) nb = max(nb, reduce_blocks(box_voxels(G.b[k])));
-    asd_reduce_kernel<<<dim3(nb, G.n), 256, 0, st>>>(ws, G, partials, counters, asd);
+    if (!hd.hd) {
+        asd_reduce_kernel<false><<<dim3(nb, G.n), 256, 0, st>>>(ws, G, partials, counters, asd, nullptr, nullptr);
+        IRS_LAUNCH_CHECK();
+        return IRS_OK;
+    }
+    asd_reduce_kernel<true><<<dim3(nb, G.n), 256, 0, st>>>(ws, G, partials, counters, asd, hd.hd, hd.hd_q);
+    IRS_LAUNCH_CHECK();
+    hd_select_kernel<<<dim3(2, G.n), kSelectThreads, 0, st>>>(ws, G, counters, hd.q, hd.hd, hd.hd_q);
     IRS_LAUNCH_CHECK();
     return IRS_OK;
+}
+
+// both entry points: validation before any CUDA call, then the pairs of the range in launch groups of IRS_ASD_MAX_BOXES boxes
+int surface_distances(const short* seg_a, long long a_chain_stride, const short* seg_b, const int* labels_host, int n_labels,
+                      const int* boxes_host, const float* spacing_host, int pair_begin, int pair_end, float* workspace,
+                      long long workspace_floats, double* partials, unsigned int* counters, double* asd, const HdOut& hd,
+                      int C, int D, int H, int W, void* stream) {
+    IRS_CHECK_DIMS(C, D, H, W);
+    if (!seg_a || !seg_b || !labels_host || !boxes_host || !spacing_host || !partials || !counters || !asd ||
+        n_labels < 1 || n_labels > 32 || pair_begin < 0 || pair_end < pair_begin || pair_end > C * n_labels)
+        return IRS_ERR_BAD_ARG;
+    for (int i = 0; i < n_labels; ++i)
+        if (labels_host[i] == 0) return IRS_ERR_UNSUPPORTED;
+    for (int k = 0; k < 3; ++k)
+        if (bad_spacing(spacing_host[k])) return IRS_ERR_BAD_ARG;
+    const bool lists = hd.hd != nullptr;
+    // spacing is (x, y, z): the W axis is weighted by spacing[0]^2
+    const float w[3] = {spacing_host[0] * spacing_host[0], spacing_host[1] * spacing_host[1], spacing_host[2] * spacing_host[2]};
+    long long need = 0;
+    for (int p = pair_begin; p < pair_end; ++p) {
+        const int* bx = boxes_host + (size_t)p * kBox;
+        if (bx[6] <= 0 || bx[7] <= 0) continue;
+        if (bx[0] < 0 || bx[1] < 0 || bx[2] < 0 || bx[0] > bx[3] || bx[1] > bx[4] || bx[2] > bx[5] || bx[3] >= D ||
+            bx[4] >= H || bx[5] >= W)
+            return IRS_ERR_BAD_ARG;
+        need += 2LL * (bx[3] - bx[0] + 1) * (bx[4] - bx[1] + 1) * (bx[5] - bx[2] + 1);
+        // the contour of A is a subset of A: |A| + |B| floats hold both lists
+        if (lists) need += (long long)bx[6] + bx[7];
+    }
+    if (need > workspace_floats || (need > 0 && !workspace)) return IRS_ERR_WORKSPACE;
+    if (pair_end == pair_begin) return IRS_OK;
+    cudaStream_t st = (cudaStream_t)stream;
+    cudaError_t e = cudaMemsetAsync(counters, 0, sizeof(unsigned int) * (lists ? IRS_SD_COUNTERS : IRS_ASD_MAX_BOXES), st);
+    if (e != cudaSuccess) return (int)e;
+    // an empty structure on either side gives inf (the reference's `except: ASD = inf`); the others are overwritten below
+    const int n_pairs = pair_end - pair_begin;
+    for (double* out : {asd, hd.hd, hd.hd_q}) {
+        if (!out) continue;
+        fill_kernel<<<(n_pairs + 255) / 256, 256, 0, st>>>(out + pair_begin, n_pairs, (double)INFINITY);
+        IRS_LAUNCH_CHECK();
+    }
+    IrsDims d{D, H, W};
+    AsdGroup G;
+    G.n = 0;
+    long long off = 0;
+    for (int p = pair_begin; p < pair_end; ++p) {
+        const int* bx = boxes_host + (size_t)p * kBox;
+        if (bx[6] <= 0 || bx[7] <= 0) continue;
+        if (G.n == 0) G.line0[0][0] = G.line0[1][0] = G.line0[2][0] = 0;
+        AsdBox& B = G.b[G.n];
+        B.off = off;
+        B.c = p / n_labels;
+        B.label = labels_host[p % n_labels];
+        B.pair = p;
+        B.z0 = bx[0]; B.y0 = bx[1]; B.x0 = bx[2];
+        B.nd = bx[3] - bx[0] + 1; B.nh = bx[4] - bx[1] + 1; B.nw = bx[5] - bx[2] + 1;
+        B.cap_a = bx[6];
+        off += 2 * box_voxels(B) + (lists ? (long long)bx[6] + bx[7] : 0LL);
+        G.line0[0][G.n + 1] = G.line0[0][G.n] + (long long)B.nd * B.nh;
+        G.line0[1][G.n + 1] = G.line0[1][G.n] + 2LL * B.nd * B.nw;
+        G.line0[2][G.n + 1] = G.line0[2][G.n] + 2LL * B.nh * B.nw;
+        if (++G.n == IRS_ASD_MAX_BOXES) {
+            IRS_TRY(launch_group(seg_a, a_chain_stride, seg_b, d, G, w, workspace, partials, counters, asd, hd, st));
+            G.n = 0;
+        }
+    }
+    return launch_group(seg_a, a_chain_stride, seg_b, d, G, w, workspace, partials, counters, asd, hd, st);
 }
 
 }  // namespace
@@ -292,57 +497,18 @@ extern "C" int irs_average_surface_distance(const short* seg_a, long long a_chai
                                             const float* spacing_host, int pair_begin, int pair_end, float* workspace,
                                             long long workspace_floats, double* partials, unsigned int* counters,
                                             double* asd, int C, int D, int H, int W, void* stream) {
-    IRS_CHECK_DIMS(C, D, H, W);
-    if (!seg_a || !seg_b || !labels_host || !boxes_host || !spacing_host || !partials || !counters || !asd ||
-        n_labels < 1 || n_labels > 32 || pair_begin < 0 || pair_end < pair_begin || pair_end > C * n_labels)
-        return IRS_ERR_BAD_ARG;
-    for (int i = 0; i < n_labels; ++i)
-        if (labels_host[i] == 0) return IRS_ERR_UNSUPPORTED;
-    for (int k = 0; k < 3; ++k)
-        if (bad_spacing(spacing_host[k])) return IRS_ERR_BAD_ARG;
-    // spacing is (x, y, z): the W axis is weighted by spacing[0]^2
-    const float w[3] = {spacing_host[0] * spacing_host[0], spacing_host[1] * spacing_host[1], spacing_host[2] * spacing_host[2]};
-    long long need = 0;
-    for (int p = pair_begin; p < pair_end; ++p) {
-        const int* bx = boxes_host + (size_t)p * kBox;
-        if (bx[6] <= 0 || bx[7] <= 0) continue;
-        if (bx[0] < 0 || bx[1] < 0 || bx[2] < 0 || bx[0] > bx[3] || bx[1] > bx[4] || bx[2] > bx[5] || bx[3] >= D ||
-            bx[4] >= H || bx[5] >= W)
-            return IRS_ERR_BAD_ARG;
-        need += 2LL * (bx[3] - bx[0] + 1) * (bx[4] - bx[1] + 1) * (bx[5] - bx[2] + 1);
-    }
-    if (need > workspace_floats || (need > 0 && !workspace)) return IRS_ERR_WORKSPACE;
-    if (pair_end == pair_begin) return IRS_OK;
-    cudaStream_t st = (cudaStream_t)stream;
-    cudaError_t e = cudaMemsetAsync(counters, 0, sizeof(unsigned int) * IRS_ASD_MAX_BOXES, st);
-    if (e != cudaSuccess) return (int)e;
-    // an empty structure on either side gives inf (the reference's `except: ASD = inf`); the others are overwritten below
-    const int n_pairs = pair_end - pair_begin;
-    fill_kernel<<<(n_pairs + 255) / 256, 256, 0, st>>>(asd + pair_begin, n_pairs, (double)INFINITY);
-    IRS_LAUNCH_CHECK();
-    IrsDims d{D, H, W};
-    AsdGroup G;
-    G.n = 0;
-    long long off = 0;
-    for (int p = pair_begin; p < pair_end; ++p) {
-        const int* bx = boxes_host + (size_t)p * kBox;
-        if (bx[6] <= 0 || bx[7] <= 0) continue;
-        if (G.n == 0) G.line0[0][0] = G.line0[1][0] = G.line0[2][0] = 0;
-        AsdBox& B = G.b[G.n];
-        B.off = off;
-        B.c = p / n_labels;
-        B.label = labels_host[p % n_labels];
-        B.pair = p;
-        B.z0 = bx[0]; B.y0 = bx[1]; B.x0 = bx[2];
-        B.nd = bx[3] - bx[0] + 1; B.nh = bx[4] - bx[1] + 1; B.nw = bx[5] - bx[2] + 1;
-        off += 2 * box_voxels(B);
-        G.line0[0][G.n + 1] = G.line0[0][G.n] + (long long)B.nd * B.nh;
-        G.line0[1][G.n + 1] = G.line0[1][G.n] + 2LL * B.nd * B.nw;
-        G.line0[2][G.n + 1] = G.line0[2][G.n] + 2LL * B.nh * B.nw;
-        if (++G.n == IRS_ASD_MAX_BOXES) {
-            IRS_TRY(launch_group(seg_a, a_chain_stride, seg_b, d, G, w, workspace, partials, counters, asd, st));
-            G.n = 0;
-        }
-    }
-    return launch_group(seg_a, a_chain_stride, seg_b, d, G, w, workspace, partials, counters, asd, st);
+    return surface_distances(seg_a, a_chain_stride, seg_b, labels_host, n_labels, boxes_host, spacing_host, pair_begin,
+                             pair_end, workspace, workspace_floats, partials, counters, asd, HdOut{0.0, nullptr, nullptr}, C,
+                             D, H, W, stream);
+}
+
+extern "C" int irs_surface_distances(const short* seg_a, long long a_chain_stride, const short* seg_b,
+                                     const int* labels_host, int n_labels, const int* boxes_host, const float* spacing_host,
+                                     double percentile, int pair_begin, int pair_end, float* workspace,
+                                     long long workspace_floats, double* partials, unsigned int* counters, double* asd,
+                                     double* hd, double* hd_q, int C, int D, int H, int W, void* stream) {
+    if (!hd || !hd_q || !(percentile >= 0.0 && percentile <= 100.0)) return IRS_ERR_BAD_ARG;
+    return surface_distances(seg_a, a_chain_stride, seg_b, labels_host, n_labels, boxes_host, spacing_host, pair_begin,
+                             pair_end, workspace, workspace_floats, partials, counters, asd, HdOut{percentile, hd, hd_q}, C,
+                             D, H, W, stream);
 }

@@ -468,6 +468,25 @@ def average_surface_distance(seg_a, seg_b, labels, spacing, workspace_bytes=512 
     1, 1, D, H, W); seg_a may be one volume shared by all samples; spacing (x, y, z).  The distance transforms run over the
     bounding box of each (sample, structure), 8 bytes per box voxel, in batches of pairs whose workspace fits
     `workspace_bytes` (a pair larger than that runs alone).  One host synchronisation per 32 labels (the box table)."""
+    return _surface_distances(seg_a, seg_b, labels, spacing, workspace_bytes, None)[0]
+
+
+def surface_distances(seg_a, seg_b, labels, spacing, percentile=95.0, workspace_bytes=512 << 20):
+    """float64 (asd, hd, hd_q), each (C, n_labels), of the structures A = seg_a == l and B = seg_b[c] == l from one distance
+    transform: asd is average_surface_distance's to the bit; hd = max(max d_AB, max d_BA) is the Hausdorff distance of the two
+    label contours; hd_q = max(P_q(d_AB), P_q(d_BA)) with P_q numpy's default percentile (method 'linear') of the directed
+    distances d_AB (every contour voxel of A to the contour of B) and d_BA, q = `percentile` in [0, 100] (95: HD95).  Each
+    contour voxel counts once: no surface-area weights (those of the DeepMind surface-distance package).  inf when A or B is
+    empty.  Arguments and batching as average_surface_distance, with |A| + |B| more workspace floats per pair for the
+    distance lists."""
+    q = float(percentile)
+    if not 0.0 <= q <= 100.0:
+        raise ValueError(f'percentile must lie in [0, 100], got {percentile}')
+    return _surface_distances(seg_a, seg_b, labels, spacing, workspace_bytes, q)
+
+
+def _surface_distances(seg_a, seg_b, labels, spacing, workspace_bytes, percentile):
+    """(asd,) with percentile None (irs_average_surface_distance), else (asd, hd, hd_q) (irs_surface_distances)"""
     import ctypes
     lib = _lib.load()
     _lib.require_cuda(seg_a, seg_b)
@@ -483,10 +502,11 @@ def average_surface_distance(seg_a, seg_b, labels, spacing, workspace_bytes=512 
     if len(sp) != 3:
         raise ValueError('spacing: three values (x, y, z)')
     labels = [int(x) for x in labels]
+    hausdorff = percentile is not None
     dev = seg_b.device
-    out = torch.empty(C, len(labels), device=dev, dtype=torch.float64)
+    outs = tuple(torch.empty(C, len(labels), device=dev, dtype=torch.float64) for _ in range(3 if hausdorff else 1))
     partials = torch.empty(_lib.ASD_PARTIALS_DOUBLES, device=dev, dtype=torch.float64)
-    counters = torch.empty(_lib.ASD_MAX_BOXES, device=dev, dtype=torch.int32)
+    counters = torch.empty(_lib.SD_COUNTERS if hausdorff else _lib.ASD_MAX_BOXES, device=dev, dtype=torch.int32)
     budget = max(1, int(workspace_bytes) // 4)
     for l0 in range(0, len(labels), 32):
         chunk = labels[l0:l0 + 32]
@@ -497,7 +517,9 @@ def average_surface_distance(seg_a, seg_b, labels, spacing, workspace_bytes=512 
                                          _lib.stream()))
         bh = boxes.cpu().view(-1, 8)
         ext = (bh[:, 3:6] - bh[:, 0:3] + 1).long()
-        need = torch.where((bh[:, 6] > 0) & (bh[:, 7] > 0), 2 * ext.prod(1), torch.zeros_like(ext[:, 0])).tolist()
+        # workspace floats per pair: the two distance channels over the box, plus |A| + |B| for the Hausdorff lists
+        per_pair = 2 * ext.prod(1) + (bh[:, 6].long() + bh[:, 7].long() if hausdorff else 0)
+        need = torch.where((bh[:, 6] > 0) & (bh[:, 7] > 0), per_pair, torch.zeros_like(ext[:, 0])).tolist()
         batches, begin, acc = [], 0, 0   # consecutive pairs whose workspace fits the budget
         for p, f in enumerate(need):
             if acc + f > budget and p > begin:
@@ -506,14 +528,20 @@ def average_surface_distance(seg_a, seg_b, labels, spacing, workspace_bytes=512 
             acc += f
         batches.append((begin, len(need), acc))
         ws = torch.empty(max(1, max(b[2] for b in batches)), device=dev, dtype=torch.float32)
-        asd = torch.empty(C, n, device=dev, dtype=torch.float64)
+        res = tuple(torch.empty(C, n, device=dev, dtype=torch.float64) for _ in outs)
         host_boxes = bh.contiguous().numpy()
         for b, e, f in batches:
-            _lib.check(lib.irs_average_surface_distance(
-                _lib.ptr(seg_a), stride, _lib.ptr(seg_b), lab, n, host_boxes.ctypes.data_as(ctypes.c_void_p), sp, b, e,
-                _lib.ptr(ws), ws.numel(), _lib.ptr(partials), _lib.ptr(counters), _lib.ptr(asd), C, D, H, W, _lib.stream()))
-        out[:, l0:l0 + n] = asd
-    return out
+            common = (_lib.ptr(seg_a), stride, _lib.ptr(seg_b), lab, n, host_boxes.ctypes.data_as(ctypes.c_void_p), sp)
+            scratch = (_lib.ptr(ws), ws.numel(), _lib.ptr(partials), _lib.ptr(counters))
+            if hausdorff:
+                _lib.check(lib.irs_surface_distances(*common, percentile, b, e, *scratch, *(_lib.ptr(r) for r in res),
+                                                     C, D, H, W, _lib.stream()))
+            else:
+                _lib.check(lib.irs_average_surface_distance(*common, b, e, *scratch, _lib.ptr(res[0]), C, D, H, W,
+                                                            _lib.stream()))
+        for o, r in zip(outs, res):
+            o[:, l0:l0 + n] = r
+    return outs
 
 
 def _mask_u8(mask, V):

@@ -22,6 +22,7 @@ which calls the adjoint op (the closed forms of SURVEY Appendix A, no scatter at
     calc_no_non_diffeomorphic_voxels (utils/util.py:209-212)              irsgmcmc::log_det_jacobian
     calc_DSC_GPU (utils/util.py:123-148)                                  irsgmcmc::dice_counts
     calc_metrics, ASD part (utils/util.py:171-176)                        irsgmcmc::average_surface_distance
+    (no reference counterpart: Hausdorff distance and HD95, calc_HD_GPU)   irsgmcmc::surface_distances
     (no reference counterpart: posterior of the warped segmentation)      irsgmcmc::label_counts_update (in place), ::label_posterior
     Trainer._SGLD_transition (trainer/trainer.py:291-356)                 irsgmcmc::sgld_step (the fused transition, in place)
 
@@ -417,6 +418,19 @@ def average_surface_distance(seg_a: Tensor, seg_b: Tensor, labels: Sequence[int]
 @average_surface_distance.register_fake
 def _(seg_a, seg_b, labels, spacing):
     return seg_b.new_empty(seg_b.shape[0], len(labels), dtype=torch.float64)
+
+
+@_op('surface_distances')
+def surface_distances(seg_a: Tensor, seg_b: Tensor, labels: Sequence[int], spacing: Sequence[float],
+                      percentile: float = 95.0) -> Tuple[Tensor, Tensor, Tensor]:
+    """float64 (asd, hd, hd_q), each (C, n_labels): average surface distance, Hausdorff distance and the larger of the two
+    directed percentiles (numpy's method 'linear', 95: HD95) of seg_a == l and seg_b[c] == l from one distance transform"""
+    return ops.surface_distances(seg_a.contiguous(), seg_b.contiguous(), list(labels), list(spacing), percentile)
+
+
+@surface_distances.register_fake
+def _(seg_a, seg_b, labels, spacing, percentile=95.0):
+    return tuple(seg_b.new_empty(seg_b.shape[0], len(labels), dtype=torch.float64) for _ in range(3))
 
 
 # ---- posterior of the warped segmentation ---------------------------------------------------------------------------------

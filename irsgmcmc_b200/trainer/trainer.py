@@ -409,7 +409,7 @@ class Trainer:
 
     @torch.no_grad()
     def _test_VI(self, var_params_q_v=None, no_samples=None, modules=None, speed_test_samples=100, with_ASD=True,
-                 with_seg_posterior=False, with_jacobian_posterior=False):
+                 with_seg_posterior=False, with_jacobian_posterior=False, with_HD=False, HD_percentile=95.0):
         """
         evaluation of the fitted q(v) (reference trainer.py:226-289): `no_samples_VI_test` draws from q(v) -> Sobolev smoothing ->
         transformation -> number of folded voxels + log det J, warped image and segmentation, ASD / DSC per structure, the sample on
@@ -424,6 +424,9 @@ class Trainer:
         with_jacobian_posterior=True (S >= 1, else ValueError) adds 'jacobian_posterior', the posterior of log det J over the
         S draws with the entries of _run_MCMC's ('SDlogJ' and 'folded_fraction' are (S, 1)); with save_dir,
         VI_log_det_J_mean.nii.gz, VI_log_det_J_std_dev.nii.gz and VI_fold_probability.nii.gz.
+        with_HD=True (needs the segmentations, like 'ASD') adds 'HD' and 'HD95' (the key follows HD_percentile: 'HD99' for 99),
+        (S, structures) arrays of the Hausdorff distance and its percentile per draw (utils.util.calc_HD_GPU; with with_ASD, one
+        distance transform gives all three); with with_seg_posterior, 'HD_majority' and 'HD95_majority' per structure.
         """
         from .. import ops
         from ..utils import SobolevGrad, calc_metrics
@@ -457,7 +460,7 @@ class Trainer:
             return transformation, displacement, registration_module(moving['im'], transformation)
 
         mean, m2, count = torch.zeros((3, *self.dims), device=dev), torch.zeros((3, *self.dims), device=dev), 0
-        folded, dsc, asd = [], [], []
+        folded, dsc, asd, hd, hd_q = [], [], [], [], []
         for test_sample_no in range(1, S + 1):
             transformation, displacement, im_moving_warped = register(sample_q_v(vp, no_samples=1))
             count = ops.welford_update(displacement.contiguous(), count, mean, m2)
@@ -468,11 +471,17 @@ class Trainer:
                                                                      jac['folds'], jac['mean'], jac['m2'], jac['scratch'])
             if with_seg:
                 seg_moving_warped = registration_module(moving['seg'], transformation)
-                if with_ASD:
+                if with_ASD and not with_HD:
                     ASD, DSC = calc_metrics(seg_fixed, seg_moving_warped, self.structures_dict, self.im_spacing)
                     asd.append(ASD[0])
                 else:
                     DSC = calc_DSC_GPU(1, seg_fixed, seg_moving_warped, self.structures_dict)
+                    if with_HD:
+                        ASD, HD, HD_q = self._surface_distances(seg_fixed, seg_moving_warped, 1, with_ASD, HD_percentile)
+                        if with_ASD:
+                            asd.append(ASD[0])
+                        hd.append(HD[0])
+                        hd_q.append(HD_q[0])
                 dsc.append(DSC[0])
                 if with_seg_posterior:
                     ops.label_counts_update(seg_moving_warped.contiguous(), seg_labels, seg_counts)
@@ -490,11 +499,13 @@ class Trainer:
         result = {'no_non_diffeomorphic_voxels': folded, 'DSC': np.asarray(dsc), 'mean': mean, 'std_dev': std_dev,
                   'ASD': np.asarray(asd) if (with_seg and with_ASD) else 'unavailable: no segmentations / structures, or with_ASD=False',
                   'displacement_mu': displacement_mu, 'im_moving_warped_mu': im_moving_warped_mu, 'n': count}
+        if with_HD:
+            result.update(self._HD_entries(np.asarray(hd), np.asarray(hd_q), with_seg, HD_percentile))
         if with_seg_posterior:
             prob, majority, entropy, summary = ops.label_posterior(seg_counts, S, seg_labels, seg_fixed.contiguous())
             post = {'labels': seg_labels, 'n': S, 'probability': prob, 'majority': majority, 'entropy': entropy,
                     'summary': summary}
-            result['seg_posterior'] = self._seg_posterior(post, with_ASD, 'VI')
+            result['seg_posterior'] = self._seg_posterior(post, with_ASD, 'VI', with_HD, HD_percentile)
         if with_jacobian_posterior:
             p_fold, mean_ld, std_ld, summary = ops.jacobian_posterior(jac['folds'], jac['mean'], jac['m2'], S, jac['mask'])
             post = {'n': S, 'fold_probability': p_fold, 'log_det_J_mean': mean_ld, 'log_det_J_std': std_ld, 'summary': summary}
@@ -564,7 +575,7 @@ class Trainer:
 
     # -- the loop around it (reference trainer.py:358-476) -------------------------------------------------------------
     def _run_MCMC(self, data_loss=None, reg_loss=None, speed_test_iters=100, with_ASD=False, with_R_hat=False,
-                  with_seg_posterior=False, with_jacobian_posterior=False):
+                  with_seg_posterior=False, with_jacobian_posterior=False, with_HD=False, HD_percentile=95.0):
         """burn-in + sampling; returns {'mean','std_dev', 'im_mean','im_std', 'n', 'DSC', 'ASD', 'no_non_diffeomorphic_voxels',
         'samples_per_sec'}; posterior statistics are over the kept samples of ALL ranks.  'ASD' (average surface distance,
         reference utils/util.py:171-176 through SimpleITK on the host): with_ASD=True computes it per kept sample on the device
@@ -599,7 +610,14 @@ class Trainer:
         of log det J over the finite mask voxels, and 'folded_fraction', the folded share of the mask, as (kept samples,
         chains) arrays.  Registration challenges that report SDlogJ clip det J at 1e-9 instead of leaving the non-positive
         voxels out.  With save_dir, MCMC_log_det_J_mean.nii.gz, MCMC_log_det_J_std_dev.nii.gz and
-        MCMC_fold_probability.nii.gz are written as well.  With with_jacobian_posterior=False nothing of this runs."""
+        MCMC_fold_probability.nii.gz are written as well.  With with_jacobian_posterior=False nothing of this runs.
+
+        with_HD=True adds 'HD' and 'HD95' (the key follows HD_percentile: 'HD99' for 99), one (chains, structures) array per
+        kept sample like 'ASD': the Hausdorff distance of the label contours and the larger of the two directed percentiles
+        of the contour distances (numpy's default percentile; utils.util.calc_HD_GPU, the label-contour / distance transform
+        kernels of the ASD plus a radix select on the device).  With with_ASD as well, one distance transform per kept sample
+        gives all three.  With with_seg_posterior, the structures also get 'HD_majority' and 'HD95_majority'.  With
+        with_HD=False nothing of this runs."""
         if self.SGLD_params is None:
             self._SGLD_init()
         s = self.sampler
@@ -615,7 +633,7 @@ class Trainer:
                 self._gmm_pushed = True
             else:
                 self._GMM_init()
-        dsc, asd, folded = [], [], []
+        dsc, asd, folded, hd, hd_q = [], [], [], [], []
         total = self.no_iters_burn_in + self.no_samples_MCMC
         if with_R_hat:
             n_kept = sum(1 for i in range(1, total + 1) if self._is_kept(i))
@@ -646,9 +664,15 @@ class Trainer:
                     seg_w = s.warp_segmentation(transformation=T)
                     seg_f = self.fixed['seg'].to(s.device).expand(self.no_chains, -1, -1, -1, -1)
                     dsc.append(calc_DSC_GPU(self.no_chains, seg_f, seg_w, self.structures_dict))
-                    if with_ASD:
+                    if with_ASD and not with_HD:
                         from ..utils.util import calc_metrics
                         asd.append(calc_metrics(seg_f, seg_w, self.structures_dict, self.im_spacing, no_samples=self.no_chains)[0])
+                    elif with_HD:
+                        ASD, HD, HD_q = self._surface_distances(seg_f, seg_w, self.no_chains, with_ASD, HD_percentile)
+                        if with_ASD:
+                            asd.append(ASD)
+                        hd.append(HD)
+                        hd_q.append(HD_q)
                 # after the segmentation warp, so that the segmentation posterior reuses it; the transformation and the warp
                 # read what accumulate() reads and write nothing it reads, so the order changes no result
                 s.accumulate(seg_warped=seg_w, transformation=T)
@@ -679,12 +703,15 @@ class Trainer:
                   'ASD': asd if with_ASD else 'unavailable: not requested (with_ASD=True computes the label-contour average '
                                               'Hausdorff distance of reference utils/util.py:171-176 per kept sample with the CUDA '
                                               'distance transform kernels; parity with SimpleITK unpinned)'}
+        if with_HD:
+            with_seg = bool(self.structures_dict and s.moving_seg is not None and 'seg' in self.fixed)
+            result.update(self._HD_entries(hd, hd_q, with_seg, HD_percentile))
         if with_R_hat:
             result['R_hat'] = self._R_hat(traces)
         if with_seg_posterior:
             post = s.segmentation_posterior(seg_fixed=self.fixed['seg'])
             s.disable_segmentation_posterior()
-            result['seg_posterior'] = self._seg_posterior(post, with_ASD, 'MCMC')
+            result['seg_posterior'] = self._seg_posterior(post, with_ASD, 'MCMC', with_HD, HD_percentile)
         if with_jacobian_posterior:
             post = s.jacobian_posterior()
             s.disable_jacobian_posterior()
@@ -704,6 +731,27 @@ class Trainer:
             torch.cuda.synchronize()
             result['samples_per_sec'] = self.no_chains * speed_test_iters / (time.perf_counter() - t0)
         return result
+
+    @staticmethod
+    def _HD_key(percentile):
+        """'HD95' for the 95th percentile, 'HD99.5' for 99.5"""
+        return f'HD{float(percentile):g}'
+
+    def _surface_distances(self, seg_fixed, seg_warped, no_samples, with_ASD, percentile):
+        """(ASD or None, HD, HD_q) of the warped segmentations, (no_samples, structures) each: one distance transform for all
+        three when with_ASD (the ASD is calc_ASD_GPU's to the bit), calc_HD_GPU otherwise"""
+        from ..utils.util import calc_HD_GPU, calc_surface_distances_GPU
+        if with_ASD:
+            return calc_surface_distances_GPU(no_samples, seg_fixed, seg_warped, self.structures_dict, self.im_spacing,
+                                              percentile)
+        return (None,) + calc_HD_GPU(no_samples, seg_fixed, seg_warped, self.structures_dict, self.im_spacing, percentile)
+
+    def _HD_entries(self, hd, hd_q, available, percentile):
+        """the 'HD' and 'HD95' entries of _run_MCMC / _test_VI(with_HD=True)"""
+        if not available:
+            why = 'unavailable: no segmentations / structures'
+            return {'HD': why, self._HD_key(percentile): why}
+        return {'HD': hd, self._HD_key(percentile): hd_q}
 
     def _R_hat(self, traces):
         """the 'R_hat' entry of _run_MCMC(with_R_hat=True) from the filled accumulators and this rank's traces (N, C, 4); frees
@@ -730,11 +778,12 @@ class Trainer:
             save_im_to_disk(diag['im'][0].cpu(), os.path.join(self.save_dir, 'MCMC_R_hat_im.nii.gz'), sp)
         return diag
 
-    def _seg_posterior(self, post, with_ASD, model):
+    def _seg_posterior(self, post, with_ASD, model, with_HD=False, HD_percentile=95.0):
         """the 'seg_posterior' entry of _run_MCMC / _test_VI(with_seg_posterior=True) from the dict of
         SGLDSampler.segmentation_posterior (computed with the fixed segmentation): per structure the expected volume S / n, the
-        uncertain voxels U, the soft Dice 2 O / (S + n |F|) of the probability map and the Dice (and ASD) of the majority
-        segmentation; {model}_seg_majority.nii.gz and {model}_seg_entropy.nii.gz in save_dir"""
+        uncertain voxels U, the soft Dice 2 O / (S + n |F|) of the probability map and the Dice (and ASD, and with with_HD the
+        Hausdorff distance and its percentile: 'HD_majority', 'HD95_majority') of the majority segmentation;
+        {model}_seg_majority.nii.gz and {model}_seg_entropy.nii.gz in save_dir"""
         from .. import ops
         from ..utils.util import calc_ASD_GPU
         n, labels, majority = post['n'], post['labels'], post['majority']
@@ -742,7 +791,11 @@ class Trainer:
         summary = post['summary'].cpu().numpy()
         fixed_sizes = ops.dice_counts(seg_f, seg_f, labels)[0, :, 0].cpu().numpy()   # |F_l|
         dsc = calc_DSC_GPU(1, seg_f, majority, self.structures_dict)[0]
-        asd = calc_ASD_GPU(1, seg_f, majority, self.structures_dict, self.im_spacing)[0] if with_ASD else None
+        if with_HD:   # one distance transform for the ASD and both Hausdorff figures
+            asd, hd, hd_q = (None if x is None else x[0]
+                             for x in self._surface_distances(seg_f, majority, 1, with_ASD, HD_percentile))
+        else:
+            asd = calc_ASD_GPU(1, seg_f, majority, self.structures_dict, self.im_spacing)[0] if with_ASD else None
         structures = {}
         for j, name in enumerate(self.structures_dict):
             S, O, U = (int(x) for x in summary[j])
@@ -751,6 +804,9 @@ class Trainer:
                                 'soft_DSC': 2.0 * O / den if den else float('nan'), 'DSC_majority': float(dsc[j])}
             if with_ASD:
                 structures[name]['ASD_majority'] = float(asd[j])
+            if with_HD:
+                structures[name]['HD_majority'] = float(hd[j])
+                structures[name][f'{self._HD_key(HD_percentile)}_majority'] = float(hd_q[j])
         post['structures'] = structures
         if self.save_dir is not None and (not torch.distributed.is_initialized() or torch.distributed.get_rank() == 0):
             import os

@@ -135,21 +135,54 @@ def calc_DSC_GPU(no_samples, seg_fixed, seg_moving, structures_dict):
     return (2.0 * cnt[..., 2] / (cnt[..., 0] + cnt[..., 1])).float().numpy()
 
 
+def _segmentations_for_surface_kernels(no_samples, seg_fixed, seg_moving, structures_dict, spacing, name):
+    """(seg_a, seg_b, labels, spacing) as the surface kernels take them: the first no_samples volumes, a fixed volume
+    expanded over the samples passed once; CPU tensors, other dtypes and label 0 are refused"""
+    labels = [int(x) for x in structures_dict.values()]
+    a, b = seg_fixed[:no_samples], seg_moving[:no_samples].contiguous()
+    if not (a.is_cuda and b.is_cuda) or a.dtype != torch.int16 or b.dtype != torch.int16:
+        raise NotImplementedError(f'{name} needs int16 CUDA segmentations: irsgmcmc_b200 has no CPU path')
+    if 0 in labels:
+        raise NotImplementedError(f'{name}: label 0 is the background of the surface kernels')
+    a = a[:1].contiguous() if a.stride(0) == 0 else a.contiguous()
+    sp = [float(x) for x in np.asarray(spacing.cpu() if hasattr(spacing, 'cpu') else spacing, dtype=np.float64).reshape(-1)[:3]]
+    return a, b, labels, sp
+
+
 @torch.no_grad()
 def calc_ASD_GPU(no_samples, seg_fixed, seg_moving, structures_dict, spacing):
     """average surface distance per sample and structure (the reference's calc_metrics, utils/util.py:171-176), float64
     (no_samples, structures), inf where a structure is empty: the label-contour / exact Euclidean distance transform kernels,
     one host synchronisation per call and no volume copies.  Same definition as calc_ASD_host, which the tests compare it
     with.  int16 CUDA segmentations only -- no PyTorch path."""
-    labels = [int(x) for x in structures_dict.values()]
-    a, b = seg_fixed[:no_samples], seg_moving[:no_samples].contiguous()
-    if not (a.is_cuda and b.is_cuda) or a.dtype != torch.int16 or b.dtype != torch.int16:
-        raise NotImplementedError('calc_ASD_GPU needs int16 CUDA segmentations: irsgmcmc_b200 has no CPU path')
-    if 0 in labels:
-        raise NotImplementedError('calc_ASD_GPU: label 0 is the background of the surface kernels')
-    a = a[:1].contiguous() if a.stride(0) == 0 else a.contiguous()
-    sp = [float(x) for x in np.asarray(spacing.cpu() if hasattr(spacing, 'cpu') else spacing, dtype=np.float64).reshape(-1)[:3]]
+    a, b, labels, sp = _segmentations_for_surface_kernels(no_samples, seg_fixed, seg_moving, structures_dict, spacing,
+                                                          'calc_ASD_GPU')
     return ops.average_surface_distance(a, b, labels, sp).cpu().numpy()
+
+
+@torch.no_grad()
+def calc_surface_distances_GPU(no_samples, seg_fixed, seg_moving, structures_dict, spacing, percentile=95.0):
+    """(ASD, HD, HD_q), each float64 (no_samples, structures), from one distance transform (ops.surface_distances): ASD is
+    calc_ASD_GPU's to the bit, HD and HD_q are calc_HD_GPU's.  One host synchronisation per call."""
+    a, b, labels, sp = _segmentations_for_surface_kernels(no_samples, seg_fixed, seg_moving, structures_dict, spacing,
+                                                          'calc_surface_distances_GPU')
+    return tuple(t.cpu().numpy() for t in ops.surface_distances(a, b, labels, sp, percentile))
+
+
+@torch.no_grad()
+def calc_HD_GPU(no_samples, seg_fixed, seg_moving, structures_dict, spacing, percentile=95.0):
+    """(HD, HD_q) per sample and structure, float64 (no_samples, structures) each, inf where a structure is empty, 0 where the
+    two coincide: HD = max(max d_AB, max d_BA), the Hausdorff distance of the two label contours (what ITK's
+    HausdorffDistanceImageFilter returns on the contour images calc_ASD_host builds), and HD_q = max(P_q(d_AB), P_q(d_BA)) with
+    P_q numpy's default np.percentile (method 'linear') -- HD95 for the default q = 95, the symmetric form MONAI's
+    compute_hausdorff_distance(percentile=q) uses.  d_AB holds the distance from every contour voxel of A to the contour of B
+    once: no surface-area weights, unlike the DeepMind surface-distance package.  The label-contour / exact Euclidean distance
+    transform kernels of calc_ASD_GPU plus a radix select on the device; same definition as calc_HD_host, which the tests
+    compare it with.  int16 CUDA segmentations only -- no PyTorch path."""
+    a, b, labels, sp = _segmentations_for_surface_kernels(no_samples, seg_fixed, seg_moving, structures_dict, spacing,
+                                                          'calc_HD_GPU')
+    _, hd, hd_q = ops.surface_distances(a, b, labels, sp, percentile)
+    return hd.cpu().numpy(), hd_q.cpu().numpy()
 
 
 def _label_contour(mask):
@@ -188,6 +221,29 @@ def calc_ASD_host(seg_fixed_structure, seg_moving_structure, spacing=(1.0, 1.0, 
     d_to_b = ndimage.distance_transform_edt(~cb, sampling=sampling)
     d_to_a = ndimage.distance_transform_edt(~ca, sampling=sampling)
     return 0.5 * (float(d_to_b[ca].mean()) + float(d_to_a[cb].mean()))
+
+
+def calc_HD_host(seg_fixed_structure, seg_moving_structure, spacing=(1.0, 1.0, 1.0), percentile=95.0):
+    """
+    (HD, HD_q) of two binary structures on the host, the restatement calc_HD_GPU is tested against: the bounding-box crop,
+    label contours and scipy distance transforms of calc_ASD_host, then HD = max of the two directed maxima and HD_q = max of
+    np.percentile(d_AB, q) and np.percentile(d_BA, q) (method 'linear'), d_AB = the distances of the contour voxels of A to the
+    contour of B.  (inf, inf) when a structure is empty.
+    """
+    from scipy import ndimage
+    a, b = np.asarray(seg_fixed_structure).astype(bool), np.asarray(seg_moving_structure).astype(bool)
+    if not a.any() or not b.any():
+        return float('inf'), float('inf')
+    idx = np.argwhere(a | b)
+    lo, hi = np.maximum(idx.min(0) - 1, 0), np.minimum(idx.max(0) + 2, a.shape)
+    box = tuple(slice(int(l), int(h)) for l, h in zip(lo, hi))
+    a, b = a[box], b[box]
+    ca, cb = _label_contour(a), _label_contour(b)
+    sampling = [float(x) for x in np.asarray(spacing).reshape(-1)[:3]][::-1]
+    d_ab = ndimage.distance_transform_edt(~cb, sampling=sampling)[ca]
+    d_ba = ndimage.distance_transform_edt(~ca, sampling=sampling)[cb]
+    hd = max(float(d_ab.max()), float(d_ba.max()))
+    return hd, max(float(np.percentile(d_ab, percentile)), float(np.percentile(d_ba, percentile)))
 
 
 @torch.no_grad()
