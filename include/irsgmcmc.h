@@ -303,6 +303,38 @@ int irs_jacobian_posterior(const int* folds, const float* mean, const float* m2,
                            unsigned long long* counters, long long* summary, void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------------ *
+ * Landmark registration error and landmark posterior (the reference has none).  Landmarks are (P,3) doubles in zero-based
+ * voxel coordinates (x, y, z) = (W, H, D); row i of the fixed landmarks p corresponds to row i of the moving landmarks q.
+ * spacing_host: 3 HOST doubles (x, y, z) in mm, finite and > 0 (both images share one grid).
+ *   irs_landmark_map: for chain c of T (C,3,D,H,W) and landmark i, the predicted moving position pred (C,P,3) doubles: per
+ *     axis i0 = min(floor(p_a), n_a - 2) clamped to [0, n_a - 2] (no coordinate, NaN included, reads outside T), f = p_a - i0;
+ *     fp64 trilinear interpolation of the fp32 corners as lerps a + f (b - a) along x, then y, then z, every operation rounded
+ *     on its own (no FMA); m_a = ((g_a + 1) (n_a - 1)) 0.5.  tre (C,P) doubles = sqrt of the sum over x, y, z of
+ *     (s_a (m_a - q_a))^2.  p should lie in [0, n_a - 1] (the Python op checks it); outside, m extrapolates the edge cell.
+ *   irs_landmark_update: folds pred / tre of C chains into acc (P, IRS_LANDMARK_ACC) doubles, chains in index order, sample
+ *     count k = count_before + c + 1: delta = m - mean, mean += delta / k, M_ab += delta_a (m_b - mean_b) over (xx, xy, xz, yy,
+ *     yz, zz), and the Welford mean / M2 of the TRE -- per landmark [0,3) mean, [3,9) M, [9] TRE mean, [10] TRE M2.  Zero acc
+ *     before the first update; splitting the chains of a sample over several calls gives the same bits.  count_before: an
+ *     integer >= 0 with count_before + C <= 2^53.  sample_stats (C,3) doubles per chain, landmarks in index order: sum TRE,
+ *     sum TRE^2, max TRE.
+ *   irs_landmark_posterior: from acc over n (1..2^53) samples, out (P, IRS_LANDMARK_COLS) doubles per landmark:
+ *     [0,3) mean position (moving voxels), [3] TRE of the mean |s o (mean - q)|, [4] E[TRE],
+ *     and for n >= 2 (NaN for n = 1): [5] unbiased std of TRE, [6,12) covariance s_a s_b M_ab / (n - 1) in mm^2 (xx, xy, xz, yy,
+ *     yz, zz), [12,15) principal standard deviations sqrt(max(lambda, 0)) in descending order (closed-form symmetric 3x3),
+ *     [15] squared Mahalanobis distance r^T Sigma^-1 r, r = s o (q - mean), by a Cholesky factorisation (+inf for a pivot <= 0).
+ * C < 1, P < 1, n_a < 2, null pointers, bad spacing or counts: IRS_ERR_BAD_ARG before any CUDA call.  No atomics, no host
+ * synchronisation, graph-capturable.
+ * ------------------------------------------------------------------------------------------------------------------ */
+#define IRS_LANDMARK_ACC 11
+#define IRS_LANDMARK_COLS 16
+int irs_landmark_map(const float* T, int C, int D, int H, int W, const double* p, const double* q, int P,
+                     const double* spacing_host, double* pred, double* tre, void* stream);
+int irs_landmark_update(const double* pred, const double* tre, int C, int P, double count_before, double* acc,
+                        double* sample_stats, void* stream);
+int irs_landmark_posterior(const double* acc, const double* q, int P, long long n, const double* spacing_host, double* out,
+                           void* stream);
+
+/* ------------------------------------------------------------------------------------------------------------------ *
  * The fused SGLD transition -- replaces Trainer._SGLD_transition, trainer/trainer.py:291-356, for all chains of this
  * GPU, including the sequential per-chain GMM Adam step (trainer.py:316-327, 68-77; optimizers/adam_rate_decay.py),
  * the regulariser's hyper-parameter Adam step (trainer.py:353-354) and the plain-SGD state update (trainer.py:351).

@@ -85,6 +85,9 @@ RHAT_MAX_COMPONENTS, RHAT_PARTIALS_DOUBLES = 4, 4 * 3 * 256
 # Jacobian posterior (include/irsgmcmc.h): reduction scratch per chain, words of the finish's summary
 JACOBIAN_REDUCE_BLOCKS, JACOBIAN_SUMMARY_WORDS = 1184, 8
 
+# landmark posterior (include/irsgmcmc.h): accumulator doubles and posterior columns per landmark
+LANDMARK_ACC, LANDMARK_COLS = 11, 16
+
 VI_STATE_SIZE, VI_STEP, VI_BETA_POW, VI_X, VI_SUMS, VI_ENTROPY = 16, 0, 1, 3, 4, 8
 
 # name -> (restype, argtypes); every symbol include/irsgmcmc.h declares
@@ -134,6 +137,9 @@ SYMBOLS = {
     'irs_label_posterior': (_i, [_vp, _vp, _i, _ll, _ll, _vp, _vp, _vp, _vp, _vp, _vp]),
     'irs_jacobian_update': (_i, [_vp, _vp, _i, _i, _i, _i, _d, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     'irs_jacobian_posterior': (_i, [_vp, _vp, _vp, _ll, _ll, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    'irs_landmark_map': (_i, [_vp, _i, _i, _i, _i, _vp, _vp, _i, _vp, _vp, _vp, _vp]),
+    'irs_landmark_update': (_i, [_vp, _vp, _i, _i, _d, _vp, _vp, _vp]),
+    'irs_landmark_posterior': (_i, [_vp, _vp, _i, _ll, _vp, _vp, _vp]),
     'irs_sgld_partials_doubles': (_sz, [ctypes.POINTER(SgldConfig)]),
     'irs_sgld_step': (_i, [ctypes.POINTER(SgldConfig), ctypes.POINTER(SgldBuffers), _vp]),
     'irs_sgld_step_profile': (_i, [ctypes.POINTER(SgldConfig), ctypes.POINTER(SgldBuffers), _vp, _vp]),

@@ -61,6 +61,16 @@ def _exp_velocity(v, no_steps=6):
     return grid + d.permute(0, 2, 3, 4, 1)
 
 
+def _texture_and_velocity(n, seed, max_velocity, dev):
+    """the generator of make_pair after its first two draws, the smoothed texture noise and the velocity (1,3,n,n,n) in voxels
+    with max |v| = max_velocity: the draws of make_pair in its order (the texture first), so that make_landmarks replays the
+    same velocity"""
+    g = torch.Generator().manual_seed(seed)
+    texture = _smooth(torch.randn(1, 1, n, n, n, generator=g).to(dev), n / 32.0)
+    v = _smooth(torch.randn(1, 3, n, n, n, generator=g).to(dev), n / 16.0)
+    return g, texture, v * (max_velocity / v.abs().max())
+
+
 def make_pair(n, seed=123, max_velocity=3.0, noise_std=0.02, sigma_v_init=0.5, u_v_init=0.1, device=None):
     """
     returns (fixed, moving, var_params_q_v) on the host, deterministic in (n, seed)
@@ -71,8 +81,8 @@ def make_pair(n, seed=123, max_velocity=3.0, noise_std=0.02, sigma_v_init=0.5, u
     moving['im']: fixed warped by exp(v) of a smooth random velocity with max |v| = max_velocity voxels + fresh noise
     mask:         head ellipsoid (about 29 % of the cube);  seg: 15 small labelled ellipsoids, int16
     """
-    g = torch.Generator().manual_seed(seed)
     dev = device or 'cpu'
+    g, texture, v = _texture_and_velocity(n, seed, max_velocity, dev)
     E = lambda c, a: _ellipsoid(n, c, a, dev)
     head = E((0.0, 0.0, 0.0), (0.74, 0.92, 0.80))
 
@@ -81,7 +91,6 @@ def make_pair(n, seed=123, max_velocity=3.0, noise_std=0.02, sigma_v_init=0.5, u
         im = torch.where(E((0.0, 0.02, -0.03), (0.74 * sc, 0.92 * sc, 0.80 * sc)), torch.tensor(val, device=dev), im)
     im = _smooth(im.view(1, 1, n, n, n), max(0.5, n / 64.0))
 
-    texture = _smooth(torch.randn(1, 1, n, n, n, generator=g).to(dev), n / 32.0)
     texture = 0.08 * texture / texture.abs().max()
     clean = (im + texture) * head
 
@@ -96,8 +105,6 @@ def make_pair(n, seed=123, max_velocity=3.0, noise_std=0.02, sigma_v_init=0.5, u
         c = (0.25 * math.sin(2.0 * ang), 0.45 * math.sin(ang), 0.4 * math.cos(ang))
         seg[E(c, (0.09, 0.11, 0.10))] = label
 
-    v = _smooth(torch.randn(1, 3, n, n, n, generator=g).to(dev), n / 16.0)
-    v = v * (max_velocity / v.abs().max())
     grid = _exp_velocity(v)
 
     moving_clean = F.grid_sample(clean, grid, mode='bilinear', padding_mode='border', align_corners=True)
@@ -113,3 +120,33 @@ def make_pair(n, seed=123, max_velocity=3.0, noise_std=0.02, sigma_v_init=0.5, u
     var_params_q_v = {'mu': torch.zeros(dims_v), 'log_var': torch.full(dims_v, math.log(sigma_v_init ** 2)),
                       'u': torch.full(dims_v, u_v_init)}
     return fixed, moving, var_params_q_v
+
+
+def make_landmarks(n, seed=123, max_velocity=3.0, no_landmarks=300, device=None):
+    """
+    Corresponding landmarks of make_pair(n, seed, max_velocity): (fixed_landmarks, moving_landmarks), (P,3) float64 host
+    tensors of zero-based (x, y, z) voxel coordinates, P = no_landmarks, row i of one corresponding to row i of the other.
+
+    make_pair builds moving = fixed o phi with phi = exp(v) (voxel units here).  The moving landmarks q are moving-mask voxels
+    drawn with a generator of their own (make_pair's draws are unchanged), kept where phi(q) lies in [1, n - 2] on every
+    axis; the fixed landmarks are p = phi(q) from the same sampling grid, so the fixed image at p shows what the moving image
+    shows at q.  A registration of the pair estimates T ~ phi^-1, which carries p back to q: the TRE of the true
+    transformation is 0 up to the grid's rounding.  ValueError when fewer than no_landmarks voxels qualify.
+    """
+    dev = device or 'cpu'
+    _, _, v = _texture_and_velocity(n, seed, max_velocity, dev)
+    grid = _exp_velocity(v)                                               # (1,D,H,W,3) normalised (x, y, z)
+    phi = (grid[0].double() + 1.0) * ((n - 1) / 2.0)                      # fixed voxel coordinates (x, y, z)
+    head = _ellipsoid(n, (0.0, 0.0, 0.0), (0.74, 0.92, 0.80), dev)
+    moving_mask = F.grid_sample(head.float().view(1, 1, n, n, n), grid, mode='nearest', padding_mode='border',
+                                align_corners=True).bool()[0, 0]          # make_pair's moving['mask']
+    ok = moving_mask & ((phi >= 1.0) & (phi <= n - 2.0)).all(-1)
+    idx = torch.nonzero(ok.flatten().cpu()).flatten()
+    if idx.numel() < no_landmarks:
+        raise ValueError(f'only {idx.numel()} moving-mask voxels map inside [1, n - 2]: fewer than {no_landmarks} landmarks')
+    g = torch.Generator().manual_seed(seed + 1)
+    pick = idx[torch.randperm(idx.numel(), generator=g)[:no_landmarks]]
+    z, y, x = pick // (n * n), (pick // n) % n, pick % n
+    q = torch.stack((x, y, z), -1).double()
+    p = phi.cpu().reshape(-1, 3)[pick]
+    return p.contiguous(), q.contiguous()

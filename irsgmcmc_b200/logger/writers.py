@@ -159,3 +159,52 @@ def save_variational_posterior_mean(save_dir, spacing, im_moving_warped, displac
     save_im_to_disk(_to_numpy(im_moving_warped)[0, 0], paths['im_moving_warped_mu'], sp)
     save_field_to_disk(_to_numpy(displacement)[0] * sp[0], paths['displacement_mu'], sp)
     return paths
+
+
+def save_landmarks_to_disk(file_path, points, covariance=None, scalars=None):
+    """landmarks -> legacy VTK POLYDATA (one vertex per point, readable by vtkPolyDataReader / ParaView): points (P, 3) in mm,
+    covariance (P, 6) = (xx, xy, xz, yy, yz, zz) as a symmetric 3x3 TENSORS array 'covariance', scalars {name: (P,)} as one
+    SCALARS array each (NaN stays NaN)"""
+    pts = _to_numpy(points).astype(np.float64).reshape(-1, 3)
+    P = pts.shape[0]
+    with open(file_path, 'wb') as f:
+        f.write(_vtk_header('irsgmcmc_b200 landmarks', 'POLYDATA'))
+        f.write(f'POINTS {P} float\n'.encode('ascii'))
+        f.write(pts.astype('>f4').tobytes())
+        f.write(f'\nVERTICES {P} {2 * P}\n'.encode('ascii'))
+        f.write(np.stack((np.ones(P), np.arange(P)), -1).astype('>i4').tobytes())
+        f.write(f'\nPOINT_DATA {P}\n'.encode('ascii'))
+        if covariance is not None:
+            c = _to_numpy(covariance).astype(np.float64).reshape(P, 6)
+            full = c[:, [0, 1, 2, 1, 3, 4, 2, 4, 5]]
+            f.write(b'TENSORS covariance float\n')
+            f.write(full.astype('>f4').tobytes())
+            f.write(b'\n')
+        for name, values in (scalars or {}).items():
+            f.write(f'SCALARS {name} float 1\nLOOKUP_TABLE default\n'.encode('ascii'))
+            f.write(_to_numpy(values).astype('>f4').reshape(P).tobytes())
+            f.write(b'\n')
+
+
+def load_landmarks_from_disk(file_path):
+    """(points (P, 3), {array name: values}) of a file written by save_landmarks_to_disk (round-trip check; not a general
+    reader): tensors come back as (P, 3, 3), scalars as (P,)"""
+    with open(file_path, 'rb') as f:
+        raw = f.read()
+    pos = raw.index(b'POINTS ')
+    line_end = raw.index(b'\n', pos)
+    P = int(raw[pos:line_end].split()[1])
+    points = np.frombuffer(raw, dtype='>f4', count=3 * P, offset=line_end + 1).reshape(P, 3).astype(np.float64)
+    arrays, pos = {}, raw.index(b'POINT_DATA')
+    pos = raw.index(b'\n', pos) + 1
+    while pos < len(raw):
+        line_end = raw.index(b'\n', pos)
+        head = raw[pos:line_end].split()
+        if head[0] == b'TENSORS':
+            arrays[head[1].decode()] = np.frombuffer(raw, dtype='>f4', count=9 * P, offset=line_end + 1).reshape(P, 3, 3)
+            pos = line_end + 1 + 36 * P + 1
+        else:   # SCALARS name float 1 / LOOKUP_TABLE default
+            lut_end = raw.index(b'\n', line_end + 1)
+            arrays[head[1].decode()] = np.frombuffer(raw, dtype='>f4', count=P, offset=lut_end + 1).copy()
+            pos = lut_end + 1 + 4 * P + 1
+    return points, arrays

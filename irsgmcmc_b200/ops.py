@@ -2,6 +2,9 @@
 Functional wrappers over the C ABI (include/irsgmcmc.h): allocate outputs with torch, pass raw pointers, launch on
 torch's current stream.  CUDA tensors only -- every function raises on CPU tensors (no fallback).
 """
+import ctypes
+import math
+
 import torch
 
 from . import _lib
@@ -625,3 +628,105 @@ def jacobian_posterior(folds, mean, m2, n, mask):
             'voxels_finite': words[3], 'voxels_finite_2': words[4], 'mask_voxels': words[7],
             'mean_log_det_J': means[0], 'mean_std_log_det_J': means[1]}
     return p_fold, mean_out, std_out, summ
+
+
+def _landmarks_host(x, name):
+    """(P, 3) float64 host copy of a landmark table"""
+    x = torch.as_tensor(x).detach().to('cpu', torch.float64)
+    if x.dim() != 2 or x.shape[1] != 3 or x.shape[0] < 1:
+        raise ValueError(f'{name} must be a (P, 3) table of (x, y, z) voxel coordinates with P >= 1')
+    return x.contiguous()
+
+
+def landmark_spacing(spacing):
+    """the three (x, y, z) spacings in mm as floats, each finite and > 0"""
+    sp = [float(s) for s in torch.as_tensor(spacing, dtype=torch.float64).reshape(-1).tolist()]
+    if len(sp) != 3 or not all(math.isfinite(s) and s > 0.0 for s in sp):
+        raise ValueError(f'spacing must be three finite positive (x, y, z) values, got {sp}')
+    return sp
+
+
+def check_landmarks(fixed_landmarks, moving_landmarks, dims):
+    """host checks of a pair of landmark tables for a (D, H, W) grid: (P, 3) each with the same P; every fixed coordinate
+    finite and in [0, n_a - 1] of its axis (x = W, y = H, z = D); every moving coordinate finite.  Returns both as (P, 3)
+    float64 host tensors."""
+    p, q = _landmarks_host(fixed_landmarks, 'fixed_landmarks'), _landmarks_host(moving_landmarks, 'moving_landmarks')
+    if p.shape != q.shape:
+        raise ValueError(f'fixed and moving landmarks must correspond row by row: {tuple(p.shape)} vs {tuple(q.shape)}')
+    D, H, W = dims
+    hi = torch.tensor([W - 1, H - 1, D - 1], dtype=torch.float64)
+    if not bool(torch.isfinite(p).all()) or bool((p < 0).any()) or bool((p > hi).any()):
+        raise ValueError(f'fixed landmarks must be finite (x, y, z) voxel coordinates inside [0, {W - 1}] x [0, {H - 1}] x '
+                         f'[0, {D - 1}]')
+    if not bool(torch.isfinite(q).all()):
+        raise ValueError('moving landmarks must be finite')
+    return p, q
+
+
+def landmark_map(T, fixed_landmarks, moving_landmarks, spacing):
+    """
+    Predicted moving positions and target registration errors of the P landmark pairs under the C transformations T
+    (C,3,D,H,W) fp32 (normalised sampling grids, SGLDSampler.transformation()).  Landmarks are (P,3) (x, y, z) voxel
+    coordinates, row i of the fixed ones corresponding to row i of the moving ones; spacing (x, y, z) in mm.  The ranges are
+    checked here on the host (check_landmarks).  Returns pred (C,P,3) fp64 (moving voxel units: where the warp samples the
+    moving image for the fixed landmark) and tre (C,P) fp64 in mm, device tensors (irs_landmark_map).
+    """
+    lib = _lib.load()
+    _lib.require_cuda(T)
+    _f32(T)
+    C, D, H, W = _dims(T)
+    if T.shape[1] != 3:
+        raise ValueError('T must be (C,3,D,H,W)')
+    p, q = check_landmarks(fixed_landmarks, moving_landmarks, (D, H, W))
+    sp = landmark_spacing(spacing)
+    P = p.shape[0]
+    pd, qd = p.to(T.device), q.to(T.device)
+    pred = torch.empty(C, P, 3, device=T.device, dtype=torch.float64)
+    tre = torch.empty(C, P, device=T.device, dtype=torch.float64)
+    _lib.check(lib.irs_landmark_map(_lib.ptr(T), C, D, H, W, _lib.ptr(pd), _lib.ptr(qd), P, (ctypes.c_double * 3)(*sp),
+                                    _lib.ptr(pred), _lib.ptr(tre), _lib.stream()))
+    return pred, tre
+
+
+def landmark_update(pred, tre, count_before, acc):
+    """
+    Fold the C samples pred (C,P,3) / tre (C,P) fp64 (landmark_map) into the landmark accumulators acc (P,11) fp64 of
+    `count_before` earlier samples, in place, chains in index order: per landmark the Welford mean (3) and co-moments
+    (xx, xy, xz, yy, yz, zz) of the predicted position and the Welford mean / M2 of the TRE.  Returns the (C,3) fp64 device
+    rows of this sample per chain, landmarks in index order: sum TRE, sum TRE^2, max TRE (irs_landmark_update).
+    """
+    lib = _lib.load()
+    _lib.require_cuda(pred, tre, acc)
+    if pred.dtype != torch.float64 or tre.dtype != torch.float64 or acc.dtype != torch.float64:
+        raise NotImplementedError('fp64 landmark tensors only')
+    if pred.dim() != 3 or pred.shape[2] != 3:
+        raise ValueError('pred must be (C,P,3)')
+    C, P = pred.shape[:2]
+    if tuple(tre.shape) != (C, P) or tuple(acc.shape) != (P, _lib.LANDMARK_ACC):
+        raise ValueError(f'tre must be ({C}, {P}) and acc ({P}, {_lib.LANDMARK_ACC})')
+    stats = torch.empty(C, 3, device=pred.device, dtype=torch.float64)
+    _lib.check(lib.irs_landmark_update(_lib.ptr(pred), _lib.ptr(tre), C, P, float(count_before), _lib.ptr(acc),
+                                       _lib.ptr(stats), _lib.stream()))
+    return stats
+
+
+def landmark_posterior(acc, n, moving_landmarks, spacing):
+    """
+    The landmark posterior from the accumulators acc (P,11) of n >= 1 samples: a (P,16) fp64 device table per landmark
+    (irs_landmark_posterior): [0:3] mean predicted position (moving voxels), [3] TRE of the mean, [4] E[TRE], and for n >= 2
+    (NaN for n = 1) [5] std of TRE, [6:12] covariance (xx, xy, xz, yy, yz, zz) in mm^2, [12:15] principal standard deviations
+    in mm (descending), [15] squared Mahalanobis distance of the moving landmark from the mean (+inf for a singular covariance).
+    """
+    lib = _lib.load()
+    _lib.require_cuda(acc)
+    if acc.dtype != torch.float64 or acc.dim() != 2 or acc.shape[1] != _lib.LANDMARK_ACC:
+        raise ValueError(f'acc must be a (P, {_lib.LANDMARK_ACC}) fp64 tensor')
+    P = acc.shape[0]
+    q = _landmarks_host(moving_landmarks, 'moving_landmarks')
+    if q.shape[0] != P or not bool(torch.isfinite(q).all()):
+        raise ValueError(f'moving_landmarks must be {P} finite rows')
+    sp = landmark_spacing(spacing)
+    out = torch.empty(P, _lib.LANDMARK_COLS, device=acc.device, dtype=torch.float64)
+    _lib.check(lib.irs_landmark_posterior(_lib.ptr(acc), _lib.ptr(q.to(acc.device)), P, int(n), (ctypes.c_double * 3)(*sp),
+                                          _lib.ptr(out), _lib.stream()))
+    return out

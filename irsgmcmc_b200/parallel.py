@@ -2,7 +2,8 @@
 Multi-GPU: chains shard by rank with no per-iteration communication (SURVEY.md section 8e).  The collectives are the
 merge of the per-rank Welford posterior moments and, when convergence diagnostics are requested, the partial sums of the split
 R-hat -- two sum all-reduces each (NCCL over NVLink on GPUs; gloo in CPU tests) --, for the segmentation posterior, one sum
-all-reduce of the integer label counts, and for the Jacobian posterior two sum all-reduces of its per-voxel Welford moments.
+all-reduce of the integer label counts, for the Jacobian posterior two sum all-reduces of its per-voxel Welford moments, and
+for the landmark posterior two fp64 sum all-reduces of its per-landmark moments.
 
 The reference has no distributed code at all; the quantity computed here is its calc_posterior_statistics
 (utils/util.py:114-120: mean and unbiased std over every kept sample of every chain).
@@ -101,6 +102,41 @@ def merge_jacobian_moments(n_local, folds, mean, m2, group=None):
     dist.all_reduce(m2_t, op=dist.ReduceOp.SUM, group=group)
     folds_t = (n_total - nv.to(torch.int32)).view_as(folds)
     return n_total, folds_t, mean_t, m2_t
+
+
+def merge_landmark_moments(n_local, acc, group=None):
+    """
+    The landmark accumulators acc (P, 11) fp64 (ops.landmark_update: mean (3), co-moments xx xy xz yy yz zz (6), TRE mean,
+    TRE M2) over the ranks of `group`: Chan's merge with n_r samples on rank r,
+        n = sum_r n_r ;  mean = sum_r n_r mean_r / n ;  M_ab = sum_r [ M_ab,r + n_r (mean_r - mean)_a (mean_r - mean)_b ]
+    for the position and the same for the TRE, in two fp64 SUM all-reduces: the first carries n in front and the n_r-weighted
+    means, the second the co-moment terms.  A rank without samples contributes nothing.  Returns (n_total, acc) with a new
+    tensor, identical on every rank; the local accumulators are kept, so sampling can continue.  One host read (n_total).
+    """
+    if not (dist.is_available() and dist.is_initialized()) or dist.get_world_size(group) == 1:
+        return int(n_local), acc.clone()
+    P = acc.shape[0]
+    n_r = float(n_local)
+    buf = torch.empty(1 + 4 * P, device=acc.device, dtype=torch.float64)
+    buf[0] = n_r
+    sums = buf[1:].view(P, 4)
+    torch.mul(acc[:, [0, 1, 2, 9]], n_r, out=sums)
+    dist.all_reduce(buf, op=dist.ReduceOp.SUM, group=group)
+    n_total = int(buf[0].item())
+    if n_total < 1:
+        return 0, torch.zeros_like(acc)
+    mean = sums / float(n_total)
+    d = acc[:, [0, 1, 2, 9]] - mean
+    out = torch.empty_like(acc)
+    out[:, [0, 1, 2, 9]] = mean
+    a, b = [0, 0, 0, 1, 1, 2], [0, 1, 2, 1, 2, 2]
+    out[:, 3:9] = acc[:, 3:9] + n_r * d[:, a] * d[:, b]
+    out[:, 10] = acc[:, 10] + n_r * d[:, 3] * d[:, 3]
+    m = out[:, [3, 4, 5, 6, 7, 8, 10]].contiguous()
+    dist.all_reduce(m, op=dist.ReduceOp.SUM, group=group)
+    out[:, 3:9] = m[:, :6]
+    out[:, 10] = m[:, 6]
+    return n_total, out
 
 
 def merge_moments(n_local, moments, group=None):

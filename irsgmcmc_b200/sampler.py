@@ -171,6 +171,8 @@ class SGLDSampler:
         self._segpost = None
         # accumulators of the Jacobian posterior (enable_jacobian_posterior): None while disabled
         self._jacpost = None
+        # landmark pairs and accumulators of the landmark posterior (enable_landmark_posterior): None while disabled
+        self._lmpost = None
 
     # ------------------------------------------------------------------------------------------------------------------
     def _make_config(self):
@@ -315,6 +317,10 @@ class SGLDSampler:
         if self._jacpost is not None:   # Jacobian posterior enabled: its accumulators travel too
             j = self._jacpost
             sd['jacpost'] = {'n': j['n'], 'folds': j['folds'].cpu(), 'mean': j['mean'].cpu(), 'm2': j['m2'].cpu()}
+        if self._lmpost is not None:   # landmark posterior enabled: the landmarks, spacing and accumulators travel too
+            lm = self._lmpost
+            sd['lmpost'] = {'fixed': lm['fixed_host'].clone(), 'moving': lm['moving_host'].clone(), 'spacing': list(lm['spacing']),
+                            'n': lm['n'], 'acc': lm['acc'].cpu()}
         return sd
 
     @torch.no_grad()
@@ -352,6 +358,15 @@ class SGLDSampler:
                 self._jacpost[name].copy_(sd['jacpost'][name])
         elif self._jacpost is not None:
             self.enable_jacobian_posterior()
+        # and for the landmark posterior (with the checkpoint's landmarks and spacing)
+        if 'lmpost' in sd:
+            lm = sd['lmpost']
+            self.enable_landmark_posterior(lm['fixed'], lm['moving'], lm['spacing'])
+            self._lmpost['n'] = int(lm['n'])
+            self._lmpost['acc'].copy_(lm['acc'])
+        elif self._lmpost is not None:
+            lm = self._lmpost
+            self.enable_landmark_posterior(lm['fixed_host'], lm['moving_host'], lm['spacing'])
 
     def set_noise(self, eps=None, jitter_unit=None):
         """explicit N(0,1) / U[0,1) numbers (C,3,D,H,W) instead of Philox: exact noise-on parity tests"""
@@ -543,8 +558,9 @@ class SGLDSampler:
         caller has it already (warp_segmentation() of the current transformations), else warped here.  Without the
         segmentation posterior `seg_warped` is not used.  When the Jacobian posterior is enabled, log det J of every chain's
         transformation is folded into its accumulators and last_jacobian_stats is overwritten: `transformation` (C,3,D,H,W)
-        fp32 if the caller has it already (transformation() of the current state), else computed here.  Without the Jacobian
-        posterior `transformation` is not used."""
+        fp32 if the caller has it already (transformation() of the current state), else computed here.  When the landmark
+        posterior is enabled, the fixed landmarks are carried through the same transformation and folded into its
+        accumulators, and last_landmark_stats is overwritten.  Without either `transformation` is not used."""
         n3, n1 = 3 * self.V, self.V
         st = _lib.stream()
         if self._rhat is not None and self._rhat['k'] >= self._rhat['N']:
@@ -558,8 +574,8 @@ class SGLDSampler:
                     not seg_warped.is_cuda or not seg_warped.is_contiguous():
                 raise ValueError(f'seg_warped must be a contiguous ({self.C}, 1, {", ".join(map(str, self.dims))}) int16 '
                                  f'CUDA tensor')
-        j = self._jacpost
-        if j is not None:
+        j, lm = self._jacpost, self._lmpost
+        if j is not None or lm is not None:
             if transformation is None:
                 transformation = self.transformation()
             if transformation.dtype != torch.float32 or tuple(transformation.shape) != (self.C, 3, *self.dims) or \
@@ -592,6 +608,15 @@ class SGLDSampler:
                                                     _lib.ptr(j['m2']), _lib.ptr(j['stats']), _lib.ptr(j['partials']),
                                                     _lib.ptr(j['counters']), st))
             j['n'] += self.C
+        if lm is not None:
+            D, H, W = self.dims
+            P = lm['P']
+            _lib.check(self.lib.irs_landmark_map(_lib.ptr(transformation), self.C, D, H, W, _lib.ptr(lm['fixed']),
+                                                 _lib.ptr(lm['moving']), P, lm['host_spacing'], _lib.ptr(lm['pred']),
+                                                 _lib.ptr(lm['tre']), st))
+            _lib.check(self.lib.irs_landmark_update(_lib.ptr(lm['pred']), _lib.ptr(lm['tre']), self.C, P, float(lm['n']),
+                                                    _lib.ptr(lm['acc']), _lib.ptr(lm['stats']), st))
+            lm['n'] += self.C
 
     def posterior_moments(self, group=None):
         """
@@ -802,3 +827,67 @@ class SGLDSampler:
             raise RuntimeError('the Jacobian posterior has no accumulated sample yet')
         p_fold, mean_out, std_out, summary = ops.jacobian_posterior(folds, mean, m2, n, self.mask.view(self.dims))
         return {'n': n, 'fold_probability': p_fold, 'log_det_J_mean': mean_out, 'log_det_J_std': std_out, 'summary': summary}
+
+    # ------------------------------------------------------------------------------------------------------------------
+    # landmark registration error and landmark posterior
+    # ------------------------------------------------------------------------------------------------------------------
+    @torch.no_grad()
+    def enable_landmark_posterior(self, fixed_landmarks, moving_landmarks, spacing):
+        """
+        Allocate (or reset) the landmark posterior for P corresponding landmark pairs: (P,3) zero-based (x, y, z) voxel
+        coordinates, row i of the fixed landmarks corresponding to row i of the moving ones (fixed ones finite and inside the
+        volume, moving ones finite: checked here, once), spacing (x, y, z) in mm.  accumulate() then also carries every fixed
+        landmark through every chain's transformation and folds the predicted moving position and its target registration
+        error (TRE) into per-landmark fp64 accumulators -- 88 P bytes, plus 32 C P bytes of per-sample scratch -- in two
+        launches with no synchronisation; moments, split R-hat, label counts, Jacobian accumulators and chain states are
+        unchanged.  last_landmark_stats keeps the per-chain TRE sums of the latest sample; landmark_posterior() gives the
+        per-landmark table.
+        """
+        from . import ops
+        p, q = ops.check_landmarks(fixed_landmarks, moving_landmarks, self.dims)
+        sp = ops.landmark_spacing(spacing)
+        P = p.shape[0]
+        dev = self.device
+        f64 = dict(device=dev, dtype=torch.float64)
+        self._lmpost = None   # release the old buffers first
+        self._lmpost = {'P': P, 'fixed_host': p, 'moving_host': q, 'fixed': p.to(dev), 'moving': q.to(dev), 'spacing': sp,
+                        'host_spacing': (ctypes.c_double * 3)(*sp), 'n': 0,
+                        'acc': torch.zeros(P, _lib.LANDMARK_ACC, **f64), 'pred': torch.empty(self.C, P, 3, **f64),
+                        'tre': torch.empty(self.C, P, **f64), 'stats': torch.zeros(self.C, 3, **f64)}
+
+    def disable_landmark_posterior(self):
+        """free the landmark buffers; accumulate() no longer reads the landmarks"""
+        self._lmpost = None
+
+    @property
+    def landmark_posterior_enabled(self):
+        return self._lmpost is not None
+
+    @property
+    def last_landmark_stats(self):
+        """(C,3) fp64 device tensor of the latest accumulated sample, per chain over the landmarks in index order: sum of the
+        TREs, sum of their squares, max TRE (mm; overwritten by every accumulate(); copy it to keep it).  The mean TRE of
+        the sample is the first column over P."""
+        if self._lmpost is None:
+            raise RuntimeError('the landmark posterior is not enabled (enable_landmark_posterior(...) before sampling)')
+        return self._lmpost['stats']
+
+    @torch.no_grad()
+    def landmark_posterior(self, group=None):
+        """
+        The landmark posterior over every sample accumulated by ALL ranks of `group` (parallel.merge_landmark_moments, two fp64
+        SUM all-reduces when torch.distributed is initialised; the local accumulators are kept, so sampling can continue).
+        Returns {'n': samples (kept samples x chains), 'table': the (P,16) fp64 device table of ops.landmark_posterior,
+                 'fixed_landmarks', 'moving_landmarks': the (P,3) fp64 host tables, 'spacing': (x, y, z)}.
+        """
+        from . import ops
+        from .parallel import merge_landmark_moments
+        lm = self._lmpost
+        if lm is None:
+            raise RuntimeError('the landmark posterior is not enabled (enable_landmark_posterior(...) before sampling)')
+        n, acc = merge_landmark_moments(lm['n'], lm['acc'], group)
+        if n < 1:
+            raise RuntimeError('the landmark posterior has no accumulated sample yet')
+        table = ops.landmark_posterior(acc, n, lm['moving_host'], lm['spacing'])
+        return {'n': n, 'table': table, 'fixed_landmarks': lm['fixed_host'].clone(), 'moving_landmarks': lm['moving_host'].clone(),
+                'spacing': list(lm['spacing'])}

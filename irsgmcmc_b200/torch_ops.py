@@ -24,6 +24,8 @@ which calls the adjoint op (the closed forms of SURVEY Appendix A, no scatter at
     calc_metrics, ASD part (utils/util.py:171-176)                        irsgmcmc::average_surface_distance
     (no reference counterpart: Hausdorff distance and HD95, calc_HD_GPU)   irsgmcmc::surface_distances
     (no reference counterpart: posterior of the warped segmentation)      irsgmcmc::label_counts_update (in place), ::label_posterior
+    (no reference counterpart: TRE and landmark posterior, calc_TRE_GPU)   irsgmcmc::landmark_map, ::landmark_update (in place),
+                                                                          ::landmark_posterior
     Trainer._SGLD_transition (trainer/trainer.py:291-356)                 irsgmcmc::sgld_step (the fused transition, in place)
 
 The drop-in modules (utils/, model/) and the fused sampler use the same launchers; this module adds the dispatcher-visible
@@ -458,6 +460,43 @@ def _(counts, n, labels, seg_fixed):
     L, D, H, W = counts.shape
     return (counts.new_empty(L, D, H, W, dtype=torch.float32), counts.new_empty(1, 1, D, H, W, dtype=torch.int16),
             counts.new_empty(1, D, H, W, dtype=torch.float32), counts.new_empty(L, 3, dtype=torch.int64))
+
+
+# ---- landmark registration error and landmark posterior ---------------------------------------------------------------------------
+@_op('landmark_map')
+def landmark_map(T: Tensor, fixed_landmarks: Tensor, moving_landmarks: Tensor, spacing: Sequence[float]) -> Tuple[Tensor, Tensor]:
+    """(pred (C, P, 3) fp64 moving voxel positions, tre (C, P) fp64 in mm) of the (P, 3) landmark pairs under the C
+    transformations T (ops.landmark_map)"""
+    return ops.landmark_map(T.contiguous(), fixed_landmarks, moving_landmarks, list(spacing))
+
+
+@landmark_map.register_fake
+def _(T, fixed_landmarks, moving_landmarks, spacing):
+    C, P = T.shape[0], fixed_landmarks.shape[0]
+    return T.new_empty(C, P, 3, dtype=torch.float64), T.new_empty(C, P, dtype=torch.float64)
+
+
+@torch.library.custom_op(f'{_NS}::landmark_update', mutates_args=('acc',), device_types='cuda')
+def landmark_update(pred: Tensor, tre: Tensor, count_before: int, acc: Tensor) -> Tensor:
+    """acc (P, 11) fp64 += the C samples pred / tre in chain order (Welford); returns the (C, 3) per-chain rows sum TRE,
+    sum TRE^2, max TRE (ops.landmark_update)"""
+    return ops.landmark_update(pred.contiguous(), tre.contiguous(), count_before, acc)
+
+
+@landmark_update.register_fake
+def _(pred, tre, count_before, acc):
+    return pred.new_empty(pred.shape[0], 3, dtype=torch.float64)
+
+
+@_op('landmark_posterior')
+def landmark_posterior(acc: Tensor, n: int, moving_landmarks: Tensor, spacing: Sequence[float]) -> Tensor:
+    """(P, 16) fp64 per-landmark posterior table from the accumulators of n samples (ops.landmark_posterior)"""
+    return ops.landmark_posterior(acc.contiguous(), n, moving_landmarks, list(spacing))
+
+
+@landmark_posterior.register_fake
+def _(acc, n, moving_landmarks, spacing):
+    return acc.new_empty(acc.shape[0], _lib.LANDMARK_COLS, dtype=torch.float64)
 
 
 # ---- the fused transition -------------------------------------------------------------------------------------------------------------

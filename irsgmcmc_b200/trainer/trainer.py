@@ -18,7 +18,7 @@ import time
 import numpy as np
 import torch
 
-from .. import parallel
+from .. import _lib, parallel
 from ..sampler import SGLDConfig, SGLDSampler
 from ..utils.util import calc_DSC_GPU, calc_no_non_diffeomorphic_voxels
 
@@ -409,7 +409,7 @@ class Trainer:
 
     @torch.no_grad()
     def _test_VI(self, var_params_q_v=None, no_samples=None, modules=None, speed_test_samples=100, with_ASD=True,
-                 with_seg_posterior=False, with_jacobian_posterior=False, with_HD=False, HD_percentile=95.0):
+                 with_seg_posterior=False, with_jacobian_posterior=False, with_HD=False, HD_percentile=95.0, with_TRE=False):
         """
         evaluation of the fitted q(v) (reference trainer.py:226-289): `no_samples_VI_test` draws from q(v) -> Sobolev smoothing ->
         transformation -> number of folded voxels + log det J, warped image and segmentation, ASD / DSC per structure, the sample on
@@ -427,6 +427,9 @@ class Trainer:
         with_HD=True (needs the segmentations, like 'ASD') adds 'HD' and 'HD95' (the key follows HD_percentile: 'HD99' for 99),
         (S, structures) arrays of the Hausdorff distance and its percentile per draw (utils.util.calc_HD_GPU; with with_ASD, one
         distance transform gives all three); with with_seg_posterior, 'HD_majority' and 'HD95_majority' per structure.
+        with_TRE=True (needs 'landmarks' in both the fixed and the moving dict with the same P, and S >= 1, else ValueError) adds
+        'TRE' (S, 1), the mean target registration error of the landmarks per draw, and 'landmark_posterior' over the S draws
+        with the entries of _run_MCMC's; with save_dir, VI_landmarks.vtk.
         """
         from .. import ops
         from ..utils import SobolevGrad, calc_metrics
@@ -452,6 +455,12 @@ class Trainer:
                    'mean': torch.zeros(*self.dims, device=dev), 'm2': torch.zeros(*self.dims, device=dev),
                    'mask': self.fixed['mask'].to(dev).view(*self.dims), 'scratch': ops.jacobian_scratch(1, dev)}
             jac_traces = torch.zeros(S, 1, 4, device=dev, dtype=torch.float64)
+        if with_TRE:
+            if S < 1:
+                raise ValueError('with_TRE=True needs at least one sample')
+            lm_p, lm_q = self._landmark_pair()
+            lm_acc = torch.zeros(lm_p.shape[0], _lib.LANDMARK_ACC, device=dev, dtype=torch.float64)
+            lm_traces = torch.zeros(S, 1, 3, device=dev, dtype=torch.float64)
         transformation_module, registration_module, diff_op = m['transformation_module'], m['registration_module'], m['reg_loss'].diff_op
 
         def register(v):
@@ -469,6 +478,9 @@ class Trainer:
             if with_jacobian_posterior:
                 jac_traces[test_sample_no - 1] = ops.jacobian_update(transformation.contiguous(), jac['mask'], test_sample_no - 1,
                                                                      jac['folds'], jac['mean'], jac['m2'], jac['scratch'])
+            if with_TRE:
+                pred, tre = ops.landmark_map(transformation.contiguous(), lm_p, lm_q, self.im_spacing)
+                lm_traces[test_sample_no - 1] = ops.landmark_update(pred, tre, test_sample_no - 1, lm_acc)
             if with_seg:
                 seg_moving_warped = registration_module(moving['seg'], transformation)
                 if with_ASD and not with_HD:
@@ -510,6 +522,10 @@ class Trainer:
             p_fold, mean_ld, std_ld, summary = ops.jacobian_posterior(jac['folds'], jac['mean'], jac['m2'], S, jac['mask'])
             post = {'n': S, 'fold_probability': p_fold, 'log_det_J_mean': mean_ld, 'log_det_J_std': std_ld, 'summary': summary}
             result['jacobian_posterior'] = self._jacobian_posterior(post, jac_traces, 'VI', gather=False)
+        if with_TRE:
+            post = {'n': S, 'table': ops.landmark_posterior(lm_acc, S, lm_q, self.im_spacing), 'fixed_landmarks': lm_p,
+                    'moving_landmarks': lm_q, 'spacing': ops.landmark_spacing(self.im_spacing)}
+            result['TRE'], result['landmark_posterior'] = self._landmark_posterior(post, lm_traces, 'VI', gather=False)
         if speed_test_samples:   # reference trainer.py:275-289
             torch.cuda.synchronize()
             t0 = time.perf_counter()
@@ -575,7 +591,7 @@ class Trainer:
 
     # -- the loop around it (reference trainer.py:358-476) -------------------------------------------------------------
     def _run_MCMC(self, data_loss=None, reg_loss=None, speed_test_iters=100, with_ASD=False, with_R_hat=False,
-                  with_seg_posterior=False, with_jacobian_posterior=False, with_HD=False, HD_percentile=95.0):
+                  with_seg_posterior=False, with_jacobian_posterior=False, with_HD=False, HD_percentile=95.0, with_TRE=False):
         """burn-in + sampling; returns {'mean','std_dev', 'im_mean','im_std', 'n', 'DSC', 'ASD', 'no_non_diffeomorphic_voxels',
         'samples_per_sec'}; posterior statistics are over the kept samples of ALL ranks.  'ASD' (average surface distance,
         reference utils/util.py:171-176 through SimpleITK on the host): with_ASD=True computes it per kept sample on the device
@@ -617,7 +633,19 @@ class Trainer:
         of the contour distances (numpy's default percentile; utils.util.calc_HD_GPU, the label-contour / distance transform
         kernels of the ASD plus a radix select on the device).  With with_ASD as well, one distance transform per kept sample
         gives all three.  With with_seg_posterior, the structures also get 'HD_majority' and 'HD95_majority'.  With
-        with_HD=False nothing of this runs."""
+        with_HD=False nothing of this runs.
+
+        with_TRE=True (needs 'landmarks' in both the fixed and the moving dict: (P,3) zero-based (x, y, z) voxel coordinates,
+        row i of one corresponding to row i of the other, else ValueError) adds 'TRE', the mean target registration error
+        (mm, spacing im_spacing) of the landmarks per kept sample and chain of every rank, a (kept samples, chains) array, and
+        'landmark_posterior' (SGLDSampler.enable_landmark_posterior, over every kept sample of every chain of every rank): the
+        per-landmark arrays 'mean_position' (moving voxels), 'TRE_of_mean', 'expected_TRE', 'TRE_std', 'covariance' (P,6)
+        mm^2, 'principal_std' (P,3) mm, 'mahalanobis2', the summaries 'mean_TRE_of_mean', 'mean_expected_TRE',
+        'initial_TRE' / 'mean_initial_TRE' (the identity transformation), 'coverage' {50, 90, 95: share of the true moving
+        landmarks inside the posterior's credible ellipsoid of that level}, 'uncertainty_error_spearman' (rank correlation of
+        sqrt(trace covariance) with the TRE of the mean), and 'TRE_max' / 'TRE_std' (max and population std over the
+        landmarks) per kept sample and chain.  With save_dir, MCMC_landmarks.vtk is written as well.  With with_TRE=False
+        nothing of this runs."""
         if self.SGLD_params is None:
             self._SGLD_init()
         s = self.sampler
@@ -627,6 +655,8 @@ class Trainer:
             s.enable_segmentation_posterior(list(self.structures_dict.values()))
         if with_jacobian_posterior:
             s.enable_jacobian_posterior()
+        if with_TRE:
+            s.enable_landmark_posterior(*self._landmark_pair(), self.im_spacing)
         if not self._gmm_pushed:
             if data_loss is not None or reg_loss is not None:
                 self._push_hyper(data_loss, reg_loss)
@@ -646,6 +676,11 @@ class Trainer:
             jac_traces = torch.zeros(sum(1 for i in range(1, total + 1) if self._is_kept(i)), self.no_chains, 4,
                                      device=s.device, dtype=torch.float64)
             k_jac = 0
+        if with_TRE:
+            # per kept sample, this rank's rows of the landmark TRE sums: a device copy, no synchronisation
+            lm_traces = torch.zeros(sum(1 for i in range(1, total + 1) if self._is_kept(i)), self.no_chains, 3,
+                                    device=s.device, dtype=torch.float64)
+            k_lm = 0
         from ..utils.diff_op import GradientOperator
         diff_op = GradientOperator()
         it = 0
@@ -682,6 +717,9 @@ class Trainer:
                 if with_jacobian_posterior:
                     jac_traces[k_jac].copy_(s.last_jacobian_stats)
                     k_jac += 1
+                if with_TRE:
+                    lm_traces[k_lm].copy_(s.last_landmark_stats)
+                    k_lm += 1
                 n_folded, log_det_J = calc_no_non_diffeomorphic_voxels(T, diff_op)
                 folded.append(n_folded)
                 if self.save_dir is not None:
@@ -716,6 +754,10 @@ class Trainer:
             post = s.jacobian_posterior()
             s.disable_jacobian_posterior()
             result['jacobian_posterior'] = self._jacobian_posterior(post, jac_traces, 'MCMC')
+        if with_TRE:
+            post = s.landmark_posterior()
+            s.disable_landmark_posterior()
+            result['TRE'], result['landmark_posterior'] = self._landmark_posterior(post, lm_traces, 'MCMC')
         if self.save_dir is not None and (not torch.distributed.is_initialized() or torch.distributed.get_rank() == 0):
             # MCMC_sample_{mean,std_dev}[_masked].vtk like the reference (trainer.py:457-460, logger/logger.py:110-131)
             from ..logger import save_displacement_mean_and_std_dev
@@ -850,6 +892,47 @@ class Trainer:
                               ('fold_probability', 'fold_probability')):
                 save_im_to_disk(post[key].cpu(), os.path.join(self.save_dir, f'{model}_{name}.nii.gz'), sp)
         return post
+
+    def _landmark_pair(self):
+        """the (fixed, moving) landmark tables of the image dicts, (P,3) each"""
+        p, q = self.fixed.get('landmarks'), self.moving.get('landmarks')
+        if p is None or q is None:
+            raise ValueError("with_TRE=True needs 'landmarks' in both the fixed and the moving dict")
+        if tuple(p.shape) != tuple(q.shape) or p.dim() != 2 or p.shape[1] != 3:
+            raise ValueError(f'fixed and moving landmarks must both be (P, 3) with the same P: {tuple(p.shape)} vs '
+                             f'{tuple(q.shape)}')
+        return p, q
+
+    def _landmark_posterior(self, post, traces, model, gather=True):
+        """('TRE', 'landmark_posterior') of _run_MCMC / _test_VI(with_TRE=True) from the dict of
+        SGLDSampler.landmark_posterior and this rank's per-sample rows (N, C, 3) = (sum TRE, sum TRE^2, max TRE); with gather,
+        all ranks' rows at their global chain offsets (one SUM all-reduce of a zero-padded buffer, as the R-hat traces).
+        {model}_landmarks.vtk in save_dir: the mean positions in mm, the covariance, E[TRE], the TRE of the mean and d^2"""
+        from ..utils.util import landmark_posterior_summary
+        if gather:
+            s = self.sampler
+            allt = torch.zeros(traces.shape[0], self.no_chains_total, 3, device=traces.device, dtype=torch.float64)
+            allt[:, s.chain_offset:s.chain_offset + self.no_chains] = traces
+            if torch.distributed.is_available() and torch.distributed.is_initialized() and \
+                    torch.distributed.get_world_size() > 1:
+                torch.distributed.all_reduce(allt, op=torch.distributed.ReduceOp.SUM)
+            traces = allt
+        t = traces.cpu().numpy()
+        P = post['table'].shape[0]
+        mean = t[..., 0] / P
+        out = landmark_posterior_summary(post['table'], post['fixed_landmarks'], post['moving_landmarks'], post['spacing'])
+        out['n'] = post['n']
+        out['TRE_max'] = t[..., 2]
+        out['TRE_std'] = np.sqrt(np.maximum(t[..., 1] / P - mean * mean, 0.0))   # population std over the landmarks
+        if self.save_dir is not None and (not torch.distributed.is_initialized() or torch.distributed.get_rank() == 0):
+            import os
+            from ..logger import save_landmarks_to_disk
+            os.makedirs(self.save_dir, exist_ok=True)
+            sp = np.asarray(post['spacing'], dtype=np.float64)
+            save_landmarks_to_disk(os.path.join(self.save_dir, f'{model}_landmarks.vtk'), out['mean_position'] * sp,
+                                   out['covariance'], {'expected_TRE': out['expected_TRE'], 'TRE_of_mean': out['TRE_of_mean'],
+                                                       'mahalanobis2': out['mahalanobis2']})
+        return mean, out
 
     def _is_kept(self, sample_no):
         """reference trainer.py:414-415"""

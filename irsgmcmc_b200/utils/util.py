@@ -256,3 +256,101 @@ def calc_metrics(seg_fixed, seg_moving, structures_dict, spacing, GPU=True, no_s
     DSC = calc_DSC_GPU(no_samples, seg_fixed, seg_moving, structures_dict)
     ASD = calc_ASD_GPU(no_samples, seg_fixed, seg_moving, structures_dict, spacing)
     return ASD, DSC
+
+
+@torch.no_grad()
+def calc_TRE_GPU(T, fixed_landmarks, moving_landmarks, spacing):
+    """target registration error per transformation and landmark pair, float64 (C, P) in mm: T (C,3,D,H,W) fp32 normalised
+    sampling grids (SGLDSampler.transformation()), landmarks (P,3) zero-based (x, y, z) voxel coordinates with row i of the
+    fixed ones corresponding to row i of the moving ones, spacing (x, y, z) in mm.  The fixed landmark is carried to the moving
+    image by trilinear interpolation of T (where the warp samples the moving image for it) and compared with the moving
+    landmark.  CUDA kernel (ops.landmark_map), one host synchronisation; same definition as calc_TRE_host, which the tests
+    compare it with bit for bit.  CUDA T only -- no PyTorch path."""
+    if not T.is_cuda:
+        raise NotImplementedError('calc_TRE_GPU needs a CUDA transformation: irsgmcmc_b200 has no CPU path')
+    return ops.landmark_map(T.contiguous(), fixed_landmarks, moving_landmarks, spacing)[1].cpu().numpy()
+
+
+def landmark_predict_host(T, fixed_landmarks):
+    """(C, P, 3) float64 predicted moving positions of the fixed landmarks under T (C,3,D,H,W) on the host: the arithmetic of
+    irs_landmark_predict restated in numpy, every operation rounded on its own (bit-equal to the kernel)"""
+    T = np.asarray(T.detach().cpu() if hasattr(T, 'detach') else T, dtype=np.float32)
+    p = np.asarray(fixed_landmarks.detach().cpu() if hasattr(fixed_landmarks, 'detach') else fixed_landmarks, dtype=np.float64)
+    C, _, D, H, W = T.shape
+    n = np.array([W, H, D])
+    fl = np.floor(p)
+    with np.errstate(invalid='ignore'):
+        i0 = np.where(fl >= 0.0, np.where(fl <= n - 2, fl, n - 2), 0.0).astype(np.int64)   # NaN: 0
+    f = p - i0
+    x0, y0, z0 = i0[:, 0], i0[:, 1], i0[:, 2]
+    fx, fy, fz = f[:, 0], f[:, 1], f[:, 2]
+
+    def lerp(a, b, t):
+        return a + t * (b - a)
+
+    Td = T.astype(np.float64)
+    out = np.empty((C, p.shape[0], 3))
+    for ch in range(3):
+        t = Td[:, ch]
+
+        def at(dz, dy, dx):
+            return t[:, z0 + dz, y0 + dy, x0 + dx]
+        c00, c10 = lerp(at(0, 0, 0), at(0, 0, 1), fx), lerp(at(0, 1, 0), at(0, 1, 1), fx)
+        c01, c11 = lerp(at(1, 0, 0), at(1, 0, 1), fx), lerp(at(1, 1, 0), at(1, 1, 1), fx)
+        g = lerp(lerp(c00, c10, fy), lerp(c01, c11, fy), fz)
+        out[:, :, ch] = ((g + 1.0) * float(n[ch] - 1)) * 0.5
+    return out
+
+
+def landmark_tre_host(pred, moving_landmarks, spacing):
+    """(C, P) float64 |s o (pred - q)| with the squares summed in x, y, z order, as irs_landmark_tre"""
+    q = np.asarray(moving_landmarks.detach().cpu() if hasattr(moving_landmarks, 'detach') else moving_landmarks, dtype=np.float64)
+    s = [float(x) for x in np.asarray(spacing, dtype=np.float64).reshape(-1)[:3]]
+    acc = np.zeros(pred.shape[:2])
+    for a in range(3):
+        d = s[a] * (pred[..., a] - q[:, a])
+        acc = acc + d * d
+    return np.sqrt(acc)
+
+
+def calc_TRE_host(T, fixed_landmarks, moving_landmarks, spacing):
+    """calc_TRE_GPU restated in numpy on the host, float64 (C, P) in mm, bit-equal to the kernel"""
+    return landmark_tre_host(landmark_predict_host(T, fixed_landmarks), moving_landmarks, spacing)
+
+
+# the columns of the per-landmark posterior table (ops.landmark_posterior)
+LANDMARK_POSTERIOR_COLUMNS = {'mean_position': slice(0, 3), 'TRE_of_mean': 3, 'expected_TRE': 4, 'TRE_std': 5,
+                              'covariance': slice(6, 12), 'principal_std': slice(12, 15), 'mahalanobis2': 15}
+
+
+def landmark_posterior_summary(table, fixed_landmarks, moving_landmarks, spacing):
+    """
+    Host summaries of the (P, 16) landmark posterior table (ops.landmark_posterior) and the per-landmark arrays:
+      the columns by name (LANDMARK_POSTERIOR_COLUMNS) as numpy arrays;
+      'mean_TRE_of_mean', 'mean_expected_TRE'  means over the landmarks (mm);
+      'initial_TRE' (P,) and 'mean_initial_TRE'  |s o (p - q)|, the TRE of the identity transformation;
+      'coverage'  {50, 90, 95: fraction of landmarks whose squared Mahalanobis distance is <= the chi-square(3) quantile},
+                  the share of true positions inside the posterior's credible ellipsoid (NaN with fewer than two samples);
+      'uncertainty_error_spearman'  Spearman rank correlation of sqrt(trace covariance) with the TRE of the mean (NaN when
+                  undefined).
+    """
+    from scipy import stats
+    t = np.asarray(table.detach().cpu() if hasattr(table, 'detach') else table, dtype=np.float64)
+    p = np.asarray(fixed_landmarks.detach().cpu() if hasattr(fixed_landmarks, 'detach') else fixed_landmarks, dtype=np.float64)
+    q = np.asarray(moving_landmarks.detach().cpu() if hasattr(moving_landmarks, 'detach') else moving_landmarks, dtype=np.float64)
+    out = {name: t[:, col] for name, col in LANDMARK_POSTERIOR_COLUMNS.items()}
+    out['mean_TRE_of_mean'] = float(out['TRE_of_mean'].mean())
+    out['mean_expected_TRE'] = float(out['expected_TRE'].mean())
+    out['initial_TRE'] = landmark_tre_host(p[None], q, spacing)[0]
+    out['mean_initial_TRE'] = float(out['initial_TRE'].mean())
+    d2 = out['mahalanobis2']
+    out['coverage'] = {level: float('nan') if np.isnan(d2).any() else float(np.mean(d2 <= stats.chi2.ppf(level / 100.0, 3)))
+                       for level in (50, 90, 95)}
+    cov = out['covariance']
+    spread = np.sqrt(cov[:, 0] + cov[:, 3] + cov[:, 5])
+    ok = np.isfinite(spread) & np.isfinite(out['TRE_of_mean'])
+    rho = float('nan')
+    if ok.sum() >= 2 and np.ptp(spread[ok]) > 0 and np.ptp(out['TRE_of_mean'][ok]) > 0:
+        rho = float(stats.spearmanr(spread[ok], out['TRE_of_mean'][ok])[0])
+    out['uncertainty_error_spearman'] = rho
+    return out
